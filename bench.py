@@ -4,6 +4,7 @@ baseline beside it.
 
     python bench.py --gpus N --steps K --warmup W            # our arm
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU algorithm on the host cores
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's y = H*psi as DIR/hpsi.npy
 
 A step is one H·psi apply (MatMult_KronSumShell, src/DMRGKron.cpp:1827-1869) on the synthetic sweep-midpoint
 superblock of BASELINE.json configs[2] (J1-J2 12x6 cylinder, J2/J1 = 0.5, m = 2048 kept states; the largest
@@ -45,7 +46,29 @@ def parse():
     ap.add_argument("--no-sweep", action="store_true", help="skip the seconds-per-sweep measurement (DMRG-SquareLattice.x on the metric's config)")
     ap.add_argument("--sweep-msweeps", default="512,1024,2048", help="-msweeps of the seconds-per-sweep run (the last entry is the one reported)")
     ap.add_argument("--no-extras", action="store_true", help="only the H*psi line (no lanczos / sparse-sector / sweep sections)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None, help="write y = H*psi of the last timed step as DIR/hpsi.npy (float64; a fixed "
+                    "seeded sample of rows when the whole vector exceeds %d MB), so that two builds can be compared output for output" % (DUMP_BYTES // 10**6))
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+DUMP_BYTES = 64 * 10**6   # all files --dump-outputs writes, together
+
+
+def dump_outputs(path, arrays):
+    """float64 .npy files of what the timed path returned; a vector beyond its share of DUMP_BYTES is cut to a fixed, seeded,
+    sorted sample of its entries (the same for every run with the same arguments)."""
+    os.makedirs(path, exist_ok=True)
+    cap = (DUMP_BYTES // len(arrays) - 4096) // 8
+    for name, a in arrays.items():
+        a = np.asarray(a, dtype=np.float64).ravel()
+        if a.size > cap:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, cap, replace=False))]
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 def workload_label(config, m, n):
@@ -400,6 +423,14 @@ def main():
         barrier()
         ms = e0.elapsed_time(e1)
     launches = P.launch_count() - l0
+    # the result of the last timed apply, whole vector on rank 0 (each rank computed its own rows)
+    yh = y.get()
+    if world > 1:
+        ymask = np.zeros(n); ymask[rb:re_] = yh[rb:re_]
+        yt = torch.from_numpy(ymask).to(dev)
+        dist.all_reduce(yt)
+        yh = yt.cpu().numpy()
+        del yt
     soak()
     clocks = sampler.stop()
     t_local = torch.tensor([ms], dtype=torch.float64, device=dev)
@@ -408,15 +439,8 @@ def main():
     ms = float(t_local.item())
     ms_step = ms / args.steps
     value = st["alg_bytes_global"] / (ms_step * 1e-3) / 1e9  # one H*psi of the whole superblock, sharded over the ranks
-
-    # the result of the timed applies, whole vector on rank 0 (each rank computed its own rows)
-    yh = y.get()
-    if world > 1:
-        ymask = np.zeros(n); ymask[rb:re_] = yh[rb:re_]
-        yt = torch.from_numpy(ymask).to(dev)
-        dist.all_reduce(yt)
-        yh = yt.cpu().numpy()
-        del yt
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"hpsi": yh})
 
     # per-stage timing of the dominant kernel (chain_kernel) for the roofline
     f1, f2 = H.stage_flops()
