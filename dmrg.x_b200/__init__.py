@@ -364,8 +364,8 @@ class HShell:
         return a.value, b.value
 
     def MatMult_sharded(self, x, y):
-        """distributed MatMult: x holds this rank's rows on entry (full-length buffer), is all-gathered in place, then this
-        rank's rows of y are computed"""
+        """distributed MatMult: x holds this rank's rows on entry (full-length buffer), receives the sector halo its
+        tiles read in place, then this rank's rows of y are computed"""
         _chk(lib().dmrgx_hshell_apply_sharded(self.h, x.ptr, y.ptr))
 
     def MatMult_stage(self, stage, x, y):

@@ -137,7 +137,6 @@ struct Plan {
        so that the CTAs resident at any time work on the same range of left-operator groups: their V and right-factor
        panels (a fraction of the 270 + 93 MB at 12x6 m = 2048) then fit in L2 together instead of being re-read. */
     std::vector<int> item_phase;
-    bool phase_order = false;
     BufRef d_items, d_segs, d_reduces, scratch;
     void upload(Ctx* ctx);
     void run(Ctx* ctx, const double* x = nullptr, double* y = nullptr) const;
@@ -174,7 +173,6 @@ struct HShell {
     std::unique_ptr<SparsePlan> sparse; /* when set, the apply is one spmm launch and stage1 / stage2 are empty */
     BufRef work;                 /* V panels of stage 1 */
     BufRef xbuf, ybuf;           /* device staging of the host-buffer entry point */
-    void* h_pinned = nullptr;
     std::vector<BufRef> keep;    /* pre-summed right factors etc. */
     std::vector<std::shared_ptr<Operator>> keep_ops; /* operator products of correlators */
     long long alg_bytes = 0;     /* SURVEY §8d: 16*D + distinct operator tile bytes */
@@ -182,7 +180,6 @@ struct HShell {
     long long alg_bytes_global = 0; /* the same two figures for the whole (unsharded) operator */
     double alg_flops_global = 0;
     int nterms = 0;
-    ~HShell();
 };
 
 struct XForm {

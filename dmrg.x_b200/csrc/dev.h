@@ -1,5 +1,5 @@
-/*  dev.h — the thin device layer.  Everything above it (block.cpp, kron.cpp, hshell.cpp, eigs.cpp,
- *  truncate.cpp, abi.cpp) is plain C++ that plans work on the host and hands flat POD work lists
+/*  dev.h — the thin device layer.  Everything above it (block.cpp, hshell.cpp, eigs.cpp, truncate.cpp,
+ *  predict.cpp, plan.cpp, abi.cpp) is plain C++ that plans work on the host and hands flat POD work lists
  *  to the sm_100a kernels in dev_cuda.cu through the functions declared here.
  *
  *  The product library libdmrgx_b200.so links dev_cuda.cu and nothing else behind this interface; there
@@ -57,19 +57,15 @@ struct WorkItem {
 
 constexpr int TILE = 64;  /* maximum tile extent of a work item */
 
-struct Stream;            /* device, stream, solver handle */
+struct Stream;            /* device, stream, device heap, communicator */
 
 int init(int device, void* user_stream, Stream** out); /* 0 on success; fails loudly without a CUDA device */
 void destroy(Stream*);
 const char* last_error();
-int device_of(Stream*);
 void make_current(Stream*);   /* cudaSetDevice(device of the stream): called at every C-ABI entry point */
-void* raw_stream(Stream*);
 
 void* malloc_bytes(Stream*, size_t bytes);
 void free_bytes(Stream*, void* p);
-void* malloc_pinned(size_t bytes);
-void free_pinned(void* p);
 void h2d(Stream*, void* dst, const void* src, size_t bytes);
 void d2h(Stream*, void* dst, const void* src, size_t bytes);
 void d2d(Stream*, void* dst, const void* src, size_t bytes);
@@ -78,15 +74,14 @@ void sync(Stream*);
 /* number of kernel launches issued through this layer so far (bench.py's gpu_launches) */
 long long launch_count();
 
-/* ---- collectives: one process per GPU, NCCL over NVLink/NVSwitch (SURVEY.md §8e).  The path has exactly three exchange
-   steps: the all-gather of the sharded superblock vector before an apply, the all-reduce of a handful of scalars per
-   Lanczos step, and broadcasts of eigenvector / rotated-operator panels from the rank that computed them.  All calls
-   are enqueued on the context's stream (device-ordered, no host synchronisation). ---- */
+/* ---- collectives: one process per GPU, NCCL over NVLink/NVSwitch (SURVEY.md §8e).  The exchange steps of the path: the
+   sector-halo exchange of the sharded superblock vector before an apply, the all-reduce of a handful of scalars per
+   Lanczos step, in-place all-gathers of the finished ground state and of the rotated-operator panels, and broadcasts of
+   density-matrix eigenvectors and eigenvalues from the rank that computed them.  All calls are enqueued on the context's
+   stream (device-ordered, no host synchronisation). ---- */
 constexpr int COMM_ID_BYTES = 128;                       /* ncclUniqueId */
 int comm_unique_id(void* out);                           /* rank 0 creates it, the launcher hands it to the others */
 int comm_init(Stream*, int rank, int world, const void* id);
-int comm_rank(Stream*);
-int comm_world(Stream*);
 void allreduce_sum(Stream*, double* d_buf, long long n); /* in place */
 /* in place: rank r owns d_buf[offsets[r] .. offsets[r+1]) and receives all other ranges */
 void allgatherv(Stream*, double* d_buf, const long long* offsets);
@@ -147,11 +142,6 @@ void run_reduce(Stream*, const ReduceItem* d_items, int nitems, double* y, const
 /* vector kernels of the thick-restart Lanczos (all results stay on the device) */
 /* x[i] = u(seed, first + i): depends on the GLOBAL index only */
 void fill_random(Stream*, double* x, long long n, unsigned long long seed, long long first = 0);
-void multidot(Stream*, const double* V, long long ldv, int nvec, const double* w, long long n, double* d_out);
-/* w -= Σ_i d_coef[i] V_i ; if d_dots2: d_dots2[i] = V_i·w_new (fused second Gram-Schmidt pass);
-   if d_nrm2: *d_nrm2 = ||w_new||²  */
-void multiaxpy(Stream*, const double* V, long long ldv, int nvec, const double* d_coef, double* w, long long n, double* d_dots2,
-               double* d_nrm2);
 /* One fused Gram-Schmidt pass over the basis (a single read of V, deterministic reductions finished by the last block, no
    host involvement):   if d_coef:  w -= Σ_i d_coef[i]·V_i   (in place);   then, on the updated w,
    if d_dots: d_dots[i] = V_i·w (i < nvec);   if d_nrm2: *d_nrm2 = w·w.   nvec <= 40. */
@@ -169,16 +159,14 @@ void gs_final(Stream*, const double* V, long long ldv, int nvec, const double* w
 void scale_inv_norm(Stream*, const double* w, const double* d_nrm2, double* v, long long n);
 /* in place: V_a <- Σ_i S[i*kk+a] V_i  (i < ncv, a < kk), S on the device */
 void ritz_rotate(Stream*, double* V, long long ldv, long long n, int ncv, const double* d_S, int kk);
+/* *d_out = x·y (the reduction of gs_pass: one launch, fixed summation order) */
 void dot(Stream*, const double* x, const double* y, long long n, double* d_out);
-void scal(Stream*, double* x, long long n, double a);
 
-/* dense symmetric eigendecomposition of an n×n block (in place): on exit row k of A (row-major) is the
-   k-th eigenvector, eigenvalues ascending in d_w */
-int syevd(Stream*, int n, double* d_A, double* d_w);
-/* the same for a batch of independent blocks: block b is n[b]×n[b] at d_A[b], eigenvalues to d_w[b].  The blocks are
-   spread over a pool of solver streams (largest first) so that small and medium blocks, which cannot fill 148 SMs
-   one at a time, run concurrently; ordered after everything queued on the main stream, and the main stream
-   continues only when all blocks are done.  Returns 0 or the first failure. */
+/* dense symmetric eigendecomposition of a batch of independent blocks, in place: block b is n[b]×n[b] at d_A[b]; on exit
+   row k of it (row-major) is the k-th eigenvector, eigenvalues ascending in d_w[b].  Blocks of up to 64 states are solved by
+   one cyclic-Jacobi launch on a side stream; the larger ones, all together, by batched block Jacobi on the main stream.
+   Ordered after everything queued on the main stream, which continues only when all blocks are done.  Returns 0 or the
+   first failure. */
 int syevd_batch(Stream*, int nblocks, const int* n, double* const* d_A, double* const* d_w);
 /* dst[k][:] = src[(n-1-k)][:], k < m   (the m largest eigenvectors, descending) */
 void gather_rows_reversed(Stream*, const double* src, int n, int m, double* dst);

@@ -57,7 +57,6 @@ struct Stream {
     bool own = false;
     double* partials = nullptr; /* deterministic two-stage reductions */
     unsigned int* ticket = nullptr; /* "last block finishes the reduction" counter of gs_pass */
-    int* info = nullptr;
     int num_sms = 148;
     struct Arena { char* base = nullptr; size_t size = 0; std::map<size_t, size_t> free; /* offset -> length of the free ranges */ };
     std::vector<Arena> arenas;   /* what was actually cudaMalloc'ed */
@@ -93,7 +92,6 @@ int init(int device, void* user_stream, Stream** out) {
         CUDA_OK(cudaGetDeviceProperties(&prop, device));
         st->num_sms = prop.multiProcessorCount;
         CUDA_OK(cudaMalloc(&st->partials, sizeof(double) * RED_BLOCKS * RED_MAXVEC));
-        CUDA_OK(cudaMalloc(&st->info, sizeof(int) * 4));
         CUDA_OK(cudaMalloc(&st->ticket, sizeof(unsigned int)));
         CUDA_OK(cudaMemset(st->ticket, 0, sizeof(unsigned int)));
         *out = st;
@@ -116,13 +114,10 @@ void destroy(Stream* st) {
     for (auto& ar : st->arenas) cudaFree(ar.base);
     cudaFree(st->partials);
     cudaFree(st->ticket);
-    cudaFree(st->info);
     if (st->own) cudaStreamDestroy(st->s);
     delete st;
 }
-int device_of(Stream* st) { return st->device; }
 void make_current(Stream* st) { cudaSetDevice(st->device); }
-void* raw_stream(Stream* st) { return (void*)st->s; }
 
 /* Device memory: a stream-ordered heap.  A DMRG sweep frees and allocates panels of slowly varying sizes every step; handing
    each one back to the driver (cudaFreeAsync) let the pool fragment and re-map (200-700 ms stalls inside single steps), and
@@ -201,8 +196,6 @@ void free_bytes(Stream* st, void* p) {
         return;
     }
 }
-void* malloc_pinned(size_t bytes) { void* p = nullptr; CUDA_OK(cudaMallocHost(&p, bytes ? bytes : 8)); return p; }
-void free_pinned(void* p) { if (p) cudaFreeHost(p); }
 void h2d(Stream* st, void* dst, const void* src, size_t bytes) { if (bytes) CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, st->s)); }
 void d2h(Stream* st, void* dst, const void* src, size_t bytes) { if (bytes) CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToHost, st->s)); }
 void d2d(Stream* st, void* dst, const void* src, size_t bytes) { if (bytes) CUDA_OK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, st->s)); }
@@ -566,7 +559,7 @@ void run_chain(Stream* st, const WorkItem* d_items, int nitems, const Segment* d
         st->chain_cfg = true;
     }
     /* fewer than four waves of the 444 resident CTAs: the deeper copy ring (cold operands, short items) */
-    static const int deep_below = getenv("DMRGX_CHAIN_DEEP_BELOW") ? atoi(getenv("DMRGX_CHAIN_DEEP_BELOW")) : 1800;
+    constexpr int deep_below = 1800;
     if (nitems < deep_below) chain_kernel<3><<<nitems, NTHREADS, smem3, st->s>>>(d_items, d_segs, x, y, w);
     else chain_kernel<2><<<nitems, NTHREADS, smem2, st->s>>>(d_items, d_segs, x, y, w);
     LAUNCH_CHECK();
@@ -828,82 +821,6 @@ void fill_random(Stream* st, double* x, long long n, unsigned long long seed, lo
     LAUNCH_CHECK();
 }
 
-template <int NV>
-__global__ void __launch_bounds__(256) multidot_kernel(const double* __restrict__ V, long long ldv, int nvec, const double* __restrict__ w,
-                                                       long long n, double* __restrict__ partials) {
-    double s[NV];
-#pragma unroll
-    for (int i = 0; i < NV; ++i) s[i] = 0.0;
-    for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < n; q += (long long)gridDim.x * blockDim.x) {
-        const double wq = w[q];
-#pragma unroll
-        for (int i = 0; i < NV; ++i)
-            if (i < nvec) s[i] += V[i * ldv + q] * wq;
-    }
-    __shared__ double sh[NV][8];
-    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-#pragma unroll
-    for (int i = 0; i < NV; ++i) {
-        double v = warp_sum(s[i]);
-        if (lane == 0) sh[i][wid] = v;
-    }
-    __syncthreads();
-    if (threadIdx.x < NV) {
-        double v = 0.0;
-        for (int k = 0; k < 8; ++k) v += sh[threadIdx.x][k];
-        partials[(long long)blockIdx.x * NV + threadIdx.x] = v;
-    }
-}
-template <int NV>
-__global__ void reduce_partials_kernel(const double* __restrict__ partials, int nblocks, int nvec, double* __restrict__ out) {
-    const int i = blockIdx.x; /* one block (32 threads) per output */
-    if (i >= nvec) return;
-    double v = 0.0;
-    for (int b = threadIdx.x; b < nblocks; b += 32) v += partials[(long long)b * NV + i];
-    v = warp_sum(v);
-    if (threadIdx.x == 0) out[i] = v;
-}
-
-void multidot(Stream* st, const double* V, long long ldv, int nvec, const double* w, long long n, double* d_out) {
-    constexpr int NV = 8;
-    const int blocks = (int)std::max<long long>(1, std::min<long long>((n + 255) / 256, RED_BLOCKS));
-    for (int v0 = 0; v0 < nvec; v0 += NV) {
-        const int nv = std::min(NV, nvec - v0);
-        multidot_kernel<NV><<<blocks, 256, 0, st->s>>>(V + (long long)v0 * ldv, ldv, nv, w, n, st->partials);
-        LAUNCH_CHECK();
-        reduce_partials_kernel<NV><<<nv, 32, 0, st->s>>>(st->partials, blocks, nv, d_out + v0);
-        LAUNCH_CHECK();
-    }
-}
-void dot(Stream* st, const double* x, const double* y, long long n, double* d_out) { multidot(st, x, n, 1, y, n, d_out); }
-
-template <int NV>
-__global__ void __launch_bounds__(256) multiaxpy_kernel(const double* __restrict__ V, long long ldv, int nvec, const double* __restrict__ coef,
-                                                        double* __restrict__ w, long long n) {
-    __shared__ double c[NV];
-    if (threadIdx.x < NV) c[threadIdx.x] = (threadIdx.x < nvec) ? coef[threadIdx.x] : 0.0;
-    __syncthreads();
-    for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < n; q += (long long)gridDim.x * blockDim.x) {
-        double acc = w[q];
-#pragma unroll
-        for (int i = 0; i < NV; ++i)
-            if (i < nvec) acc -= c[i] * V[i * ldv + q];
-        w[q] = acc;
-    }
-}
-void multiaxpy(Stream* st, const double* V, long long ldv, int nvec, const double* d_coef, double* w, long long n, double* d_dots2,
-               double* d_nrm2) {
-    constexpr int NV = 8;
-    const int blocks = (int)std::max<long long>(1, std::min<long long>((n + 255) / 256, RED_BLOCKS));
-    for (int v0 = 0; v0 < nvec; v0 += NV) {
-        const int nv = std::min(NV, nvec - v0);
-        multiaxpy_kernel<NV><<<blocks, 256, 0, st->s>>>(V + (long long)v0 * ldv, ldv, nv, d_coef + v0, w, n);
-        LAUNCH_CHECK();
-    }
-    if (d_dots2) multidot(st, V, ldv, nvec, w, n, d_dots2);
-    if (d_nrm2) dot(st, w, w, n, d_nrm2);
-}
-
 /* ---- fused Gram-Schmidt pass -------------------------------------------------------------------
  *  HBM-bound: one streaming read of nvec basis vectors (+ one read / optional write of w) per pass.  Each thread keeps
  *  its basis elements in registers between the update and the dot products, so the "reorthogonalise and measure" step
@@ -980,6 +897,8 @@ void gs_pass(Stream* st, const double* V, long long ldv, int nvec, double* w, lo
 #undef GS_LAUNCH
     LAUNCH_CHECK();
 }
+/* w = y is only read: gs_pass writes w only when it is given coefficients */
+void dot(Stream* st, const double* x, const double* y, long long n, double* d_out) { gs_pass(st, x, n, 1, const_cast<double*>(y), n, nullptr, d_out, nullptr); }
 
 template <int NV>
 __global__ void __launch_bounds__(256) gs_final_kernel(const double* __restrict__ V, long long ldv, int nvec, const double* __restrict__ w, long long n,
@@ -1066,15 +985,6 @@ void ritz_rotate(Stream* st, double* V, long long ldv, long long n, int ncv, con
     if (ncv > RITZ_MAX) throw std::runtime_error("ritz_rotate: ncv too large");
     const int blocks = (int)std::max<long long>(1, std::min<long long>((n + 255) / 256, RED_BLOCKS));
     ritz_rotate_kernel<<<blocks, 256, sizeof(double) * ncv * kk, st->s>>>(V, ldv, n, ncv, d_S, kk);
-    LAUNCH_CHECK();
-}
-
-__global__ void scal_kernel(double* x, long long n, double a) {
-    for (long long q = blockIdx.x * (long long)blockDim.x + threadIdx.x; q < n; q += (long long)gridDim.x * blockDim.x) x[q] *= a;
-}
-void scal(Stream* st, double* x, long long n, double a) {
-    const int blocks = (int)std::max<long long>(1, std::min<long long>((n + 255) / 256, RED_BLOCKS));
-    scal_kernel<<<blocks, 256, 0, st->s>>>(x, n, a);
     LAUNCH_CHECK();
 }
 
@@ -1178,8 +1088,6 @@ int comm_init(Stream* st, int rank, int world, const void* idbytes) {
     st->rank = rank; st->world = world;
     return 0;
 }
-int comm_rank(Stream* st) { return st->rank; }
-int comm_world(Stream* st) { return st->world; }
 void allreduce_sum(Stream* st, double* d_buf, long long n) {
     if (st->world <= 1 || n <= 0) return;
     NCCL_OK(nccl().AllReduce(d_buf, d_buf, (size_t)n, ncclDouble, ncclSum, st->comm, st->s));
@@ -1351,7 +1259,6 @@ struct EigJob {
     double* outW;    /* n */
     double* norm2;   /* squared Frobenius norm */
     int* active;     /* any rotation since the flag was last cleared */
-    double* maxoff;  /* largest off-diagonal weight of a sub-problem since last cleared (diagnostics, DMRGX_TRACE) */
     int n, np, nb, pad;
 };
 
@@ -1366,12 +1273,11 @@ __device__ __forceinline__ void eig_pair(int nb, int r, int k, int& I, int& J) {
    the previous step, already ordered by weight) x (site states), so the diagonal of rho is informative and the sorted matrix
    starts out graded — the form on which the sorted block Jacobi converges fastest.  perm[i] = original coordinate at position i
    (the rank array of the finish step doubles as scratch for it). */
-__global__ void __launch_bounds__(256) eig_perm_kernel(const EigJob* __restrict__ jobs, int* __restrict__ perm_ws, const int* __restrict__ perm_off, int presort) {
+__global__ void __launch_bounds__(256) eig_perm_kernel(const EigJob* __restrict__ jobs, int* __restrict__ perm_ws, const int* __restrict__ perm_off) {
     const EigJob jb = jobs[blockIdx.y];
     int* perm = perm_ws + perm_off[blockIdx.y];
     const int n = jb.n;
     for (int i = blockIdx.x * 256 + threadIdx.x; i < n; i += gridDim.x * 256) {
-        if (!presort) { perm[i] = i; continue; }
         const double di = jb.outA[(long long)i * n + i];
         int rk = 0;
         for (int j = 0; j < n; ++j) { const double dj = jb.outA[(long long)j * n + j]; rk += (dj > di || (dj == di && j < i)) ? 1 : 0; }
@@ -1401,7 +1307,7 @@ __global__ void __launch_bounds__(1024) eig_norm_kernel(const EigJob* __restrict
     __syncthreads();
     if (threadIdx.x < 32) {
         s = warp_sum(red[threadIdx.x]);
-        if (threadIdx.x == 0) { *jb.norm2 = s; *jb.maxoff = 0.0; *jb.active = 0; }
+        if (threadIdx.x == 0) { *jb.norm2 = s; *jb.active = 0; }
     }
 }
 
@@ -1414,8 +1320,10 @@ __device__ __forceinline__ int eig_find(const int* __restrict__ prefix, int njob
 }
 
 constexpr int ESUB_THREADS = 1024; /* the sub-problem is latency-bound (three barriers per rotation round): all the threads an SM has */
-__global__ void __launch_bounds__(ESUB_THREADS) eig_sub_kernel(const EigJob* __restrict__ jobs, const int* __restrict__ prefix, int njobs, int round, int max_inner,
-                                                               int pattern, double adapt) {
+/* one CTA per SM, stated: with it the compiler spends the 64 registers a thread has on keeping the rotation rounds'
+   thread-invariant shared-memory addresses instead of recomputing them from threadIdx every round (without it: 48
+   registers, and tools/eig_probe.py 2048 solves 5 % slower on a B200 at 1000 W) */
+__global__ void __launch_bounds__(ESUB_THREADS, 1) eig_sub_kernel(const EigJob* __restrict__ jobs, const int* __restrict__ prefix, int njobs, int round, bool first) {
     extern __shared__ double jsm[];
     double* A = jsm;                 /* [64][65] */
     double* V = jsm + ET * JAC_LD;   /* rotation, columns = eigenvectors */
@@ -1440,8 +1348,7 @@ __global__ void __launch_bounds__(ESUB_THREADS) eig_sub_kernel(const EigJob* __r
        Rayleigh quotients with the original matrix, which squares this error. */
     const double thr = 1e-27 * *jb.norm2;
     bool rotated = false;
-    double off_entry = 0.0;
-    for (int sweep = 0; sweep < max_inner; ++sweep) {
+    for (int sweep = 0; sweep < 2; ++sweep) {
         double off = 0.0, offw = 0.0; /* off-diagonal weight: all of it / the part inside the two diagonal blocks */
         for (int e = tid; e < ET * ET; e += ESUB_THREADS) {
             const int i = e >> 6, j = e & 63;
@@ -1453,13 +1360,13 @@ __global__ void __launch_bounds__(ESUB_THREADS) eig_sub_kernel(const EigJob* __r
         __syncthreads();
         if (tid == 0) { double o = 0, ow = 0; for (int w = 0; w < ESUB_THREADS / 32; ++w) { o += red[w]; ow += redw[w]; } offsh = o; offwsh = ow; }
         __syncthreads();
-        if (sweep == 0) off_entry = offsh;
         if (offsh <= thr) break;
         rotated = true;
-        /* inner sweep `sweep` is a FULL cyclic sweep (63 rounds: all 2016 pairs) when bit `sweep` of `pattern` is set, else a
+        /* two inner sweeps: FULL cyclic sweeps (63 rounds: all 2016 pairs) in the first outer sweep of the solve; after it a
            CROSS sweep (32 rounds: the 1024 pairs (p in block I, q in block J) only — where the off-diagonal weight sits once
-           both diagonal blocks have been diagonalised by an earlier visit) */
-        const bool full = ((pattern >> sweep) & 1) && offwsh > adapt * offsh;
+           both diagonal blocks have been diagonalised by an earlier visit), then a full one.  A sweep that finds no weight
+           left inside the two diagonal blocks is a cross sweep. */
+        const bool full = (first || sweep == 1) && offwsh > 0.0;
         const int nrounds = full ? ET - 1 : EB;
         for (int rr = 0; rr < nrounds; ++rr) {
             if (tid < ET / 2) {
@@ -1541,7 +1448,6 @@ __global__ void __launch_bounds__(ESUB_THREADS) eig_sub_kernel(const EigJob* __r
     __syncthreads();
     const bool changed = rotated || moved;
     if (tid == 0) { jb.rot[k] = changed ? 1 : 0; if (rotated) *jb.active = 1; }
-    if (tid == 0 && rotated) atomicMax((unsigned long long*)jb.maxoff, (unsigned long long)__double_as_longlong(off_entry));
     if (!changed) return;
     double* Q = jb.Q + (long long)k * ET * ET;
     for (int e = tid; e < ET * ET; e += ESUB_THREADS) {
@@ -1771,7 +1677,7 @@ int syevd_batch(Stream* st, int nblocks, const int* n, double* const* d_A, doubl
             jb.A = pd; pd += (size_t)jb.np * jb.np;
             jb.VT = pd; pd += (size_t)jb.np * jb.np;
             jb.Q = pd; pd += (size_t)(jb.nb / 2) * ET * ET;
-            jb.norm2 = pd; jb.maxoff = pd + 1; pd += 2;
+            jb.norm2 = pd; pd += 2; /* one used: every piece stays a multiple of 2 doubles */
             lam_off[(size_t)q] = pd - wd; pd += jb.np;
             jb.rot = pi; pi += jb.nb / 2;
             jb.active = pi; pi += 2;
@@ -1788,23 +1694,11 @@ int syevd_batch(Stream* st, int nblocks, const int* n, double* const* d_A, doubl
     eig_norm_kernel<<<nj, 1024, 0, st->s>>>(d_jobs);
     LAUNCH_CHECK();
     CUDA_OK(cudaMemcpyAsync(d_tab, rank_off.data(), (size_t)nj * 4, cudaMemcpyHostToDevice, st->s));
-    eig_perm_kernel<<<dim3(4, nj), 256, 0, st->s>>>(d_jobs, wi, d_tab, getenv("DMRGX_JAC_NO_PRESORT") ? 0 : 1); /* (experiment hook) */
+    eig_perm_kernel<<<dim3(4, nj), 256, 0, st->s>>>(d_jobs, wi, d_tab);
     LAUNCH_CHECK();
     eig_init_kernel<<<dim3(64, nj), 256, 0, st->s>>>(d_jobs, wi, d_tab);
     LAUNCH_CHECK();
     CUDA_OK(cudaStreamSynchronize(st->s)); /* d_tab is reused for the prefix tables below */
-    /* inner cyclic sweeps per sub-problem: two while the matrix is far from diagonal, one once the sweeps are in their
-       convergent phase (tunable for experiments) */
-    static const int max_inner = getenv("DMRGX_JAC_INNER") ? atoi(getenv("DMRGX_JAC_INNER")) : 2;
-    static const int late_inner = getenv("DMRGX_JAC_INNER_LATE") ? atoi(getenv("DMRGX_JAC_INNER_LATE")) : 2;
-    static const int late_from = getenv("DMRGX_JAC_LATE_FROM") ? atoi(getenv("DMRGX_JAC_LATE_FROM")) : 6;
-    /* bit i: inner sweep i is a full cyclic sweep (else cross pairs only); first sweep of the solve / later sweeps */
-    static const int pattern_first = getenv("DMRGX_JAC_PATTERN_FIRST") ? atoi(getenv("DMRGX_JAC_PATTERN_FIRST")) : 3;
-    /* a full sweep is replaced by a cross sweep while the weight inside the diagonal blocks is below this fraction of the sub-problem's
-       off-diagonal weight (0: never) */
-    static const double adapt = getenv("DMRGX_JAC_ADAPT") ? atof(getenv("DMRGX_JAC_ADAPT")) : 0.0;
-    static const int pattern_alt = getenv("DMRGX_JAC_PATTERN_ALT") ? atoi(getenv("DMRGX_JAC_PATTERN_ALT")) : 2; /* even sweeps (experiments) */
-    static const int pattern_rest = getenv("DMRGX_JAC_PATTERN") ? atoi(getenv("DMRGX_JAC_PATTERN")) : 2; /* cross, then full: the sweep count of (full, full) at 3/4 of its rounds */
     int sweeps_done = 0;
     /* live jobs are a prefix-compacted copy of the job list (largest first); tables re-uploaded when a matrix finishes */
     std::vector<int> live((size_t)nj);
@@ -1835,8 +1729,7 @@ int syevd_batch(Stream* st, int nblocks, const int* n, double* const* d_A, doubl
         CUDA_OK(cudaStreamSynchronize(st->s)); /* host tables are reused below */
         /* one sweep of the largest live matrix (smaller ones complete at least one sweep of their own in the same rounds) */
         for (int rr = 0; rr < maxnb - 1; ++rr, ++round) {
-            eig_sub_kernel<<<sub_prefix[nl], ESUB_THREADS, sub_smem, st->s>>>(d_live, d_tab, nl, round, sweeps_done >= late_from ? late_inner : max_inner,
-                                                                                   sweeps_done == 0 ? pattern_first : ((sweeps_done & 1) ? pattern_rest : pattern_alt), adapt);
+            eig_sub_kernel<<<sub_prefix[nl], ESUB_THREADS, sub_smem, st->s>>>(d_live, d_tab, nl, round, sweeps_done == 0);
             LAUNCH_CHECK();
             eig_apply_kernel<<<app_prefix[nl], 128, app_smem, st->s>>>(d_live, d_tab + nl + 1, nl, round);
             LAUNCH_CHECK();
@@ -1845,12 +1738,6 @@ int syevd_batch(Stream* st, int nblocks, const int* n, double* const* d_A, doubl
         /* which matrices went through the whole sweep without a rotation? */
         for (int q = 0; q < nl; ++q) CUDA_OK(cudaMemcpyAsync(&h_active[(size_t)q], jobs[(size_t)live[(size_t)q]].active, 4, cudaMemcpyDeviceToHost, st->s));
         CUDA_OK(cudaStreamSynchronize(st->s));
-        if (getenv("DMRGX_TRACE")) {
-            double mo[2] = {0, 0};
-            cudaMemcpy(mo, jobs[(size_t)live[0]].norm2, 16, cudaMemcpyDeviceToHost);
-            cudaMemset(jobs[(size_t)live[0]].maxoff, 0, 8);
-            fprintf(stderr, "[trace] block Jacobi: round %d, %d live, largest n %d: max off(S)/||A|| %.3e\n", round, nl, jobs[(size_t)live[0]].n, sqrt(mo[1] / mo[0]));
-        }
         std::vector<int> next;
         for (int q = 0; q < nl; ++q) if (h_active[(size_t)q]) next.push_back(live[(size_t)q]);
         for (int q : next) CUDA_OK(cudaMemsetAsync(jobs[(size_t)q].active, 0, 4, st->s));
@@ -1907,7 +1794,5 @@ int syevd_batch(Stream* st, int nblocks, const int* n, double* const* d_A, doubl
     free_bytes(st, wd);
     return rc;
 }
-
-int syevd(Stream* st, int n, double* d_A, double* d_w) { return syevd_batch(st, 1, &n, &d_A, &d_w); }
 
 }  // namespace dev

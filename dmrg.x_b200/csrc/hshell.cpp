@@ -46,10 +46,6 @@ Kron* kron_create(const Block* L, const Block* R, const std::vector<double>& qn_
     return k.release();
 }
 
-HShell::~HShell() {
-    if (h_pinned) dev::free_pinned(h_pinned);
-}
-
 namespace {
 struct RightFactor { double coef; const Operator* B; };
 struct Group {
@@ -527,11 +523,9 @@ static HShell* build_shell(const Kron* kron, const std::vector<Group>& groups, i
            heavy ones (about one item per 40 full-tile chunks of work).  Parts of a cut chain go through the scratch buffer and
            the reduce pass, so more parts than needed to even out the last wave only add traffic: measured optima were 574 items
            at m = 512, 858 at m = 1024 and 2012 at m = 2048 (profiles/r1_chain_kernel.md). */
-        const char* tgt = getenv("DMRGX_STAGE2_WAVES"); /* experiment hook: fixed number of waves */
         const double chunks_total = probe.flops / (2.0 * 64 * 64 * 16);
-        const double target_items = tgt ? 444.0 * atof(tgt) : std::min(3.0 * 444.0, std::max(444.0, chunks_total / 40.0));
+        const double target_items = std::min(3.0 * 444.0, std::max(444.0, chunks_total / 40.0));
         if (probe.flops > 0 && (double)probe.items.size() < target_items) H->stage2.split_item_cost = 0.5 * probe.flops / target_items;
-        H->stage2.phase_order = getenv("DMRGX_NO_PHASE_ORDER") == nullptr;
     }
     for (int p = 0; p < np; ++p) {
         const int nLp = lr1[p] - lr0[p], nRp = SR.size[kron->pairs[p].ir];
@@ -623,18 +617,6 @@ static void plan_halo(HShell* H, const Kron* kron, const std::vector<Group>& gro
 
 static HShell* build_sharded(const Kron* kron, const std::vector<Group>& groups, int nterms) {
     Ctx* ctx = kron->ctx;
-    if (ctx->world <= 1 && getenv("DMRGX_FAKE_WORLD")) {
-        /* profiling hook: plan and run ONE rank's shard of a `world`-way split on a single GPU (ncu is single-GPU only); the rows
-           outside the shard are not computed */
-        const int fw = std::max(1, atoi(getenv("DMRGX_FAKE_WORLD"))), fr = std::min(fw - 1, std::max(0, getenv("DMRGX_FAKE_RANK") ? atoi(getenv("DMRGX_FAKE_RANK")) : 0));
-        long long gb = 0; double gf = 0;
-        const std::vector<long long> cuts = shard_rows(kron, groups, nterms, fw, gb, gf);
-        HShell* H = build_shell(kron, groups, nterms, cuts[(size_t)fr], cuts[(size_t)fr + 1]);
-        H->row_begin = 0; H->row_end = H->n; /* host-buffer entry points keep working on the whole vector */
-        H->row_cuts = {0, H->n};
-        H->alg_bytes_global = gb; H->alg_flops_global = gf;
-        return H;
-    }
     if (ctx->world <= 1) {
         HShell* H = build_shell(kron, groups, nterms);
         H->row_cuts = {0, H->n};
@@ -800,13 +782,11 @@ void hshell_apply(HShell* H, const double* d_x, double* d_y) {
 }
 
 /* The distributed form of the callback: x is a full-length buffer in which only this rank's rows are valid on entry;
-   the exchange step of the path (the VecScatter-to-all of src/DMRGKron.cpp:1833-1834) is an in-place all-gather over
-   NVLink, after which this rank computes its own rows of y. */
+   the exchange step of the path (the VecScatter-to-all of src/DMRGKron.cpp:1833-1834) is the sector-halo exchange over
+   NVLink, which brings this rank the rows of x its tiles read (plan_halo); then this rank computes its own rows of y. */
 void hshell_apply_sharded(HShell* H, double* d_x, double* d_y) {
-    if (H->ctx->world > 1) {
-        if (getenv("DMRGX_FULL_GATHER")) dev::allgatherv(H->ctx->st, d_x, H->row_cuts.data()); /* experiment hook: the reference's all-gather */
-        else dev::exchange_ranges(H->ctx->st, d_x, (int)H->halo_from.size(), H->halo_from.data(), H->halo_to.data(), H->halo_off.data(), H->halo_cnt.data());
-    }
+    if (H->ctx->world > 1)
+        dev::exchange_ranges(H->ctx->st, d_x, (int)H->halo_from.size(), H->halo_from.data(), H->halo_to.data(), H->halo_off.data(), H->halo_cnt.data());
     hshell_apply(H, d_x, d_y);
 }
 

@@ -38,7 +38,7 @@ void Plan::upload(Ctx* ctx) {
     }
     std::vector<size_t> ord(items.size());
     for (size_t i = 0; i < ord.size(); ++i) ord[i] = i;
-    const bool by_phase = phase_order && item_phase.size() == items.size();
+    const bool by_phase = item_phase.size() == items.size();
     std::stable_sort(ord.begin(), ord.end(), [&](size_t a, size_t b) {
         if (by_phase && item_phase[a] != item_phase[b]) return item_phase[a] < item_phase[b];
         return cost[a] > cost[b];

@@ -26,13 +26,9 @@ const char* last_error() { return g_err.c_str(); }
 long long launch_count() { return g_launches; }
 int init(int device, void*, Stream** out) { *out = new Stream{device}; return 0; }
 void destroy(Stream* s) { delete s; }
-int device_of(Stream* s) { return s->device; }
 void make_current(Stream*) {}
-void* raw_stream(Stream*) { return nullptr; }
 void* malloc_bytes(Stream*, size_t b) { return std::malloc(b ? b : 8); }
 void free_bytes(Stream*, void* p) { std::free(p); }
-void* malloc_pinned(size_t b) { return std::malloc(b ? b : 8); }
-void free_pinned(void* p) { std::free(p); }
 void h2d(Stream*, void* d, const void* s, size_t b) { if (b) std::memcpy(d, s, b); }
 void d2h(Stream*, void* d, const void* s, size_t b) { if (b) std::memcpy(d, s, b); }
 void d2d(Stream*, void* d, const void* s, size_t b) { if (b) std::memmove(d, s, b); }
@@ -132,16 +128,11 @@ void fill_random(Stream*, double* x, long long n, unsigned long long seed, long 
     ++g_launches;
     for (long long i = 0; i < n; ++i) x[i] = (double)(splitmix64(seed + (unsigned long long)(first + i) * 0x9E3779B97F4A7C15ULL) >> 11) / 9007199254740992.0 - 0.5;
 }
-void multidot(Stream*, const double* V, long long ldv, int nvec, const double* w, long long n, double* out) {
+void dot(Stream*, const double* x, const double* y, long long n, double* out) {
     ++g_launches;
-    for (int i = 0; i < nvec; ++i) { double s = 0; for (long long q = 0; q < n; ++q) s += V[i * ldv + q] * w[q]; out[i] = s; }
-}
-void dot(Stream* st, const double* x, const double* y, long long n, double* out) { multidot(st, x, n, 1, y, n, out); }
-void multiaxpy(Stream* st, const double* V, long long ldv, int nvec, const double* coef, double* w, long long n, double* dots2, double* nrm2) {
-    ++g_launches;
-    for (int i = 0; i < nvec; ++i) for (long long q = 0; q < n; ++q) w[q] -= coef[i] * V[i * ldv + q];
-    if (dots2) multidot(st, V, ldv, nvec, w, n, dots2);
-    if (nrm2) dot(st, w, w, n, nrm2);
+    double s = 0;
+    for (long long q = 0; q < n; ++q) s += x[q] * y[q];
+    *out = s;
 }
 void gs_pass(Stream*, const double* V, long long ldv, int nvec, double* w, long long n, const double* coef, double* dots, double* nrm2) {
     ++g_launches;
@@ -174,7 +165,6 @@ void ritz_rotate(Stream*, double* V, long long ldv, long long n, int ncv, const 
         for (int a = 0; a < kk; ++a) { double o = 0; for (int i = 0; i < ncv; ++i) o += S[i * kk + a] * v[i]; V[a * ldv + q] = o; }
     }
 }
-void scal(Stream*, double* x, long long n, double a) { ++g_launches; for (long long q = 0; q < n; ++q) x[q] *= a; }
 void filter_small(Stream*, double* x, long long n, double tol) { ++g_launches; for (long long q = 0; q < n; ++q) if (std::fabs(x[q]) < tol) x[q] = 0.0; }
 void axpby_out(Stream*, const double* a, const double* b, double alpha, double* out, long long n) {
     ++g_launches;
@@ -185,7 +175,7 @@ void gather_rows_reversed(Stream*, const double* src, int n, int m, double* dst)
     for (int k = 0; k < m; ++k) std::memcpy(dst + (size_t)k * n, src + (size_t)(n - 1 - k) * n, sizeof(double) * n);
 }
 /* cyclic Jacobi; row k of A on exit = k-th eigenvector, ascending eigenvalues */
-int syevd(Stream*, int n, double* A, double* w) {
+static void jacobi(int n, double* A, double* w) {
     ++g_launches;
     std::vector<double> V((size_t)n * n, 0.0);
     for (int i = 0; i < n; ++i) V[(size_t)i * n + i] = 1.0;
@@ -211,12 +201,11 @@ int syevd(Stream*, int n, double* A, double* w) {
     for (int i = 0; i < n; ++i) d[i] = a(i, i);
     std::stable_sort(ord.begin(), ord.end(), [&](int x, int y) { return d[x] < d[y]; });
     for (int k = 0; k < n; ++k) { w[k] = d[ord[k]]; for (int i = 0; i < n; ++i) A[(size_t)k * n + i] = V[(size_t)i * n + ord[k]]; }
-    return 0;
 }
 
-int syevd_batch(Stream* st, int nblocks, const int* n, double* const* A, double* const* w) {
+int syevd_batch(Stream*, int nblocks, const int* n, double* const* A, double* const* w) {
     for (int b = 0; b < nblocks; ++b)
-        if (n[b] > 0) { int e = syevd(st, n[b], A[b], w[b]); if (e) return e; }
+        if (n[b] > 0) jacobi(n[b], A[b], w[b]);
     return 0;
 }
 
@@ -229,8 +218,6 @@ static bcast_cb_t g_bcast = nullptr;
 static int g_rank = 0, g_world = 1;
 int comm_unique_id(void* out) { std::memset(out, 0, COMM_ID_BYTES); return 0; }
 int comm_init(Stream*, int rank, int world, const void*) { g_rank = rank; g_world = world; return 0; }
-int comm_rank(Stream*) { return g_rank; }
-int comm_world(Stream*) { return g_world; }
 void allreduce_sum(Stream*, double* buf, long long n) { if (g_world > 1 && n > 0) g_allreduce(buf, n); }
 void allgatherv(Stream*, double* buf, const long long* off) {
     if (g_world <= 1) return;
