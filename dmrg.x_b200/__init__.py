@@ -314,6 +314,21 @@ class KronBlocks:
         """KronConstruct(Mat_L, OpType_L, Mat_R, OpType_R, MatOut) — include/DMRGKron.hpp:309"""
         return HShell(self, single=(op_left, isite_left, op_right, isite_right))
 
+    def CorrelationMatrix(self, psi):
+        """EXTENSION (dmrgx_corr_matrix): every two-point spin correlator of psi (a DeviceVector of this superblock) in one
+        batched device pass.  Returns a dict of numpy arrays over the superblock sites (site s < nL: left-block site s, else
+        right-block site nL+nR-1-s): SzSz, SpSm, SmSp (n×n, entry [i, j] = <psi| O_i O'_j |psi>), Sz (n), and the algorithmic
+        flops of the call."""
+        n = self.left.NumSites() + self.right.NumSites()
+        out = {k: np.zeros((n, n)) for k in ("SzSz", "SpSm", "SmSp")}
+        sz = np.zeros(n)
+        fl = C.c_double()
+        _chk(lib().dmrgx_corr_matrix(self.h, psi.ptr if psi is not None else None, _p(out["SzSz"]), _p(out["SpSm"]), _p(out["SmSp"]), _p(sz),
+                                     C.byref(fl)))
+        out["Sz"] = sz
+        out["flops"] = fl.value
+        return out
+
 
 class HShell:
     """The matrix-free superblock Hamiltonian (MATSHELL with MatMult_KronSumShell)."""

@@ -345,6 +345,10 @@ int dmrgx_expect(dmrgx_hshell h1, const double* d_psi, double* value) {
     });
 }
 
+int dmrgx_corr_matrix(dmrgx_kron k, const double* d_psi, double* szsz, double* spsm, double* smsp, double* sz, double* flops) {
+    return guard([&] { corr_matrix(K(k), d_psi, szsz, spsm, smsp, sz, flops); });
+}
+
 /* microbenchmark of the chain engine on one plain product C[M,N] = A·B (selectable operand layouts), for profiling */
 int dmrgx_selftest_gemm(dmrgx_ctx cx, dmrgx_int M, dmrgx_int N, dmrgx_int K, int a_k_contig, int b_k_contig, int nseg, int reps, double* ms,
                         double* max_err) {

@@ -246,4 +246,7 @@ Block* rotate(const Block* enl, const XForm* xf);
 Wave* wave_create(const Kron*, const double* d_psi, const XForm* grown_side, bool grow_left);
 bool wave_apply(const Wave*, const XForm* shrinking_side, const Block* site, const Kron* new_kron, double* d_psi_new);
 
+/* corr.cpp: all two-point spin correlators of the superblock (extension; host n×n outputs, n = sites of both blocks) */
+void corr_matrix(const Kron*, const double* d_psi, double* szsz, double* spsm, double* smsp, double* sz, double* flops);
+
 }  // namespace dmrgx

@@ -161,6 +161,11 @@ void scale_inv_norm(Stream*, const double* w, const double* d_nrm2, double* v, l
 void ritz_rotate(Stream*, double* V, long long ldv, long long n, int ncv, const double* d_S, int kk);
 /* *d_out = x·y (the reduction of gs_pass: one launch, fixed summation order) */
 void dot(Stream*, const double* x, const double* y, long long n, double* d_out);
+/* Gram matrix of a column panel: d_G = PᵀP, row-major np×np and exactly symmetric, over rows [0,n) of the columns
+   P + c·ldp (c < np).  P must be 16-byte aligned and ldp even.  FP64 DMMA on the 32×32 tiles on or above the diagonal;
+   the rows are cut into fixed slabs whose partial tiles are summed in a fixed order (no atomics: two calls on the same
+   data give the same bits), then mirrored.  Two launches. */
+void gram(Stream*, const double* P, long long ldp, int np, long long n, double* d_G);
 
 /* dense symmetric eigendecomposition of a batch of independent blocks, in place: block b is n[b]×n[b] at d_A[b]; on exit
    row k of it (row-major) is the k-th eigenvector, eigenvalues ascending in d_w[b].  Blocks of up to 64 states are solved by

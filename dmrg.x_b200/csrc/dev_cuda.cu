@@ -68,6 +68,7 @@ struct Stream {
     int rank = 0, world = 1;
     int spmm_smem = 0;           /* dynamic shared memory spmm_kernel has been configured for on this device */
     bool chain_cfg = false;      /* chain_kernel's dynamic shared memory attribute has been set on this device */
+    bool gram_cfg = false;       /* the same for gram_kernel */
     cudaStream_t aux = nullptr;  /* side stream: the small-block eigensolver runs beside the block-Jacobi launches */
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
 };
@@ -899,6 +900,143 @@ void gs_pass(Stream* st, const double* V, long long ldv, int nvec, double* w, lo
 }
 /* w = y is only read: gs_pass writes w only when it is given coefficients */
 void dot(Stream* st, const double* x, const double* y, long long n, double* d_out) { gs_pass(st, x, n, 1, const_cast<double*>(y), n, nullptr, d_out, nullptr); }
+
+/* ================================================================================================
+ *  gram_kernel — G = PᵀP of a panel of np long columns (the correlation matrix, corr.cpp).  One CTA per (32×32 tile on or
+ *  above the diagonal, slab of GR_SLAB rows).  Chunks of 64 rows of the tile's 32 + 32 columns are staged with 16-byte
+ *  cp.async into a two-stage ring (a diagonal tile stages its columns once and reads them as both operands); warp w
+ *  multiplies rows [16w, 16w+16) of every chunk into a full 32×32 DMMA accumulator (4×4 fragments), and the four warp
+ *  partials are summed in shared memory in warp order.  The slab partial is written to a scratch area; gram_reduce_kernel
+ *  sums the slabs in index order and writes both G[i][j] and G[j][i] from the same sum.  The columns are contiguous, so
+ *  the arithmetic intensity is set by the tile width: about 4 flop per byte staged, ~np/4 per byte of DRAM traffic.
+ * ============================================================================================== */
+constexpr int GR_T = 32, GR_BK = 64, GR_S = GR_BK + 4 /* ≡ 4 mod 16: conflict-free fragment reads */, GR_THREADS = 128;
+constexpr long long GR_SLAB = 8192;
+constexpr int GR_STAGE = 2 * GR_T * GR_S; /* doubles of one stage: A and B columns */
+
+__device__ __forceinline__ void cp_async16(double* smem_dst, const double* gsrc, int src_bytes) {
+    unsigned s = (unsigned)__cvta_generic_to_shared(smem_dst);
+    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(s), "l"(gsrc), "r"(src_bytes));
+}
+
+__global__ void __launch_bounds__(GR_THREADS) gram_kernel(const double* __restrict__ P, long long ldp, int np, long long n, int nt, int ntri,
+                                                          double* __restrict__ part) {
+    extern __shared__ __align__(16) double gr_smem[];
+    const int tri = blockIdx.x % ntri, slab = blockIdx.x / ntri;
+    int ti = 0, r = tri;
+    while (r >= nt - ti) { r -= nt - ti; ++ti; }
+    const int tj = ti + r;
+    const bool diag = ti == tj;
+    const long long r0 = (long long)slab * GR_SLAB, r1 = min(n, r0 + GR_SLAB);
+    const int nchunks = (int)((r1 - r0 + GR_BK - 1) / GR_BK);
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
+
+    /* this thread's eight 16-byte copies per operand: column q >> 5 of the tile, rows 2(q & 31), +1 of the chunk; columns past
+       np are clamped to the last one (they only reach accumulator rows / columns that are never stored) */
+    const double* srcA[8];
+    const double* srcB[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+        const int q = tid + GR_THREADS * i, col = q >> 5, pr = q & 31;
+        srcA[i] = P + (long long)min(ti * GR_T + col, np - 1) * ldp + r0 + 2 * pr;
+        srcB[i] = P + (long long)min(tj * GR_T + col, np - 1) * ldp + r0 + 2 * pr;
+    }
+    auto issue = [&](int c) {
+        double* as = gr_smem + (c & 1) * GR_STAGE;
+        double* bs = as + GR_T * GR_S;
+        const long long row0 = r0 + (long long)c * GR_BK;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+            const int q = tid + GR_THREADS * i, col = q >> 5, pr = q & 31;
+            /* rows past the slab are zero-filled: a partial copy reads only the row that belongs to it */
+            const long long left = r1 - (row0 + 2 * pr);
+            const int bytes = left >= 2 ? 16 : (left == 1 ? 8 : 0);
+            const long long adv = (long long)c * GR_BK;
+            cp_async16(as + col * GR_S + 2 * pr, bytes ? srcA[i] + adv : P, bytes);
+            if (!diag) cp_async16(bs + col * GR_S + 2 * pr, bytes ? srcB[i] + adv : P, bytes);
+        }
+    };
+
+    double acc[4][4][2];
+#pragma unroll
+    for (int mi = 0; mi < 4; ++mi)
+#pragma unroll
+        for (int ni = 0; ni < 4; ++ni) { acc[mi][ni][0] = 0.0; acc[mi][ni][1] = 0.0; }
+
+    if (nchunks > 0) issue(0);
+    cp_async_commit();
+    for (int c = 0; c < nchunks; ++c) {
+        if (c + 1 < nchunks) issue(c + 1);
+        cp_async_commit();
+        cp_async_wait<1>();
+        __syncthreads();
+        const double* as = gr_smem + (c & 1) * GR_STAGE;
+        const double* bs = diag ? as : as + GR_T * GR_S;
+        const int kb = warp * 16 + t;
+#pragma unroll
+        for (int kk = 0; kk < 4; ++kk) {
+            double a[4], b[4];
+#pragma unroll
+            for (int mi = 0; mi < 4; ++mi) a[mi] = as[(mi * 8 + g) * GR_S + kb + 4 * kk];
+#pragma unroll
+            for (int ni = 0; ni < 4; ++ni) b[ni] = bs[(ni * 8 + g) * GR_S + kb + 4 * kk];
+#pragma unroll
+            for (int ni = 0; ni < 4; ++ni)
+#pragma unroll
+                for (int mi = 0; mi < 4; ++mi) dmma_m8n8k4(acc[mi][ni][0], acc[mi][ni][1], a[mi], b[ni]);
+        }
+        __syncthreads();
+    }
+    cp_async_wait<0>();
+    __syncthreads();
+    /* the four warp partials, summed in warp order */
+    double* red = gr_smem;
+#pragma unroll
+    for (int mi = 0; mi < 4; ++mi)
+#pragma unroll
+        for (int ni = 0; ni < 4; ++ni) {
+            double* p = red + warp * GR_T * GR_T + (mi * 8 + g) * GR_T + ni * 8 + 2 * t;
+            p[0] = acc[mi][ni][0];
+            p[1] = acc[mi][ni][1];
+        }
+    __syncthreads();
+    double* out = part + ((long long)slab * ntri + tri) * (GR_T * GR_T);
+    for (int e = tid; e < GR_T * GR_T; e += GR_THREADS)
+        out[e] = ((red[e] + red[GR_T * GR_T + e]) + red[2 * GR_T * GR_T + e]) + red[3 * GR_T * GR_T + e];
+}
+
+__global__ void __launch_bounds__(256) gram_reduce_kernel(const double* __restrict__ part, int np, int nt, int ntri, int nslabs, double* __restrict__ G) {
+    const long long e = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (e >= (long long)np * np) return;
+    int i = (int)(e / np), j = (int)(e % np);
+    if (i > j) { const int s = i; i = j; j = s; }
+    const int ti = i / GR_T, tj = j / GR_T;
+    const int tri = ti * nt - ti * (ti - 1) / 2 + (tj - ti);
+    const double* p = part + (long long)tri * (GR_T * GR_T) + (i % GR_T) * GR_T + (j % GR_T);
+    double s = 0.0;
+    for (int k = 0; k < nslabs; ++k) s += p[(long long)k * ntri * (GR_T * GR_T)];
+    G[e] = s;
+}
+
+void gram(Stream* st, const double* P, long long ldp, int np, long long n, double* d_G) {
+    if (np <= 0) return;
+    if (n <= 0) { memset0(st, d_G, sizeof(double) * np * np); return; }
+    if ((ldp & 1) || ((uintptr_t)P & 15)) throw std::runtime_error("gram: columns must be 16-byte aligned (P aligned, ldp even)");
+    const int nt = (np + GR_T - 1) / GR_T, ntri = nt * (nt + 1) / 2;
+    const long long nslabs = (n + GR_SLAB - 1) / GR_SLAB;
+    constexpr int smem = 2 * GR_STAGE * (int)sizeof(double);
+    static_assert(4 * GR_T * GR_T <= 2 * GR_STAGE, "the warp partials reuse the staging buffers");
+    if (!st->gram_cfg) {
+        CUDA_OK(cudaFuncSetAttribute(gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        st->gram_cfg = true;
+    }
+    double* part = (double*)malloc_bytes(st, sizeof(double) * nslabs * ntri * GR_T * GR_T);
+    gram_kernel<<<(unsigned)(nslabs * ntri), GR_THREADS, smem, st->s>>>(P, ldp, np, n, nt, ntri, part);
+    LAUNCH_CHECK();
+    gram_reduce_kernel<<<(unsigned)(((long long)np * np + 255) / 256), 256, 0, st->s>>>(part, np, nt, ntri, (int)nslabs, d_G);
+    LAUNCH_CHECK();
+    free_bytes(st, part); /* stream-ordered heap: the next user of the range is queued behind the reduction */
+}
 
 template <int NV>
 __global__ void __launch_bounds__(256) gs_final_kernel(const double* __restrict__ V, long long ldv, int nvec, const double* __restrict__ w, long long n,

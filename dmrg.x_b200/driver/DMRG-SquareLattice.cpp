@@ -1,9 +1,9 @@
 /*  DMRG-SquareLattice — the reference's executable (src/DMRG-SquareLattice.cpp:16-181) over the B200 path.
  *
  *      DMRG-SquareLattice.x -Lx 12 -Ly 6 -J1 0.5 -Jz1 1 -J2 0.25 -Jz2 0.5 -mwarmup 128 -msweeps 512,1024,2048 \
- *                           [-H_eps_tol 1e-12] [-data_dir out/] [-device 0] [-verbose] [-wavefunction_prediction 1]
+ *                           [-H_eps_tol 1e-12] [-data_dir out/] [-device 0] [-verbose] [-wavefunction_prediction 1] [-do_correlation_matrix 1]
  *
- *  Same options (plus -device and the opt-in -wavefunction_prediction, which the reference does not have), same stdout banner, same JSON files; one process drives one B200 through the C ABI
+ *  Same options (plus -device and the opt-in -wavefunction_prediction and -do_correlation_matrix, which the reference does not have), same stdout banner, same JSON files; one process drives one B200 through the C ABI
  *  (include/dmrgx.h).  There is no CPU path: without a CUDA device the context creation fails and the
  *  program exits non-zero.
  */

@@ -133,6 +133,16 @@ public:
         fp_data = fopen((data_dir + "DMRGRun.json").c_str(), "w");
         fp_corr = fopen((data_dir + "Correlations.json").c_str(), "w");
         if (!fp_step || !fp_timings || !fp_entanglement || !fp_data || !fp_corr) SETERRQ1(mpi_comm, 1, "cannot open output files in %s", data_dir.c_str());
+        /* EXTENSION, off by default: the full two-point spin correlation matrix and the structure factor at every measurement
+           step, in CorrelationMatrix.json; computed and written by rank 0 only */
+        o.GetBool("-do_correlation_matrix", &do_corr_matrix, NULL);
+        { int rank = 0, world = 1; dmrgx_ctx_rank(DmrgxContext(), &rank, &world); if (rank != 0) do_corr_matrix = PETSC_FALSE; }
+        if (do_corr_matrix) {
+            fp_corrmat = fopen((data_dir + "CorrelationMatrix.json").c_str(), "w");
+            if (!fp_corrmat) SETERRQ1(mpi_comm, 1, "cannot open %sCorrelationMatrix.json", data_dir.c_str());
+            fprintf(fp_corrmat, "[\n");
+            fflush(fp_corrmat);
+        }
         SaveStepHeaders(); fprintf(fp_step, "[\n");
         SaveTimingsHeaders(); fprintf(fp_timings, "[\n");
         fprintf(fp_entanglement, "[\n");
@@ -195,6 +205,7 @@ public:
         fprintf(fp_data, "\n}\n"); fclose(fp_data);
         if (corr_headers_printed) fprintf(fp_corr, "\n  ]\n}\n");
         fclose(fp_corr);
+        if (fp_corrmat) { fprintf(fp_corrmat, "\n]\n"); fclose(fp_corrmat); fp_corrmat = NULL; }
         init = PETSC_FALSE;
         return 0;
     }
@@ -490,6 +501,7 @@ private:
         ierr = BT_R.Load(); CHKERRQ(ierr);
         ierr = SaveEntanglementSpectra(BT_L, SysBlockEnl.Magnetization.List(), BT_R, EnvBlockEnl.Magnetization.List()); CHKERRQ(ierr);
         ierr = CalculateCorrelations_BlockDiag(KronBlocks, gsv_r, do_measurements); CHKERRQ(ierr);
+        if (do_measurements && do_corr_matrix) { ierr = CalculateCorrelationMatrix(KronBlocks, gsv_r, NumSitesTotal); CHKERRQ(ierr); }
         if (do_prediction) {
             /* both candidates: which block grows in the next step is the caller's business (the left one in the first half of a sweep,
                the right one in the second, :996-1088); the transformations that created this step's input blocks are captured now,
@@ -582,6 +594,52 @@ private:
         for (size_t icorr = 0; icorr < measurements.size(); ++icorr) fprintf(fp_corr, "%s %g", icorr ? "," : "", CorrValues[icorr]);
         fprintf(fp_corr, " ]");
         fflush(fp_corr);
+        return 0;
+    }
+
+    /** EXTENSION (-do_correlation_matrix): one record of CorrelationMatrix.json — every <S_i S_j> of the superblock from
+        dmrgx_corr_matrix (superblock site s is lattice site s), and the static structure factor
+            S(q) = (1/N) Σ_ij cos(q·(r_i - r_j)) <S_i·S_j>,   <S_i·S_j> = SzSz + (SpSm + SmSp)/2,   q = (2π kx/Lx, 2π ky/Ly),
+        written as StructureFactor[kx][ky]. */
+    PetscErrorCode CalculateCorrelationMatrix(KronBlocks_t& KronBlocks, const Vec& gsv_r, const PetscInt nsites) {
+        const size_t n = (size_t)nsites;
+        std::vector<double> szsz(n * n), spsm(n * n), smsp(n * n), sz(n);
+        DMRGX_CALL(dmrgx_corr_matrix(KronBlocks.Handle(), gsv_r.d, szsz.data(), spsm.data(), smsp.data(), sz.data(), NULL));
+        const PetscInt Lx = Ham.Lx(), Ly = Ham.Ly();
+        std::vector<PetscInt> x(n), y(n);
+        for (size_t s = 0; s < n; ++s) Ham.To2D((PetscInt)s, x[s], y[s]);
+        FILE* f = fp_corrmat;
+        fprintf(f, "%s  {\n    \"GlobIdx\": %lld,\n    \"LoopIdx\": %lld,\n    \"sites\": [", corrmat_records ? ",\n" : "", LLD(GlobIdx), LLD(LoopIdx));
+        for (size_t s = 0; s < n; ++s) fprintf(f, "%s[%lld, %lld]", s ? ", " : "", LLD(x[s]), LLD(y[s]));
+        fprintf(f, "],\n    \"Sz\": [");
+        for (size_t s = 0; s < n; ++s) fprintf(f, "%s%.17g", s ? ", " : "", sz[s]);
+        fprintf(f, "]");
+        auto matrix = [&](const char* name, const std::vector<double>& m, size_t rows, size_t cols) {
+            fprintf(f, ",\n    \"%s\": [", name);
+            for (size_t i = 0; i < rows; ++i) {
+                fprintf(f, "%s\n      [", i ? "," : "");
+                for (size_t j = 0; j < cols; ++j) fprintf(f, "%s%.17g", j ? ", " : "", m[i * cols + j]);
+                fprintf(f, "]");
+            }
+            fprintf(f, "\n    ]");
+        };
+        matrix("SzSz", szsz, n, n);
+        matrix("SpSm", spsm, n, n);
+        matrix("SmSp", smsp, n, n);
+        std::vector<double> sq((size_t)(Lx * Ly), 0.0);
+        for (PetscInt kx = 0; kx < Lx; ++kx)
+            for (PetscInt ky = 0; ky < Ly; ++ky) {
+                const double qx = 2.0 * M_PI * (double)kx / (double)Lx, qy = 2.0 * M_PI * (double)ky / (double)Ly;
+                double s = 0;
+                for (size_t i = 0; i < n; ++i)
+                    for (size_t j = 0; j < n; ++j)
+                        s += std::cos(qx * (double)(x[i] - x[j]) + qy * (double)(y[i] - y[j])) * (szsz[i * n + j] + 0.5 * (spsm[i * n + j] + smsp[i * n + j]));
+                sq[(size_t)(kx * Ly + ky)] = s / (double)n;
+            }
+        matrix("StructureFactor", sq, (size_t)Lx, (size_t)Ly);
+        fprintf(f, "\n  }");
+        fflush(f);
+        ++corrmat_records;
         return 0;
     }
 
@@ -733,6 +791,9 @@ private:
     PetscInt LoopIdx = 0, StepIdx = 0;
     std::vector<Correlator> measurements;
     PetscBool corr_headers_printed = PETSC_FALSE, corr_printed_first = PETSC_FALSE;
+    PetscBool do_corr_matrix = PETSC_FALSE;   /* -do_correlation_matrix (extension) */
+    FILE* fp_corrmat = NULL;
+    long long corrmat_records = 0;
     PetscScalar gse = 0.0;
     std::vector<PetscReal> trunc_err;
     double t0abs = 0.0;

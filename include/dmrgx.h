@@ -185,6 +185,19 @@ int dmrgx_rotate(dmrgx_block enlarged, dmrgx_xform x, dmrgx_block* out);
 /* ---- correlator kernel: <psi| A⊗B |psi> = VecDot(psi, MatMult(H1, psi)), include/DMRGBlockContainer.hpp:2287-2296 ---- */
 int dmrgx_expect(dmrgx_hshell h1, const double* d_psi, double* value);
 
+/* ---- EXTENSION: the all-pairs spin correlation matrix (no reference counterpart: there every correlator is one
+   KronConstruct + MatMult + VecDot, include/DMRGBlockContainer.hpp:2262-2296).  For the n = nL + nR superblock sites
+   (site s < nL is left-block site s, site s >= nL is right-block site nL+nR-1-s, as in dmrgx_hshell_create) and psi in the
+   superblock's one total-Sz sector, used as given (not normalised):
+       szsz[i*n+j] = <psi| Sz_i Sz_j |psi>,  spsm[i*n+j] = <psi| S+_i S-_j |psi>,  smsp[i*n+j] = <psi| S-_i S+_j |psi>,
+       sz[i] = <psi| Sz_i |psi>
+   all host buffers (n×n row-major, n).  One batched device pass: per operator type the panels O_s·psi of every site are
+   built by one contraction launch and reduced to their Gram matrix by one FP64 tensor-core launch; the same-block entries
+   equal the operator products of dmrgx_hshell_create_product.  flops (may be NULL) receives the algorithmic flops of the
+   call.  On a multi-GPU context the calling rank computes everything from its complete psi, with no collective.
+   Errors: 62 psi or an output NULL, 56 the kron has not exactly one sector, 73 a block lacks Sz_i or Sp_i (site in the message). */
+int dmrgx_corr_matrix(dmrgx_kron k, const double* d_psi, double* szsz, double* spsm, double* smsp, double* sz, double* flops);
+
 /* ---- Hamiltonians::J1J2XXZModel_SquareLattice::H(nsites): src/Hamiltonians.cpp:73-122 (host only).
         Returns the number of terms (fills at most maxterms); bc: 0 open, 1 periodic; nsites < 0 = full lattice. ---- */
 dmrgx_int dmrgx_ham_terms(dmrgx_int Lx, dmrgx_int Ly, double J1, double Jz1, double J2, double Jz2, int bcx, int bcy, dmrgx_int nsites,
