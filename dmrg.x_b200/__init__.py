@@ -329,6 +329,19 @@ class KronBlocks:
         out["flops"] = fl.value
         return out
 
+    def DimerMatrix(self, psi, bonds):
+        """EXTENSION (dmrgx_dimer_matrix): every bond–bond correlator of psi over `bonds`, a sequence of (i, j) superblock-site
+        pairs, in one batched device pass, with D_a = Sz_i Sz_j + (S+_i S-_j + S-_i S+_j)/2 in the given order.  Returns
+        DD (nb×nb, entry [a, b] = <D_a psi, D_b psi>), D (nb, <psi| D_a |psi>) and the algorithmic flops of the call."""
+        b = _l(bonds).reshape(-1, 2) if len(bonds) else np.zeros((0, 2), np.int64)
+        si, sj = _l(b[:, 0]), _l(b[:, 1])
+        nb = len(b)
+        dd = np.zeros((nb, nb))
+        d = np.zeros(nb)
+        fl = C.c_double()
+        _chk(lib().dmrgx_dimer_matrix(self.h, psi.ptr if psi is not None else None, LL(nb), _p(si), _p(sj), _p(dd), _p(d), C.byref(fl)))
+        return {"DD": dd, "D": d, "flops": fl.value}
+
 
 class HShell:
     """The matrix-free superblock Hamiltonian (MATSHELL with MatMult_KronSumShell)."""

@@ -349,6 +349,11 @@ int dmrgx_corr_matrix(dmrgx_kron k, const double* d_psi, double* szsz, double* s
     return guard([&] { corr_matrix(K(k), d_psi, szsz, spsm, smsp, sz, flops); });
 }
 
+int dmrgx_dimer_matrix(dmrgx_kron k, const double* d_psi, dmrgx_int nbonds, const dmrgx_int* site_i, const dmrgx_int* site_j, double* dd,
+                       double* d, double* flops) {
+    return guard([&] { dimer_matrix(K(k), d_psi, nbonds, site_i, site_j, dd, d, flops); });
+}
+
 /* microbenchmark of the chain engine on one plain product C[M,N] = A·B (selectable operand layouts), for profiling */
 int dmrgx_selftest_gemm(dmrgx_ctx cx, dmrgx_int M, dmrgx_int N, dmrgx_int K, int a_k_contig, int b_k_contig, int nseg, int reps, double* ms,
                         double* max_err) {

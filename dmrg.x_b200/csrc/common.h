@@ -248,5 +248,8 @@ bool wave_apply(const Wave*, const XForm* shrinking_side, const Block* site, con
 
 /* corr.cpp: all two-point spin correlators of the superblock (extension; host n×n outputs, n = sites of both blocks) */
 void corr_matrix(const Kron*, const double* d_psi, double* szsz, double* spsm, double* smsp, double* sz, double* flops);
+/* corr.cpp: the bond–bond correlators of nb isotropic bonds (extension; host nb×nb and nb outputs) */
+void dimer_matrix(const Kron*, const double* d_psi, long long nb, const long long* bond_i, const long long* bond_j, double* dd, double* d,
+                  double* flops);
 
 }  // namespace dmrgx

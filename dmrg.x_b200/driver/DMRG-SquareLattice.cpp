@@ -2,12 +2,17 @@
  *
  *      DMRG-SquareLattice.x -Lx 12 -Ly 6 -J1 0.5 -Jz1 1 -J2 0.25 -Jz2 0.5 -mwarmup 128 -msweeps 512,1024,2048 \
  *                           [-H_eps_tol 1e-12] [-data_dir out/] [-device 0] [-verbose] [-wavefunction_prediction 1] [-do_correlation_matrix 1]
+ *                           [-do_dimer_matrix 1]
  *
- *  Same options (plus -device and the opt-in -wavefunction_prediction and -do_correlation_matrix, which the reference does not have), same stdout banner, same JSON files; one process drives one B200 through the C ABI
+ *  Same options (plus -device and the opt-in -wavefunction_prediction, -do_correlation_matrix and -do_dimer_matrix, which the reference does not have), same stdout banner, same JSON files; one process drives one B200 through the C ABI
  *  (include/dmrgx.h).  There is no CPU path: without a CUDA device the context creation fails and the
  *  program exits non-zero.
  */
-static char help[] = "DMRG executable for the Spin-1/2 J1-J2 XY Model on a two-dimensional square lattice (B200 path).\n";
+static char help[] = "DMRG executable for the Spin-1/2 J1-J2 XY Model on a two-dimensional square lattice (B200 path).\n"
+                     "Extensions, off by default, computed and written by rank 0 at every measurement step:\n"
+                     "  -do_correlation_matrix 1   every <S_i S_j> and the structure factor S(q) -> CorrelationMatrix.json\n"
+                     "  -do_dimer_matrix 1         <D_a>, <D_a D_b> over the nearest-neighbour bonds (D_a = S_i.S_j) and the\n"
+                     "                             dimer structure factors of the x and y bonds -> DimerMatrix.json\n";
 
 #include <unistd.h>
 

@@ -136,12 +136,21 @@ public:
         /* EXTENSION, off by default: the full two-point spin correlation matrix and the structure factor at every measurement
            step, in CorrelationMatrix.json; computed and written by rank 0 only */
         o.GetBool("-do_correlation_matrix", &do_corr_matrix, NULL);
-        { int rank = 0, world = 1; dmrgx_ctx_rank(DmrgxContext(), &rank, &world); if (rank != 0) do_corr_matrix = PETSC_FALSE; }
+        /* EXTENSION, off by default: the dimer (bond–bond) correlation matrix of the nearest-neighbour bonds and the dimer
+           structure factors at every measurement step, in DimerMatrix.json; computed and written by rank 0 only */
+        o.GetBool("-do_dimer_matrix", &do_dimer_matrix, NULL);
+        { int rank = 0, world = 1; dmrgx_ctx_rank(DmrgxContext(), &rank, &world); if (rank != 0) do_corr_matrix = do_dimer_matrix = PETSC_FALSE; }
         if (do_corr_matrix) {
             fp_corrmat = fopen((data_dir + "CorrelationMatrix.json").c_str(), "w");
             if (!fp_corrmat) SETERRQ1(mpi_comm, 1, "cannot open %sCorrelationMatrix.json", data_dir.c_str());
             fprintf(fp_corrmat, "[\n");
             fflush(fp_corrmat);
+        }
+        if (do_dimer_matrix) {
+            fp_dimer = fopen((data_dir + "DimerMatrix.json").c_str(), "w");
+            if (!fp_dimer) SETERRQ1(mpi_comm, 1, "cannot open %sDimerMatrix.json", data_dir.c_str());
+            fprintf(fp_dimer, "[\n");
+            fflush(fp_dimer);
         }
         SaveStepHeaders(); fprintf(fp_step, "[\n");
         SaveTimingsHeaders(); fprintf(fp_timings, "[\n");
@@ -206,6 +215,7 @@ public:
         if (corr_headers_printed) fprintf(fp_corr, "\n  ]\n}\n");
         fclose(fp_corr);
         if (fp_corrmat) { fprintf(fp_corrmat, "\n]\n"); fclose(fp_corrmat); fp_corrmat = NULL; }
+        if (fp_dimer) { fprintf(fp_dimer, "\n]\n"); fclose(fp_dimer); fp_dimer = NULL; }
         init = PETSC_FALSE;
         return 0;
     }
@@ -502,6 +512,7 @@ private:
         ierr = SaveEntanglementSpectra(BT_L, SysBlockEnl.Magnetization.List(), BT_R, EnvBlockEnl.Magnetization.List()); CHKERRQ(ierr);
         ierr = CalculateCorrelations_BlockDiag(KronBlocks, gsv_r, do_measurements); CHKERRQ(ierr);
         if (do_measurements && do_corr_matrix) { ierr = CalculateCorrelationMatrix(KronBlocks, gsv_r, NumSitesTotal); CHKERRQ(ierr); }
+        if (do_measurements && do_dimer_matrix) { ierr = CalculateDimerMatrix(KronBlocks, gsv_r); CHKERRQ(ierr); }
         if (do_prediction) {
             /* both candidates: which block grows in the next step is the caller's business (the left one in the first half of a sweep,
                the right one in the second, :996-1088); the transformations that created this step's input blocks are captured now,
@@ -597,6 +608,17 @@ private:
         return 0;
     }
 
+    /** `,\n    "name": [[...], ...]` — a rows×cols row-major matrix of a CorrelationMatrix.json / DimerMatrix.json record, %.17g */
+    static void WriteJsonMatrix(FILE* f, const char* name, const std::vector<double>& m, size_t rows, size_t cols) {
+        fprintf(f, ",\n    \"%s\": [", name);
+        for (size_t i = 0; i < rows; ++i) {
+            fprintf(f, "%s\n      [", i ? "," : "");
+            for (size_t j = 0; j < cols; ++j) fprintf(f, "%s%.17g", j ? ", " : "", m[i * cols + j]);
+            fprintf(f, "]");
+        }
+        fprintf(f, "\n    ]");
+    }
+
     /** EXTENSION (-do_correlation_matrix): one record of CorrelationMatrix.json — every <S_i S_j> of the superblock from
         dmrgx_corr_matrix (superblock site s is lattice site s), and the static structure factor
             S(q) = (1/N) Σ_ij cos(q·(r_i - r_j)) <S_i·S_j>,   <S_i·S_j> = SzSz + (SpSm + SmSp)/2,   q = (2π kx/Lx, 2π ky/Ly),
@@ -614,18 +636,9 @@ private:
         fprintf(f, "],\n    \"Sz\": [");
         for (size_t s = 0; s < n; ++s) fprintf(f, "%s%.17g", s ? ", " : "", sz[s]);
         fprintf(f, "]");
-        auto matrix = [&](const char* name, const std::vector<double>& m, size_t rows, size_t cols) {
-            fprintf(f, ",\n    \"%s\": [", name);
-            for (size_t i = 0; i < rows; ++i) {
-                fprintf(f, "%s\n      [", i ? "," : "");
-                for (size_t j = 0; j < cols; ++j) fprintf(f, "%s%.17g", j ? ", " : "", m[i * cols + j]);
-                fprintf(f, "]");
-            }
-            fprintf(f, "\n    ]");
-        };
-        matrix("SzSz", szsz, n, n);
-        matrix("SpSm", spsm, n, n);
-        matrix("SmSp", smsp, n, n);
+        WriteJsonMatrix(f, "SzSz", szsz, n, n);
+        WriteJsonMatrix(f, "SpSm", spsm, n, n);
+        WriteJsonMatrix(f, "SmSp", smsp, n, n);
         std::vector<double> sq((size_t)(Lx * Ly), 0.0);
         for (PetscInt kx = 0; kx < Lx; ++kx)
             for (PetscInt ky = 0; ky < Ly; ++ky) {
@@ -636,10 +649,74 @@ private:
                         s += std::cos(qx * (double)(x[i] - x[j]) + qy * (double)(y[i] - y[j])) * (szsz[i * n + j] + 0.5 * (spsm[i * n + j] + smsp[i * n + j]));
                 sq[(size_t)(kx * Ly + ky)] = s / (double)n;
             }
-        matrix("StructureFactor", sq, (size_t)Lx, (size_t)Ly);
+        WriteJsonMatrix(f, "StructureFactor", sq, (size_t)Lx, (size_t)Ly);
         fprintf(f, "\n  }");
         fflush(f);
         ++corrmat_records;
+        return 0;
+    }
+
+    /** EXTENSION (-do_dimer_matrix): one record of DimerMatrix.json — the dimer correlations of the distinct nearest-neighbour
+        bonds a = (i, j) of the lattice (Ham.NeighborPairs(), i < j; superblock site s is lattice site s) from dmrgx_dimer_matrix:
+            Dimer[a] = <D_a>,  DimerDimer[a][b] = <D_a D_b>,  D_a = S_i·S_j,
+        and per orientation α in {x, y} the dimer structure factor
+            S_D^α(q) = (1/N_α) Σ_{a,b∈α} cos(q·(r_a - r_b)) (<D_a D_b> - <D_a><D_b>),   q = (2π kx/Lx, 2π ky/Ly),
+        written as DimerStructureFactorX / Y [kx][ky] (all zero when the lattice has no bond of that orientation).  r_a is the
+        bond's origin, the site from which the +x or +y step leads (for a wrap-around bond the one at x = Lx - 1 or y = Ly - 1). */
+    PetscErrorCode CalculateDimerMatrix(KronBlocks_t& KronBlocks, const Vec& gsv_r) {
+        const PetscInt Lx = Ham.Lx(), Ly = Ham.Ly();
+        struct Bond { PetscInt i, j, xi, yi, xj, yj, ox, oy; char dir; };
+        std::vector<Bond> bonds;
+        { /* Ly = 2 with periodic y lists every vertical bond twice */
+            std::set<std::pair<PetscInt, PetscInt>> seen;
+            for (const std::vector<PetscInt>& p : Ham.NeighborPairs()) {
+                if (!seen.insert({p[0], p[1]}).second) continue;
+                Bond b;
+                b.i = p[0]; b.j = p[1];
+                Ham.To2D(b.i, b.xi, b.yi); Ham.To2D(b.j, b.xj, b.yj);
+                b.dir = b.xi == b.xj ? 'y' : 'x';
+                const PetscInt ui = b.dir == 'y' ? b.yi : b.xi, uj = b.dir == 'y' ? b.yj : b.xj;
+                const bool from_i = ui + 1 == uj || (uj + 1 != ui && ui > uj); /* a +1 step, else the wrap-around from the last row */
+                b.ox = from_i ? b.xi : b.xj; b.oy = from_i ? b.yi : b.yj;
+                bonds.push_back(b);
+            }
+        }
+        const size_t nb = bonds.size();
+        if (nb == 0) SETERRQ(mpi_comm, 1, "-do_dimer_matrix: the lattice has no nearest-neighbour bond.");
+        std::vector<dmrgx_int> si(nb), sj(nb);
+        for (size_t a = 0; a < nb; ++a) { si[a] = bonds[a].i; sj[a] = bonds[a].j; }
+        std::vector<double> dd(nb * nb), d(nb);
+        DMRGX_CALL(dmrgx_dimer_matrix(KronBlocks.Handle(), gsv_r.d, (dmrgx_int)nb, si.data(), sj.data(), dd.data(), d.data(), NULL));
+        FILE* f = fp_dimer;
+        fprintf(f, "%s  {\n    \"GlobIdx\": %lld,\n    \"LoopIdx\": %lld,\n    \"bonds\": [", dimer_records ? ",\n" : "", LLD(GlobIdx), LLD(LoopIdx));
+        for (size_t a = 0; a < nb; ++a) {
+            const Bond& b = bonds[a];
+            fprintf(f, "%s\n      {\"sites\": [%lld, %lld], \"coords\": [[%lld, %lld], [%lld, %lld]], \"orientation\": \"%c\", \"origin\": [%lld, %lld]}",
+                    a ? "," : "", LLD(b.i), LLD(b.j), LLD(b.xi), LLD(b.yi), LLD(b.xj), LLD(b.yj), b.dir, LLD(b.ox), LLD(b.oy));
+        }
+        fprintf(f, "\n    ],\n    \"Dimer\": [");
+        for (size_t a = 0; a < nb; ++a) fprintf(f, "%s%.17g", a ? ", " : "", d[a]);
+        fprintf(f, "]");
+        WriteJsonMatrix(f, "DimerDimer", dd, nb, nb);
+        for (const char dir : {'x', 'y'}) {
+            std::vector<size_t> in;
+            for (size_t a = 0; a < nb; ++a)
+                if (bonds[a].dir == dir) in.push_back(a);
+            std::vector<double> sq((size_t)(Lx * Ly), 0.0);
+            for (PetscInt kx = 0; kx < Lx && !in.empty(); ++kx)
+                for (PetscInt ky = 0; ky < Ly; ++ky) {
+                    const double qx = 2.0 * M_PI * (double)kx / (double)Lx, qy = 2.0 * M_PI * (double)ky / (double)Ly;
+                    double s = 0;
+                    for (const size_t a : in)
+                        for (const size_t b : in)
+                            s += std::cos(qx * (double)(bonds[a].ox - bonds[b].ox) + qy * (double)(bonds[a].oy - bonds[b].oy)) * (dd[a * nb + b] - d[a] * d[b]);
+                    sq[(size_t)(kx * Ly + ky)] = s / (double)in.size();
+                }
+            WriteJsonMatrix(f, dir == 'x' ? "DimerStructureFactorX" : "DimerStructureFactorY", sq, (size_t)Lx, (size_t)Ly);
+        }
+        fprintf(f, "\n  }");
+        fflush(f);
+        ++dimer_records;
         return 0;
     }
 
@@ -794,6 +871,9 @@ private:
     PetscBool do_corr_matrix = PETSC_FALSE;   /* -do_correlation_matrix (extension) */
     FILE* fp_corrmat = NULL;
     long long corrmat_records = 0;
+    PetscBool do_dimer_matrix = PETSC_FALSE;  /* -do_dimer_matrix (extension) */
+    FILE* fp_dimer = NULL;
+    long long dimer_records = 0;
     PetscScalar gse = 0.0;
     std::vector<PetscReal> trunc_err;
     double t0abs = 0.0;

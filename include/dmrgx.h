@@ -198,6 +198,28 @@ int dmrgx_expect(dmrgx_hshell h1, const double* d_psi, double* value);
    Errors: 62 psi or an output NULL, 56 the kron has not exactly one sector, 73 a block lacks Sz_i or Sp_i (site in the message). */
 int dmrgx_corr_matrix(dmrgx_kron k, const double* d_psi, double* szsz, double* spsm, double* smsp, double* sz, double* flops);
 
+/* ---- EXTENSION: the dimer (bond–bond) correlation matrix (no reference counterpart: there every four-operator correlator
+   would be nine KronConstruct + MatMult + VecDot, include/DMRGBlockContainer.hpp:2262-2296).  Bond a joins the superblock
+   sites site_i[a] != site_j[a] (numbered as in dmrgx_corr_matrix) and stands for the isotropic bond operator, in this order:
+       D_a = Sz_i Sz_j + ½ S+_i S-_j + ½ S-_i S+_j
+   psi lies in the superblock's one total-Sz sector and is used as given (not normalised).  Host outputs:
+       dd[a*nbonds+b] = <D_a psi, D_b psi> = <psi| D_aᵀ D_b |psi>   (nbonds×nbonds row-major),   d[a] = <psi| D_a |psi>
+   Ordering convention: every operator is its block's stored (rotated) matrix, so on a truncated block two operators of the
+   same block do not commute; a same-block bond is the product in the order above and its adjoint is
+   D_aᵀ = Sz_j Sz_i + ½ S+_j S-_i + ½ S-_j S+_i.  Then d[a] = szsz + ½(spsm + smsp) at [i*n+j] of dmrgx_corr_matrix to rounding,
+   and on exact blocks dd is the true <(S_i·S_j)(S_k·S_l)>.  Nothing is symmetrised.
+   One batched device pass: the panels O_j·psi (O in Sz, S-, S+) of the bonds' second sites, then every bond panel D_a·psi
+   (one contraction launch each), then one Gram matrix over the bond panels and psi.  Device memory during the call:
+   (nj·(D + D₋ + D₊) + (nbonds + 1)·D)·8 bytes plus the plans, with D the superblock dimension, D∓ those of the sectors qn ∓ 1
+   and nj <= n the number of distinct second sites; an empty qn ± 1 sector drops its term.  flops (may be NULL) receives the
+   algorithmic flops of the call.  On a multi-GPU context the calling rank computes everything from its complete psi, with
+   no collective.
+   Errors: 62 psi, a site array or an output NULL; 63 nbonds < 1, or a site outside [0, n) or site_i == site_j (the bond
+   index in the message); 56 the kron has not exactly one sector; 73 a block lacks Sz or Sp at a site of some bond (site in
+   the message). */
+int dmrgx_dimer_matrix(dmrgx_kron k, const double* d_psi, dmrgx_int nbonds, const dmrgx_int* site_i, const dmrgx_int* site_j, double* dd,
+                       double* d, double* flops);
+
 /* ---- Hamiltonians::J1J2XXZModel_SquareLattice::H(nsites): src/Hamiltonians.cpp:73-122 (host only).
         Returns the number of terms (fills at most maxterms); bc: 0 open, 1 periodic; nsites < 0 = full lattice. ---- */
 dmrgx_int dmrgx_ham_terms(dmrgx_int Lx, dmrgx_int Ly, double J1, double Jz1, double J2, double Jz2, int bcx, int bcy, dmrgx_int nsites,
