@@ -342,6 +342,39 @@ class KronBlocks:
         _chk(lib().dmrgx_dimer_matrix(self.h, psi.ptr if psi is not None else None, LL(nb), _p(si), _p(sj), _p(dd), _p(d), C.byref(fl)))
         return {"DD": dd, "D": d, "flops": fl.value}
 
+    def SpectralLanczos(self, psi, target, op, coef, nsteps):
+        """EXTENSION (dmrgx_spectral_lanczos): continued-fraction coefficients of the start vectors phi_v = Σ_s coef[v, s] O_s psi
+        (O = Sz, S+ or S- for op = OpSz, OpSp, OpSm; coef an nvec×n array over the superblock sites) under `target`, an HShell on
+        the sector qn + op of the same two blocks.  Returns alpha and beta (nvec×nsteps, beta[:, 0] = 0), norm2 (nvec),
+        nsteps_done (nvec) and the algorithmic flops of the call; evaluate G(z) with continued_fraction()."""
+        n = self.left.NumSites() + self.right.NumSites()
+        c = _d(coef).reshape(-1, n) if np.size(coef) else np.zeros((0, n))
+        nvec, nsteps = len(c), int(nsteps)
+        alpha = np.zeros((nvec, max(nsteps, 0))); beta = np.zeros((nvec, max(nsteps, 0)))
+        norm2 = np.zeros(nvec); done = np.zeros(nvec, np.int64)
+        fl = C.c_double()
+        _chk(lib().dmrgx_spectral_lanczos(self.h, psi.ptr if psi is not None else None, target.h if target is not None else None, int(op), LL(nvec),
+                                          _p(c), LL(nsteps), _p(alpha), _p(beta), _p(norm2), _p(done), C.byref(fl)))
+        return {"alpha": alpha, "beta": beta, "norm2": norm2, "nsteps_done": done, "flops": fl.value}
+
+
+def continued_fraction(alpha, beta, norm2, nsteps_done, z):
+    """G(z) = norm2 / (z - α_0 - β_1² / (z - α_1 - … - β_{k-1}² / (z - α_{k-1}))), k = nsteps_done, for one vector (alpha, beta of
+    length >= k, scalar norm2 and k) or a batch (nvec×nsteps arrays, nvec norms and counts), at a scalar or a vector of complex z.
+    A vector with k = 0 gives 0.  With z = ω + E0 + iη, -Im G / π is the spectral function broadened by a Lorentzian of width η."""
+    a, b = np.atleast_2d(np.asarray(alpha, float)), np.atleast_2d(np.asarray(beta, float))
+    nrm, k = np.atleast_1d(np.asarray(norm2, float)), np.atleast_1d(np.asarray(nsteps_done, np.int64))
+    zz = np.atleast_1d(np.asarray(z, complex))
+    G = np.zeros((len(nrm), len(zz)), complex)
+    for v in range(len(nrm)):
+        g = np.zeros(len(zz), complex)
+        for t in range(int(k[v]) - 1, -1, -1):
+            g = 1.0 / (zz - a[v, t] - (b[v, t + 1] ** 2 * g if t + 1 < k[v] else 0.0))
+        G[v] = nrm[v] * g if k[v] > 0 else 0.0
+    if np.ndim(norm2) == 0:
+        G = G[0]
+    return G if np.ndim(z) else G[..., 0]
+
 
 class HShell:
     """The matrix-free superblock Hamiltonian (MATSHELL with MatMult_KronSumShell)."""

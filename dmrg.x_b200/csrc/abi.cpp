@@ -354,6 +354,11 @@ int dmrgx_dimer_matrix(dmrgx_kron k, const double* d_psi, dmrgx_int nbonds, cons
     return guard([&] { dimer_matrix(K(k), d_psi, nbonds, site_i, site_j, dd, d, flops); });
 }
 
+int dmrgx_spectral_lanczos(dmrgx_kron k, const double* d_psi, dmrgx_hshell h_target, int op, dmrgx_int nvec, const double* coef, dmrgx_int nsteps,
+                           double* alpha, double* beta, double* norm2, dmrgx_int* nsteps_done, double* flops) {
+    return guard([&] { spectral_lanczos(K(k), d_psi, H(h_target), op, nvec, coef, nsteps, alpha, beta, norm2, nsteps_done, flops); });
+}
+
 /* microbenchmark of the chain engine on one plain product C[M,N] = A·B (selectable operand layouts), for profiling */
 int dmrgx_selftest_gemm(dmrgx_ctx cx, dmrgx_int M, dmrgx_int N, dmrgx_int K, int a_k_contig, int b_k_contig, int nseg, int reps, double* ms,
                         double* max_err) {

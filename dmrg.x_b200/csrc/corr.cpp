@@ -14,8 +14,14 @@
  *  The dimer matrix is the Gram matrix of the bond panels  D̃_a psi = Sz_i (Sz_j psi) + ½ S+_i (S-_j psi) + ½ S-_i (S+_j psi)
  *  (bond a = (i, j) in the caller's order), built in two chain-kernel plans: the single-operator panels of every second site j
  *  in all three sectors, then every bond panel as the sum of its three terms in psi's sector.
+ *
+ *  The spectral recurrence (continued-fraction method, K. Hallberg, PRB 52, R9827 (1995)) starts from  phi_v = Σ_s coef[v][s] O_s psi
+ *  in the sector qn + op: the n single-operator panels are one chain-kernel plan, the start vectors of a batch are one GEMM
+ *  plan  Phi = C·P  over them, and every vector then runs a plain three-term Lanczos recurrence of the target shell, the whole
+ *  batch advanced by dev::lanczos_batch with no host synchronisation until the batch is finished.
  */
 #include <algorithm>
+#include <cmath>
 #include <memory>
 #include <set>
 #include <string>
@@ -239,6 +245,130 @@ void dimer_matrix(const Kron* kron, const double* d_psi, long long nb, const lon
     for (long long a = 0; a < nb; ++a) {
         for (long long b = 0; b < nb; ++b) dd[a * nb + b] = 0.25 * G[(size_t)(a * np + b)];
         d[a] = 0.5 * G[(size_t)(a * np + nb)];
+    }
+    if (flops) *flops = total;
+}
+
+/* Device memory for the three recurrence columns (v_prev, v, H·v) of a batch: it holds as many vectors as fit, at least one */
+constexpr double SPECTRAL_BATCH_BYTES = 2.0 * (1LL << 30);
+/* a start vector whose norm is at most this fraction of Σ_s |coef_s|·‖O_s psi‖ is zero up to rounding: norm2 = 0, no steps */
+constexpr double SPECTRAL_ZERO_REL = 1e-12;
+
+void spectral_lanczos(const Kron* kron, const double* d_psi, HShell* h, int op, long long nvec, const double* coef, long long nsteps,
+                      double* alpha, double* beta, double* norm2, long long* nsteps_done, double* flops) {
+    if (!d_psi) throw Err(ERR_ARG_WRONG, "psi is NULL.");
+    if (!h) throw Err(ERR_ARG_WRONG, "the target shell is NULL.");
+    if (!coef) throw Err(ERR_ARG_WRONG, "the coefficient array is NULL.");
+    if (!alpha || !beta || !norm2 || !nsteps_done) throw Err(ERR_ARG_WRONG, "an output array is NULL.");
+    if (op != OP_SZ && op != OP_SP && op != OP_SM)
+        throw Err(ERR_ARG_OUTOFRANGE, "op must be DMRGX_OP_SZ, DMRGX_OP_SP or DMRGX_OP_SM (got " + std::to_string(op) + ").");
+    if (nvec < 1) throw Err(ERR_ARG_OUTOFRANGE, "the spectral recurrence needs at least one vector (got " + std::to_string(nvec) + ").");
+    if (nsteps < 1) throw Err(ERR_ARG_OUTOFRANGE, "the spectral recurrence needs at least one step (got " + std::to_string(nsteps) + ").");
+    const Block *L = kron->L, *R = kron->R;
+    const int nL = L->nsites, n = nL + R->nsites;
+    for (long long i = 0; i < nvec * n; ++i)
+        if (!std::isfinite(coef[i]))
+            throw Err(ERR_ARG_OUTOFRANGE, "coefficient " + std::to_string(i % n) + " of vector " + std::to_string(i / n) + " is not finite.");
+    const double qn = single_sector(kron, "the spectral recurrence");
+    Ctx* ctx = kron->ctx;
+    if (ctx->world > 1) throw Err(ERR_SUP, "the spectral recurrence needs a single-GPU context: the sharded apply of the target shell is collective.");
+    const Kron* tk = h->kron;
+    std::set<double> tq;
+    for (const KronPair& p : tk->pairs) tq.insert(p.qn);
+    if (tk->L != L || tk->R != R || tq.size() != 1 || *tq.begin() != qn + op)
+        throw Err(ERR_ARG_WRONGSTATE, "the target shell must be built on a Kron of the same two blocks whose single sector is qn + op = " +
+                                          std::to_string(qn + op) + ".");
+    std::vector<char> used(n, 0);
+    for (long long i = 0; i < nvec * n; ++i)
+        if (coef[i] != 0.0) used[i % n] = 1;
+    for (int s = 0; s < n; ++s)
+        if (used[s]) require_site_ops(kron, s);
+    std::fill(alpha, alpha + nvec * nsteps, 0.0);
+    std::fill(beta, beta + nvec * nsteps, 0.0);
+    std::fill(norm2, norm2 + nvec, 0.0);
+    std::fill(nsteps_done, nsteps_done + nvec, 0LL);
+    const long long D = tk->nstates(), ld = (D + 1) & ~1LL;
+    double total = 0;
+    if (D > 0) {
+        dev::Stream* st = ctx->st;
+        /* the n single-operator panels O_s psi in the sector qn + op, one plan; a site no vector uses is a zero column, so the
+           GEMM below always runs over all n sites and a vector's bits do not depend on the others */
+        BufRef Pb = std::make_shared<DevBuf>(ctx, (size_t)n * ld * 8), Cb = std::make_shared<DevBuf>(ctx, (size_t)(nvec * n) * 8);
+        BufRef pnb = std::make_shared<DevBuf>(ctx, (size_t)n * 8);
+        double* P = Pb->as<double>();
+        dev::h2d(st, Cb->p, coef, (size_t)(nvec * n) * 8);
+        Plan panels;
+        for (int s = 0; s < n; ++s) {
+            if (used[s]) plan_panel(panels, tk, {{s < nL, site_op(kron, s, op), kron, d_psi, 1.0}}, P + (long long)s * ld);
+            else dev::memset0(st, P + (long long)s * ld, (size_t)ld * 8);
+        }
+        panels.upload(ctx);
+        panels.run(ctx);
+        total += panels.flops;
+        /* ‖O_s psi‖: the scale below which a start vector is rounding noise */
+        std::vector<double> pn2(n, 0.0);
+        for (int s = 0; s < n; ++s)
+            if (used[s]) dev::dot(st, P + (long long)s * ld, P + (long long)s * ld, D, pnb->as<double>() + s);
+        dev::d2h(st, pn2.data(), pnb->p, (size_t)n * 8);
+        dev::sync(st);
+        for (int s = 0; s < n; ++s) pn2[s] = used[s] ? std::sqrt(pn2[s]) : 0.0;
+
+        const int nb = (int)std::max<long long>(1, std::min<long long>(nvec, (long long)(SPECTRAL_BATCH_BYTES / (3.0 * 8.0 * (double)ld))));
+        const int nblk = dev::lanczos_blocks(D);
+        BufRef slots = std::make_shared<DevBuf>(ctx, (size_t)3 * nb * ld * 8);
+        BufRef scal = std::make_shared<DevBuf>(ctx, (size_t)(2 * nb * nsteps + 4 * nb + (long long)nb * nblk) * 8);
+        BufRef ints = std::make_shared<DevBuf>(ctx, (size_t)nb * (8 + 4 + 4));
+        double* slot[3] = {slots->as<double>(), slots->as<double>() + (long long)nb * ld, slots->as<double>() + 2LL * nb * ld};
+        dev::LanczosBatch lb;
+        lb.nsteps = (int)nsteps; lb.n = D; lb.ld = ld;
+        lb.alpha = scal->as<double>(); lb.beta = lb.alpha + (long long)nb * nsteps;
+        lb.norm2 = lb.beta + (long long)nb * nsteps; lb.a = lb.norm2 + nb; lb.scale = lb.a + nb;
+        double* zero2 = lb.scale + nb;
+        lb.zero2 = zero2; lb.partials = zero2 + nb;
+        lb.ndone = ints->as<long long>(); lb.done = (int*)(lb.ndone + nb); lb.tickets = (unsigned int*)(lb.done + nb);
+        dev::memset0(st, lb.tickets, (size_t)nb * 4);
+        std::vector<double> hz(nb);
+        for (long long b0 = 0; b0 < nvec; b0 += nb) {
+            const int m = (int)std::min<long long>(nb, nvec - b0);
+            lb.nb = m;
+            for (int c = 0; c < m; ++c) {
+                double sig = 0;
+                for (int s = 0; s < n; ++s) sig += std::fabs(coef[(b0 + c) * n + s]) * pn2[s];
+                hz[c] = (SPECTRAL_ZERO_REL * sig) * (SPECTRAL_ZERO_REL * sig);
+            }
+            dev::h2d(st, zero2, hz.data(), (size_t)m * 8);
+            dev::memset0(st, lb.alpha, (size_t)2 * nb * nsteps * 8);
+            dev::memset0(st, lb.ndone, (size_t)nb * (8 + 4));
+            /* start vectors: Phi[c] = Σ_s coef[b0 + c][s] P_s, one GEMM plan (the chain engine's plain product) into the y slot */
+            int ip = 0, ic = 1, iy = 2;
+            Plan comb;
+            Contribution g;
+            g.r0 = 0; g.c0 = 0; g.nr = m; g.nc = (int)D;
+            g.seg = make_seg(dev::SEG_GEMM);
+            g.seg.A = Cb->as<double>() + b0 * n; g.seg.lda_m = n; g.seg.lda_k = 1; g.seg.K = n;
+            g.seg.B = P; g.seg.ldb_k = ld; g.seg.ldb_n = 1;
+            emit_cells(comb, slot[iy], false, ld, m, (int)D, {g}, true);
+            comb.upload(ctx);
+            comb.run(ctx);
+            total += comb.flops;
+            auto rotate = [&] { const int p = ip; ip = ic; ic = iy; iy = p; };
+            dev::lanczos_batch(st, lb, 0, -1, slot[ip], slot[ic], slot[iy]);
+            rotate();
+            for (long long t = 0; t < nsteps; ++t) {
+                for (int c = 0; c < m; ++c) hshell_apply(h, slot[ic] + (long long)c * ld, slot[iy] + (long long)c * ld);
+                dev::lanczos_batch(st, lb, 1, (int)t, slot[ip], slot[ic], slot[iy]);
+                if (t + 1 < nsteps) {
+                    dev::lanczos_batch(st, lb, 2, (int)t, slot[ip], slot[ic], slot[iy]);
+                    rotate();
+                }
+            }
+            dev::d2h(st, alpha + b0 * nsteps, lb.alpha, (size_t)m * nsteps * 8);
+            dev::d2h(st, beta + b0 * nsteps, lb.beta, (size_t)m * nsteps * 8);
+            dev::d2h(st, norm2 + b0, lb.norm2, (size_t)m * 8);
+            dev::d2h(st, nsteps_done + b0, lb.ndone, (size_t)m * 8);
+            dev::sync(st); /* the combine plan and hz are reused by the next batch */
+        }
+        total += (double)nvec * (double)nsteps * h->alg_flops + (double)nvec * (10.0 * (double)nsteps + 2.0) * (double)D;
     }
     if (flops) *flops = total;
 }

@@ -167,6 +167,35 @@ void dot(Stream*, const double* x, const double* y, long long n, double* d_out);
    data give the same bits), then mirrored.  Two launches. */
 void gram(Stream*, const double* P, long long ldp, int np, long long n, double* d_G);
 
+/* Plain three-term Lanczos recurrence over nb independent columns (spectral.cpp), all state on the device.  Column c of a
+   slot is slot + c·ld, rows [0, n).  The caller keeps three slots per column and rotates them (prev, cur, y) <- (cur, y, prev)
+   after passes 0 and 2; y = H·cur is its own apply.  cur holds u_t = c_t·v_t (c_t = *scale, the norm the recurrence found).
+     pass 0 (start):  b2 = y·y;  norm2 = b2, or 0 when b2 <= zero2 (the column is then done with 0 steps), else scale = sqrt(b2)
+     pass 1 (step t): cur = v_t = cur / c_t;  y = w = y / c_t - β_t·prev  (β_0 = 0, prev unread);  α_t = v_t·w
+                      t = nsteps - 1: the column is done with nsteps steps
+     pass 2 (step t): y = w - α_t·v_t;  β_{t+1}² = y·y;  β_{t+1} <= LANCZOS_BETA_REL·sqrt(α_t² + β_t²): done with t + 1 steps,
+                      else beta[t+1] = β_{t+1} and scale = β_{t+1}
+   A done column is skipped by every later pass.  Each column's sums are cut into lanczos_blocks(n) fixed block partials that
+   the column's last block adds in block order: the bits of a column do not depend on nb or on the other columns.  One launch
+   per pass for the whole batch. */
+constexpr double LANCZOS_BETA_REL = 1e-10;
+struct LanczosBatch {
+    int nb = 0, nsteps = 0;
+    long long n = 0, ld = 0;
+    double* alpha = nullptr;        /* nb × nsteps: α_t */
+    double* beta = nullptr;         /* nb × nsteps: β_t, β_0 = 0 (zeroed by the caller, like alpha) */
+    double* norm2 = nullptr;        /* nb */
+    long long* ndone = nullptr;     /* nb, zeroed by the caller */
+    double* a = nullptr;            /* nb: α of the current step */
+    double* scale = nullptr;        /* nb: c_t */
+    const double* zero2 = nullptr;  /* nb */
+    int* done = nullptr;            /* nb, zeroed by the caller */
+    double* partials = nullptr;     /* nb × lanczos_blocks(n) */
+    unsigned int* tickets = nullptr; /* nb, zeroed by the caller; every pass leaves them zero */
+};
+int lanczos_blocks(long long n);
+void lanczos_batch(Stream*, const LanczosBatch&, int pass, int t, const double* prev, double* cur, double* y);
+
 /* dense symmetric eigendecomposition of a batch of independent blocks, in place: block b is n[b]×n[b] at d_A[b]; on exit
    row k of it (row-major) is the k-th eigenvector, eigenvalues ascending in d_w[b].  Blocks of up to 64 states are solved by
    one cyclic-Jacobi launch on a side stream; the larger ones, all together, by batched block Jacobi on the main stream.

@@ -1038,6 +1038,88 @@ void gram(Stream* st, const double* P, long long ldp, int np, long long n, doubl
     free_bytes(st, part); /* stream-ordered heap: the next user of the range is queued behind the reduction */
 }
 
+/* ================================================================================================
+ *  lanczos_kernel — one pass of the batched continued-fraction recurrence (spectral.cpp, dev.h: lanczos_batch).  CTA
+ *  blockIdx.x = column · nblk + block: the column's rows are strided over its nblk blocks (nblk from n only), each block
+ *  writes one partial, and the block that draws the column's last ticket adds the nblk partials in block order and updates
+ *  that column's scalars.  HBM-bound streaming: pass 1 reads three vectors and writes two, pass 2 reads two and writes one.
+ * ============================================================================================== */
+constexpr int LZ_THREADS = 256;
+int lanczos_blocks(long long n) { return (int)std::max<long long>(1, std::min<long long>((n + 4 * LZ_THREADS - 1) / (4 * LZ_THREADS), RED_BLOCKS)); }
+
+__global__ void __launch_bounds__(LZ_THREADS) lanczos_kernel(LanczosBatch L, int pass, int t, int nblk, const double* __restrict__ prev,
+                                                             double* __restrict__ cur, double* __restrict__ y) {
+    const int col = blockIdx.x / nblk, blk = blockIdx.x % nblk;
+    /* done is only written by the finisher of a column, after every block of that column has passed this test */
+    if (L.done[col]) return;
+    const long long off = (long long)col * L.ld, stride = (long long)nblk * LZ_THREADS;
+    double* u = cur + off;
+    double* w = y + off;
+    double s = 0.0;
+    if (pass == 0) {
+        for (long long q = (long long)blk * LZ_THREADS + threadIdx.x; q < L.n; q += stride) { const double x = w[q]; s += x * x; }
+    } else if (pass == 1) {
+        const double c = L.scale[col], inv = 1.0 / c;
+        if (t > 0) {
+            const double* p = prev + off;
+            for (long long q = (long long)blk * LZ_THREADS + threadIdx.x; q < L.n; q += stride) {
+                const double v = u[q] * inv, x = w[q] * inv - c * p[q];
+                u[q] = v; w[q] = x; s += v * x;
+            }
+        } else {
+            for (long long q = (long long)blk * LZ_THREADS + threadIdx.x; q < L.n; q += stride) {
+                const double v = u[q] * inv, x = w[q] * inv;
+                u[q] = v; w[q] = x; s += v * x;
+            }
+        }
+    } else {
+        const double a = L.a[col];
+        for (long long q = (long long)blk * LZ_THREADS + threadIdx.x; q < L.n; q += stride) { const double x = w[q] - a * u[q]; w[q] = x; s += x * x; }
+    }
+    __shared__ double sh[LZ_THREADS / 32];
+    __shared__ bool last;
+    const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+    s = warp_sum(s);
+    if (lane == 0) sh[wid] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double r = 0.0;
+        for (int k = 0; k < LZ_THREADS / 32; ++k) r += sh[k];
+        L.partials[(long long)col * nblk + blk] = r;
+        __threadfence();
+        last = atomicAdd(&L.tickets[col], 1u) == (unsigned)nblk - 1;
+    }
+    __syncthreads();
+    if (!last || wid != 0) return;
+    __threadfence();
+    double r = 0.0;
+    for (int b = lane; b < nblk; b += 32) r += __ldcg(L.partials + (long long)col * nblk + b);
+    r = warp_sum(r);
+    if (lane != 0) return;
+    L.tickets[col] = 0u;
+    if (pass == 0) {
+        const bool zero = r <= L.zero2[col];
+        L.norm2[col] = zero ? 0.0 : r;
+        if (zero) L.done[col] = 1;
+        else L.scale[col] = sqrt(r);
+    } else if (pass == 1) {
+        L.a[col] = r;
+        L.alpha[(long long)col * L.nsteps + t] = r;
+        if (t == L.nsteps - 1) { L.ndone[col] = L.nsteps; L.done[col] = 1; }
+    } else {
+        const double beta = sqrt(r), bt = t > 0 ? L.scale[col] : 0.0, a = L.a[col];
+        if (beta <= LANCZOS_BETA_REL * sqrt(a * a + bt * bt)) { L.ndone[col] = t + 1; L.done[col] = 1; }
+        else { L.beta[(long long)col * L.nsteps + t + 1] = beta; L.scale[col] = beta; }
+    }
+}
+
+void lanczos_batch(Stream* st, const LanczosBatch& L, int pass, int t, const double* prev, double* cur, double* y) {
+    if (L.nb <= 0 || L.n <= 0) return;
+    const int nblk = lanczos_blocks(L.n);
+    lanczos_kernel<<<(unsigned)((long long)L.nb * nblk), LZ_THREADS, 0, st->s>>>(L, pass, t, nblk, prev, cur, y);
+    LAUNCH_CHECK();
+}
+
 template <int NV>
 __global__ void __launch_bounds__(256) gs_final_kernel(const double* __restrict__ V, long long ldv, int nvec, const double* __restrict__ w, long long n,
                                                        const double* __restrict__ coef, const double* __restrict__ nrm2_in, double* __restrict__ nrm2_out,

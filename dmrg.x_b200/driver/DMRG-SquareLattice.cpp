@@ -2,9 +2,9 @@
  *
  *      DMRG-SquareLattice.x -Lx 12 -Ly 6 -J1 0.5 -Jz1 1 -J2 0.25 -Jz2 0.5 -mwarmup 128 -msweeps 512,1024,2048 \
  *                           [-H_eps_tol 1e-12] [-data_dir out/] [-device 0] [-verbose] [-wavefunction_prediction 1] [-do_correlation_matrix 1]
- *                           [-do_dimer_matrix 1]
+ *                           [-do_dimer_matrix 1] [-do_spectral_function 1 [-spectral_nsteps 64] [-spectral_ops zz,pm,mp]]
  *
- *  Same options (plus -device and the opt-in -wavefunction_prediction, -do_correlation_matrix and -do_dimer_matrix, which the reference does not have), same stdout banner, same JSON files; one process drives one B200 through the C ABI
+ *  Same options (plus -device and the opt-in -wavefunction_prediction, -do_correlation_matrix, -do_dimer_matrix and -do_spectral_function, which the reference does not have), same stdout banner, same JSON files; one process drives one B200 through the C ABI
  *  (include/dmrgx.h).  There is no CPU path: without a CUDA device the context creation fails and the
  *  program exits non-zero.
  */
@@ -12,7 +12,11 @@ static char help[] = "DMRG executable for the Spin-1/2 J1-J2 XY Model on a two-d
                      "Extensions, off by default, computed and written by rank 0 at every measurement step:\n"
                      "  -do_correlation_matrix 1   every <S_i S_j> and the structure factor S(q) -> CorrelationMatrix.json\n"
                      "  -do_dimer_matrix 1         <D_a>, <D_a D_b> over the nearest-neighbour bonds (D_a = S_i.S_j) and the\n"
-                     "                             dimer structure factors of the x and y bonds -> DimerMatrix.json\n";
+                     "                             dimer structure factors of the x and y bonds -> DimerMatrix.json\n"
+                     "  -do_spectral_function 1    continued-fraction coefficients of the dynamical structure factor S(q, w) on\n"
+                     "                             the Lx x Ly momentum grid -> SpectralFunction.json (single-GPU runs only)\n"
+                     "  -spectral_nsteps N         Lanczos steps per momentum and operator (default 64)\n"
+                     "  -spectral_ops zz,pm,mp     which of <Sz Sz>, <S+ S->, <S- S+> to compute (default all three)\n";
 
 #include <unistd.h>
 

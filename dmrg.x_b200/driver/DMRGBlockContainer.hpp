@@ -139,7 +139,32 @@ public:
         /* EXTENSION, off by default: the dimer (bond–bond) correlation matrix of the nearest-neighbour bonds and the dimer
            structure factors at every measurement step, in DimerMatrix.json; computed and written by rank 0 only */
         o.GetBool("-do_dimer_matrix", &do_dimer_matrix, NULL);
-        { int rank = 0, world = 1; dmrgx_ctx_rank(DmrgxContext(), &rank, &world); if (rank != 0) do_corr_matrix = do_dimer_matrix = PETSC_FALSE; }
+        /* EXTENSION, off by default: the dynamical structure factor S(q, ω) by the continued-fraction method at every measurement
+           step, in SpectralFunction.json; computed and written by rank 0 of a single-GPU run */
+        o.GetBool("-do_spectral_function", &do_spectral, NULL);
+        o.GetInt("-spectral_nsteps", &spectral_nsteps, NULL);
+        if (spectral_nsteps < 1) SETERRQ1(mpi_comm, 1, "-spectral_nsteps must be at least 1. Got %lld.", LLD(spectral_nsteps));
+        if (o.Has("-spectral_ops")) {
+            std::string list;
+            o.GetString("-spectral_ops", list, NULL);
+            for (char& c : list) if (c == ',') c = ' ';
+            std::istringstream iss(list);
+            spectral_ops = {false, false, false};
+            bool any = false;
+            for (std::string item; iss >> item; any = true) {
+                const int k = item == "zz" ? 0 : item == "pm" ? 1 : item == "mp" ? 2 : -1;
+                if (k < 0) SETERRQ1(mpi_comm, PETSC_ERR_ARG_WRONG, "-spectral_ops: unknown item '%s' (the items are zz, pm and mp).", item.c_str());
+                spectral_ops[(size_t)k] = true;
+            }
+            if (!any) SETERRQ(mpi_comm, PETSC_ERR_ARG_WRONG, "-spectral_ops: the list is empty (the items are zz, pm and mp).");
+        }
+        {
+            int rank = 0, world = 1;
+            dmrgx_ctx_rank(DmrgxContext(), &rank, &world);
+            /* the recurrence applies H on one GPU; the sharded apply is collective and a rank-0-only pass cannot use it */
+            if (world > 1 && do_spectral) SETERRQ1(mpi_comm, PETSC_ERR_SUP, "-do_spectral_function runs on one GPU only (this run has %d ranks).", world);
+            if (rank != 0) do_corr_matrix = do_dimer_matrix = do_spectral = PETSC_FALSE;
+        }
         if (do_corr_matrix) {
             fp_corrmat = fopen((data_dir + "CorrelationMatrix.json").c_str(), "w");
             if (!fp_corrmat) SETERRQ1(mpi_comm, 1, "cannot open %sCorrelationMatrix.json", data_dir.c_str());
@@ -151,6 +176,12 @@ public:
             if (!fp_dimer) SETERRQ1(mpi_comm, 1, "cannot open %sDimerMatrix.json", data_dir.c_str());
             fprintf(fp_dimer, "[\n");
             fflush(fp_dimer);
+        }
+        if (do_spectral) {
+            fp_spectral = fopen((data_dir + "SpectralFunction.json").c_str(), "w");
+            if (!fp_spectral) SETERRQ1(mpi_comm, 1, "cannot open %sSpectralFunction.json", data_dir.c_str());
+            fprintf(fp_spectral, "[\n");
+            fflush(fp_spectral);
         }
         SaveStepHeaders(); fprintf(fp_step, "[\n");
         SaveTimingsHeaders(); fprintf(fp_timings, "[\n");
@@ -216,6 +247,7 @@ public:
         fclose(fp_corr);
         if (fp_corrmat) { fprintf(fp_corrmat, "\n]\n"); fclose(fp_corrmat); fp_corrmat = NULL; }
         if (fp_dimer) { fprintf(fp_dimer, "\n]\n"); fclose(fp_dimer); fp_dimer = NULL; }
+        if (fp_spectral) { fprintf(fp_spectral, "\n]\n"); fclose(fp_spectral); fp_spectral = NULL; }
         init = PETSC_FALSE;
         return 0;
     }
@@ -494,7 +526,8 @@ private:
         total_matvecs += eps_stats.nmatvec;
         double h_bytes = 0, h_flops = 0;
         { dmrgx_int hn, hnt, t1, t2; dmrgx_hshell_stats(H.h, &hn, &hnt, &h_bytes, &h_flops, &t1, &t2); }
-        ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr);
+        /* -do_spectral_function: the zz recurrence runs on this step's H, which then lives until the measurement */
+        if (!(do_measurements && do_spectral)) { ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr); }
         const double tdiag = Tick();
         total_matvec_flops += h_flops * (double)eps_stats.nmatvec;
         timings_data.tDiag = tdiag - tkron;
@@ -513,6 +546,10 @@ private:
         ierr = CalculateCorrelations_BlockDiag(KronBlocks, gsv_r, do_measurements); CHKERRQ(ierr);
         if (do_measurements && do_corr_matrix) { ierr = CalculateCorrelationMatrix(KronBlocks, gsv_r, NumSitesTotal); CHKERRQ(ierr); }
         if (do_measurements && do_dimer_matrix) { ierr = CalculateDimerMatrix(KronBlocks, gsv_r); CHKERRQ(ierr); }
+        if (do_measurements && do_spectral) {
+            ierr = CalculateSpectralFunction(KronBlocks, H, gsv_r, gse_r, NumSitesTotal, Terms, SysBlockEnl, EnvBlockEnl); CHKERRQ(ierr);
+            ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr);
+        }
         if (do_prediction) {
             /* both candidates: which block grows in the next step is the caller's business (the left one in the first half of a sweep,
                the right one in the second, :996-1088); the transformations that created this step's input blocks are captured now,
@@ -720,6 +757,82 @@ private:
         return 0;
     }
 
+    /** EXTENSION (-do_spectral_function): one record of SpectralFunction.json — the continued-fraction coefficients of the
+        dynamical structure factor from dmrgx_spectral_lanczos.  For every q = (2π kx/Lx, 2π ky/Ly) the start vectors are
+            A_cos psi = Σ_s cos(q·r_s)/√N · O_s psi,   A_sin psi = Σ_s sin(q·r_s)/√N · O_s psi   (superblock site s is lattice site s),
+        so that for a real psi and H  S(q, ω) = S_cos(ω) + S_sin(ω), with S_part(ω) = -Im G_part(ω + E0 + iη) / π and
+        G = norm2 / (z - α_0 - β_1² / (z - α_1 - …)).  zz takes O = Sz under this step's H; pm = <S+ S-> takes O = S- under the H of
+        the sector qn - 1 and mp = <S- S+> takes O = S+ under the H of the sector qn + 1, both built from the enlarged blocks.  An
+        empty shifted sector gives zeros.  Written per operator as [kx][ky] -> {"cos": ..., "sin": ...}, each part holding norm2,
+        steps (the recurrence length) and the first `steps` of alpha and beta (beta[0] = 0).  At equal time,
+        Σ_parts (zz + (pm + mp)/2) norm2 = StructureFactor[kx][ky] of CorrelationMatrix.json. */
+    PetscErrorCode CalculateSpectralFunction(KronBlocks_t& KronBlocks, const ShellMat& H, const Vec& gsv_r, const PetscScalar E0, const PetscInt nsites,
+                                             const std::vector<Hamiltonians::Term>& Terms, Block& SysBlockEnl, Block& EnvBlockEnl) {
+        const PetscInt Lx = Ham.Lx(), Ly = Ham.Ly();
+        const size_t n = (size_t)nsites, nq = (size_t)(Lx * Ly), nvec = 2 * nq, ns = (size_t)spectral_nsteps;
+        std::vector<PetscInt> x(n), y(n);
+        for (size_t s = 0; s < n; ++s) Ham.To2D((PetscInt)s, x[s], y[s]);
+        std::vector<double> coef(nvec * n);
+        for (PetscInt kx = 0; kx < Lx; ++kx)
+            for (PetscInt ky = 0; ky < Ly; ++ky) {
+                const double qx = 2.0 * M_PI * (double)kx / (double)Lx, qy = 2.0 * M_PI * (double)ky / (double)Ly;
+                const size_t v = 2 * (size_t)(kx * Ly + ky);
+                for (size_t s = 0; s < n; ++s) {
+                    const double ph = qx * (double)x[s] + qy * (double)y[s];
+                    coef[v * n + s] = std::cos(ph) / std::sqrt((double)n);
+                    coef[(v + 1) * n + s] = std::sin(ph) / std::sqrt((double)n);
+                }
+            }
+        FILE* f = fp_spectral;
+        fprintf(f, "%s  {\n    \"GlobIdx\": %lld,\n    \"LoopIdx\": %lld,\n    \"E0\": %.17g,\n    \"NSteps\": %lld,\n    \"sites\": [",
+                spectral_records ? ",\n" : "", LLD(GlobIdx), LLD(LoopIdx), E0, LLD(spectral_nsteps));
+        for (size_t s = 0; s < n; ++s) fprintf(f, "%s[%lld, %lld]", s ? ", " : "", LLD(x[s]), LLD(y[s]));
+        fprintf(f, "]");
+        const struct { const char* name; int op; } kinds[3] = {{"zz", DMRGX_OP_SZ}, {"pm", DMRGX_OP_SM}, {"mp", DMRGX_OP_SP}};
+        for (size_t k = 0; k < 3; ++k) {
+            if (!spectral_ops[k]) continue;
+            std::vector<double> alpha(nvec * ns, 0.0), beta(nvec * ns, 0.0), norm2(nvec, 0.0);
+            std::vector<dmrgx_int> steps(nvec, 0);
+            if (kinds[k].op == DMRGX_OP_SZ) {
+                DMRGX_CALL(dmrgx_spectral_lanczos(KronBlocks.Handle(), gsv_r.d, H.h, DMRGX_OP_SZ, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns,
+                                                  alpha.data(), beta.data(), norm2.data(), steps.data(), NULL));
+            } else {
+                KronBlocks_t shifted(SysBlockEnl, EnvBlockEnl, {qn_sector + kinds[k].op}, NULL, GlobIdx);
+                if (shifted.NumStates() > 0) {
+                    ShellMat Hs;
+                    PetscErrorCode ierr = shifted.KronSumConstruct(Terms, Hs); CHKERRQ(ierr);
+                    const int e = dmrgx_spectral_lanczos(KronBlocks.Handle(), gsv_r.d, Hs.h, kinds[k].op, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns,
+                                                         alpha.data(), beta.data(), norm2.data(), steps.data(), NULL);
+                    if (e) fprintf(stderr, "[dmrgx] dmrgx_spectral_lanczos: %s\n", dmrgx_last_error());
+                    ierr = MatDestroy_KronSumShell(&Hs); CHKERRQ(ierr);
+                    if (e) return e;
+                }
+            }
+            fprintf(f, ",\n    \"%s\": [", kinds[k].name);
+            for (PetscInt kx = 0; kx < Lx; ++kx) {
+                fprintf(f, "%s\n      [", kx ? "," : "");
+                for (PetscInt ky = 0; ky < Ly; ++ky) {
+                    fprintf(f, "%s{", ky ? ",\n       " : "");
+                    for (size_t part = 0; part < 2; ++part) {
+                        const size_t v = 2 * (size_t)(kx * Ly + ky) + part;
+                        fprintf(f, "%s\"%s\": {\"norm2\": %.17g, \"steps\": %lld, \"alpha\": [", part ? ", " : "", part ? "sin" : "cos", norm2[v], LLD(steps[v]));
+                        for (dmrgx_int t = 0; t < steps[v]; ++t) fprintf(f, "%s%.17g", t ? ", " : "", alpha[v * ns + (size_t)t]);
+                        fprintf(f, "], \"beta\": [");
+                        for (dmrgx_int t = 0; t < steps[v]; ++t) fprintf(f, "%s%.17g", t ? ", " : "", beta[v * ns + (size_t)t]);
+                        fprintf(f, "]}");
+                    }
+                    fprintf(f, "}");
+                }
+                fprintf(f, "]");
+            }
+            fprintf(f, "\n    ]");
+        }
+        fprintf(f, "\n  }");
+        fflush(f);
+        ++spectral_records;
+        return 0;
+    }
+
     static std::string BlockDir(const std::string& BlockType, const PetscInt& iblock) { /* :2456-2464: "Sys_000000009/" */
         std::ostringstream oss; oss << BlockType << "_" << std::setfill('0') << std::setw(9) << iblock << "/"; return oss.str();
     }
@@ -874,6 +987,11 @@ private:
     PetscBool do_dimer_matrix = PETSC_FALSE;  /* -do_dimer_matrix (extension) */
     FILE* fp_dimer = NULL;
     long long dimer_records = 0;
+    PetscBool do_spectral = PETSC_FALSE;      /* -do_spectral_function (extension) */
+    PetscInt spectral_nsteps = 64;            /* -spectral_nsteps */
+    std::vector<bool> spectral_ops = {true, true, true}; /* -spectral_ops: zz, pm, mp */
+    FILE* fp_spectral = NULL;
+    long long spectral_records = 0;
     PetscScalar gse = 0.0;
     std::vector<PetscReal> trunc_err;
     double t0abs = 0.0;

@@ -220,6 +220,30 @@ int dmrgx_corr_matrix(dmrgx_kron k, const double* d_psi, double* szsz, double* s
 int dmrgx_dimer_matrix(dmrgx_kron k, const double* d_psi, dmrgx_int nbonds, const dmrgx_int* site_i, const dmrgx_int* site_j, double* dd,
                        double* d, double* flops);
 
+/* ---- EXTENSION: the dynamical structure factor by the continued-fraction method (K. Hallberg, PRB 52, R9827 (1995); no reference
+   counterpart).  psi lies in the one total-Sz sector qn of k and is used as given (not normalised); op is DMRGX_OP_SZ, DMRGX_OP_SP
+   or DMRGX_OP_SM, whose value is the sector shift.  Vector v (v < nvec) starts from
+       phi_v = Σ_s coef[v*n+s] · O_s psi      (O = Sz, S+ or S-, superblock sites s < n numbered as in dmrgx_corr_matrix)
+   in the sector qn + op, and h_target is a shell on a kron of the SAME two block objects whose single sector is qn + op (for
+   DMRGX_OP_SZ the step's own Hamiltonian).  From phi_v/‖phi_v‖ a plain three-term Lanczos recurrence of h_target runs, with no
+   reorthogonalisation; its coefficients give  G_v(z) = <phi_v| (z - H)^-1 |phi_v> = norm2[v] / (z - α_0 - β_1²/(z - α_1 - …))
+   and reproduce the moments <phi_v| H^k |phi_v> for k < 2·nsteps.  Host outputs:
+       alpha[v*nsteps+t] = α_t,  beta[v*nsteps+t] = β_t (the coupling of steps t-1 and t, β_0 = 0),  norm2[v] = <phi_v, phi_v>,
+       nsteps_done[v] <= nsteps: the recurrence stops at an invariant subspace, β_{t+1} <= 1e-10·sqrt(α_t² + β_t²); later
+       entries are 0.  A start vector with ‖phi_v‖ <= 1e-12 · Σ_s |coef_s|·‖O_s psi‖ is zero up to rounding: norm2 = 0, no steps.
+   One batched device pass: the n panels O_s psi are one contraction launch, the start vectors of a batch are one GEMM over
+   them, and a batch of nb vectors keeps three columns each on the device (v_prev, v, H·v; nb = 2 GiB / (24·D), at least 1,
+   D the dimension of the sector qn + op).  Every step applies h_target once per vector and advances the whole batch with two
+   launches, with no host synchronisation until the batch is done.  Device memory during the call: (n + 3·nb)·D·8 bytes plus
+   the plans.  Each vector's sums run in a fixed order that does not depend on nb: a vector gives the same bits alone or in a
+   batch.  flops (may be NULL) receives the algorithmic flops: panels + start vectors + nvec·nsteps applies + recurrence.
+   Errors: 62 psi, h_target, coef or an output NULL; 63 op not one of the three, nvec < 1, nsteps < 1 or a coefficient not
+   finite; 56 k has not exactly one sector, or the context is multi-GPU (the sharded apply is collective); 73 h_target is not
+   on the sector qn + op of the same blocks, or a block lacks Sz or Sp at a site with a non-zero coefficient (site in the
+   message). */
+int dmrgx_spectral_lanczos(dmrgx_kron k, const double* d_psi, dmrgx_hshell h_target, int op, dmrgx_int nvec, const double* coef,
+                           dmrgx_int nsteps, double* alpha, double* beta, double* norm2, dmrgx_int* nsteps_done, double* flops);
+
 /* ---- Hamiltonians::J1J2XXZModel_SquareLattice::H(nsites): src/Hamiltonians.cpp:73-122 (host only).
         Returns the number of terms (fills at most maxterms); bc: 0 open, 1 periodic; nsites < 0 = full lattice. ---- */
 dmrgx_int dmrgx_ham_terms(dmrgx_int Lx, dmrgx_int Ly, double J1, double Jz1, double J2, double Jz2, int bcx, int bcy, dmrgx_int nsites,
