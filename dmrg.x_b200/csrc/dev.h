@@ -144,7 +144,7 @@ void run_reduce(Stream*, const ReduceItem* d_items, int nitems, double* y, const
 void fill_random(Stream*, double* x, long long n, unsigned long long seed, long long first = 0);
 /* One fused Gram-Schmidt pass over the basis (a single read of V, deterministic reductions finished by the last block, no
    host involvement):   if d_coef:  w -= Σ_i d_coef[i]·V_i   (in place);   then, on the updated w,
-   if d_dots: d_dots[i] = V_i·w (i < nvec);   if d_nrm2: *d_nrm2 = w·w.   nvec <= 40. */
+   if d_dots: d_dots[i] = V_i·w (i < nvec);   if d_nrm2: *d_nrm2 = w·w.   nvec <= MAX_BASIS. */
 constexpr int MAX_BASIS = 39; /* largest ncv the fused kernels take (eigs_smallest validates -H_eps_ncv against it) */
 void gs_pass(Stream*, const double* V, long long ldv, int nvec, double* w, long long n, const double* d_coef, double* d_dots, double* d_nrm2);
 /* Last step of the two-pass Gram-Schmidt, fused with the normalisation (no reduction, no all-reduce):

@@ -9,6 +9,7 @@
  */
 #include <algorithm>
 #include <cmath>
+#include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <stdexcept>
@@ -35,13 +36,36 @@ void d2d(Stream*, void* d, const void* s, size_t b) { if (b) std::memmove(d, s, 
 void memset0(Stream*, void* d, size_t b) { if (b) std::memset(d, 0, b); }
 void sync(Stream*) {}
 
+/* Preconditions of the sm_100a kernels, checked here so that a host plan the GPU would refuse or mishandle fails on the
+   CPU too.  chain_kernel's Stager keeps the element offsets of a thread's staged elements in 32-bit ints: within one
+   16-deep chunk the farthest is (extent - 1)·ld_row + (min(K, 16) - 1)·ld_k, for A (rows, lda_m, lda_k) and B (columns,
+   ldb_n, ldb_k) of every GEMM segment. */
+static void check_stager(long long ext, long long ld_row, long long ld_k, int K, int item, int seg, const char* op) {
+    const long long far = (ext - 1) * ld_row + (long long)(std::min(K, 16) - 1) * ld_k;
+    if (ld_row < 0 || ld_k < 0 || far > 2147483647LL)
+        throw std::runtime_error("run_chain: item " + std::to_string(item) + " segment " + std::to_string(seg) + ": the " + op +
+                                 " staging offset " + std::to_string(far) + " does not fit the kernel's 32-bit Stager offsets");
+}
+void check_chain_plan(const WorkItem* items, int nitems, const Segment* segs) {
+    for (int w = 0; w < nitems; ++w) {
+        const WorkItem& it = items[w];
+        if (it.tm < 1 || it.tn < 1 || it.tm > TILE || it.tn > TILE) throw std::runtime_error("run_chain: bad tile extents");
+        for (int s = it.seg_begin; s < it.seg_end; ++s) {
+            const Segment& sg = segs[s];
+            if (sg.type != SEG_GEMM || sg.K <= 0) continue;
+            check_stager(it.tm, sg.lda_m, sg.lda_k, sg.K, w, s, "A");
+            check_stager(it.tn, sg.ldb_n, sg.ldb_k, sg.K, w, s, "B");
+        }
+    }
+}
+
 void run_chain(Stream*, const WorkItem* items, int nitems, const Segment* segs, const double* xbase, double* ybase, double* wbase) {
     ++g_launches;
+    check_chain_plan(items, nitems, segs);
     std::vector<double> acc;
     for (int w = 0; w < nitems; ++w) {
         WorkItem it = items[w];
         if (it.c_in_y) it.C = (double*)((char*)(it.c_in_y == 1 ? ybase : wbase) + (size_t)it.C);
-        if (it.tm < 1 || it.tn < 1 || it.tm > TILE || it.tn > TILE) throw std::runtime_error("bad tile extents");
         acc.assign((size_t)it.tm * it.tn, 0.0);
         for (int s = it.seg_begin; s < it.seg_end; ++s) {
             Segment sg = segs[s];
@@ -82,8 +106,13 @@ void run_chain(Stream*, const WorkItem* items, int nitems, const Segment* segs, 
     }
 }
 
-void run_spmm(Stream*, const SpTile* tiles, int ntiles, const SpASlot* aslots, const SpSSlot* sslots, const SpBSlot* bslots, const double* x, double* y, int) {
+void run_spmm(Stream*, const SpTile* tiles, int ntiles, const SpASlot* aslots, const SpSSlot* sslots, const SpBSlot* bslots, const double* x, double* y, int max_nR) {
     ++g_launches;
+    if (ntiles <= 0) return;
+    /* the kernel stages a tile's rows in SP_ROWS·max_nR doubles of shared memory */
+    if (max_nR > SP_MAX_NR) throw std::runtime_error("run_spmm: max_nR " + std::to_string(max_nR) + " exceeds SP_MAX_NR");
+    for (int w = 0; w < ntiles; ++w)
+        if (tiles[w].nR > max_nR || tiles[w].nrows > SP_ROWS) throw std::runtime_error("run_spmm: tile " + std::to_string(w) + " is wider than max_nR or taller than SP_ROWS");
     for (int w = 0; w < ntiles; ++w) {
         const SpTile& tl = tiles[w];
         for (int r = 0; r < tl.nrows; ++r)
@@ -136,6 +165,7 @@ void dot(Stream*, const double* x, const double* y, long long n, double* out) {
 }
 void gs_pass(Stream*, const double* V, long long ldv, int nvec, double* w, long long n, const double* coef, double* dots, double* nrm2) {
     ++g_launches;
+    if (nvec > MAX_BASIS) throw std::runtime_error("gs_pass: nvec " + std::to_string(nvec) + " exceeds MAX_BASIS");
     if (coef) for (int i = 0; i < nvec; ++i) for (long long q = 0; q < n; ++q) w[q] -= coef[i] * V[i * ldv + q];
     if (dots) for (int i = 0; i < nvec; ++i) { double s = 0; for (long long q = 0; q < n; ++q) s += V[i * ldv + q] * w[q]; dots[i] = s; }
     if (nrm2) { double s = 0; for (long long q = 0; q < n; ++q) s += w[q] * w[q]; *nrm2 = s; }
@@ -143,6 +173,7 @@ void gs_pass(Stream*, const double* V, long long ldv, int nvec, double* w, long 
 void gs_final(Stream*, const double* V, long long ldv, int nvec, const double* w, long long n, const double* coef, const double* nrm2_in, double* nrm2_out,
               double* vout) {
     ++g_launches;
+    if (nvec > MAX_BASIS + 1) throw std::runtime_error("gs_final: nvec " + std::to_string(nvec) + " exceeds MAX_BASIS + 1");
     double s = 0;
     for (int i = 0; i < nvec; ++i) s += coef[i] * coef[i];
     const bool skip = s <= GS_REFINE_REL * GS_REFINE_REL * *nrm2_in;
@@ -159,6 +190,7 @@ void scale_inv_norm(Stream*, const double* w, const double* nrm2, double* v, lon
 }
 void ritz_rotate(Stream*, double* V, long long ldv, long long n, int ncv, const double* S, int kk) {
     ++g_launches;
+    if (ncv > MAX_BASIS + 1) throw std::runtime_error("ritz_rotate: ncv " + std::to_string(ncv) + " exceeds MAX_BASIS + 1");
     std::vector<double> v(ncv);
     for (long long q = 0; q < n; ++q) {
         for (int i = 0; i < ncv; ++i) v[i] = V[i * ldv + q];
@@ -240,6 +272,16 @@ void bcast_batch(Stream*, int n, double* const* ptr, const long long* count, con
 }
 
 }  // namespace dev
+/* the chain plan check on its own, for a test of a plan that no buffer of a test could hold: 0, or -1 with the message */
+extern "C" int plancheck_check_chain(const void* items, int nitems, const void* segs, char* msg, int len) {
+    try {
+        dev::check_chain_plan((const dev::WorkItem*)items, nitems, (const dev::Segment*)segs);
+        return 0;
+    } catch (const std::exception& e) {
+        std::snprintf(msg, (size_t)len, "%s", e.what());
+        return -1;
+    }
+}
 extern "C" void plancheck_set_collectives(void (*allreduce)(double*, long long), void (*bcast)(double*, long long, int)) {
     dev::g_allreduce = allreduce;
     dev::g_bcast = bcast;

@@ -5,6 +5,7 @@
  *  lanczos_kernel.  Same passes and stopping rules, plain sequential sums.
  */
 #include <cmath>
+#include <stdexcept>
 
 #include "dev.h"
 
@@ -13,6 +14,8 @@ namespace dev {
 int lanczos_blocks(long long) { return 1; }
 
 void lanczos_batch(Stream*, const LanczosBatch& L, int pass, int t, const double* prev, double* cur, double* y) {
+    /* lanczos_kernel strides column c by ld: shorter columns would overlap */
+    if (L.nb > 0 && L.n > 0 && L.ld < L.n) throw std::runtime_error("lanczos_batch: ld below n");
     for (int col = 0; col < L.nb; ++col) {
         if (L.done[col]) continue;
         double* u = cur + (long long)col * L.ld;
