@@ -342,20 +342,31 @@ class KronBlocks:
         _chk(lib().dmrgx_dimer_matrix(self.h, psi.ptr if psi is not None else None, LL(nb), _p(si), _p(sj), _p(dd), _p(d), C.byref(fl)))
         return {"DD": dd, "D": d, "flops": fl.value}
 
-    def SpectralLanczos(self, psi, target, op, coef, nsteps):
+    def SpectralLanczos(self, psi, target, op, coef, nsteps, overlaps=False):
         """EXTENSION (dmrgx_spectral_lanczos): continued-fraction coefficients of the start vectors phi_v = Σ_s coef[v, s] O_s psi
         (O = Sz, S+ or S- for op = OpSz, OpSp, OpSm; coef an nvec×n array over the superblock sites) under `target`, an HShell on
         the sector qn + op of the same two blocks.  Returns alpha and beta (nvec×nsteps, beta[:, 0] = 0), norm2 (nvec),
-        nsteps_done (nvec) and the algorithmic flops of the call; evaluate G(z) with continued_fraction()."""
+        nsteps_done (nvec) and the algorithmic flops of the call; evaluate G(z) with continued_fraction().
+        overlaps=True (dmrgx_spectral_lanczos_overlaps) also returns overlaps (nvec×nsteps×n): <O_s psi, v_t> of every
+        Lanczos vector with every site's panel, 0 past nsteps_done; evaluate the cross correlations with
+        dynamical_correlation() and time_correlation()."""
         n = self.left.NumSites() + self.right.NumSites()
         c = _d(coef).reshape(-1, n) if np.size(coef) else np.zeros((0, n))
         nvec, nsteps = len(c), int(nsteps)
         alpha = np.zeros((nvec, max(nsteps, 0))); beta = np.zeros((nvec, max(nsteps, 0)))
         norm2 = np.zeros(nvec); done = np.zeros(nvec, np.int64)
         fl = C.c_double()
-        _chk(lib().dmrgx_spectral_lanczos(self.h, psi.ptr if psi is not None else None, target.h if target is not None else None, int(op), LL(nvec),
-                                          _p(c), LL(nsteps), _p(alpha), _p(beta), _p(norm2), _p(done), C.byref(fl)))
-        return {"alpha": alpha, "beta": beta, "norm2": norm2, "nsteps_done": done, "flops": fl.value}
+        args = (self.h, psi.ptr if psi is not None else None, target.h if target is not None else None, int(op), LL(nvec), _p(c), LL(nsteps),
+                _p(alpha), _p(beta), _p(norm2), _p(done))
+        r = {"alpha": alpha, "beta": beta, "norm2": norm2, "nsteps_done": done}
+        if overlaps:
+            ov = np.zeros((nvec, max(nsteps, 0), n))
+            _chk(lib().dmrgx_spectral_lanczos_overlaps(*args, _p(ov), C.byref(fl)))
+            r["overlaps"] = ov
+        else:
+            _chk(lib().dmrgx_spectral_lanczos(*args, C.byref(fl)))
+        r["flops"] = fl.value
+        return r
 
 
 def continued_fraction(alpha, beta, norm2, nsteps_done, z):
@@ -374,6 +385,45 @@ def continued_fraction(alpha, beta, norm2, nsteps_done, z):
     if np.ndim(norm2) == 0:
         G = G[0]
     return G if np.ndim(z) else G[..., 0]
+
+
+def _cross(r, phases):
+    """‖phi_v‖ Σ_t ov[v, t, s]·[f(T_v)]_{t,0} with f(θ) = phases(θ) (one row per evaluation point), through one eigh of T_v"""
+    ov = np.asarray(r["overlaps"], float)
+    nvec, _, n = ov.shape
+    out = None
+    for v in range(nvec):
+        k = int(r["nsteps_done"][v])
+        if k == 0:
+            f = phases(np.zeros(0))
+            res = np.zeros((n, f.shape[0]), f.dtype)
+        else:
+            a, b = np.asarray(r["alpha"][v], float), np.asarray(r["beta"][v], float)
+            th, Y = np.linalg.eigh(np.diag(a[:k]) + np.diag(b[1:k], 1) + np.diag(b[1:k], -1))
+            f = phases(th)                                     # (npoints, k)
+            res = np.sqrt(r["norm2"][v]) * ((ov[v, :k].T @ Y) * Y[0]) @ f.T
+        if out is None:
+            out = np.zeros((nvec, n, res.shape[1]), res.dtype)
+        out[v] = res
+    return out
+
+
+def dynamical_correlation(r, z):
+    """<O_s psi| (z - H)^-1 |phi_v> ≈ ‖phi_v‖ Σ_t ov[v, t, s]·[(z - T_v)^-1]_{t,0} from a SpectralLanczos(..., overlaps=True) result
+    r, as an (nvec, n, len(z)) complex array (z a scalar: (nvec, n)).  With site sources (coef rows e_c) and z = ω + E0 + iη,
+    -Im / π is the site-resolved S_sc(ω) broadened by a Lorentzian of width η.  A vector with 0 steps gives 0."""
+    zz = np.atleast_1d(np.asarray(z, complex))
+    G = _cross(r, lambda th: 1.0 / (zz[:, None] - th[None, :]))
+    return G if np.ndim(z) else G[..., 0]
+
+
+def time_correlation(r, times, e0):
+    """<O_s psi| e^{-i(H - E0)τ} |phi_v> ≈ ‖phi_v‖ Σ_t ov[v, t, s]·[e^{-i(T_v - E0)τ}]_{t,0} for every τ in times, from a
+    SpectralLanczos(..., overlaps=True) result r, as an (nvec, n, len(times)) complex array (a scalar τ: (nvec, n)).  With op Sz
+    and site sources this is G_sc(τ) = <S^z_s(τ) S^z_c>.  A vector with 0 steps gives 0."""
+    tt = np.atleast_1d(np.asarray(times, float))
+    G = _cross(r, lambda th: np.exp(-1j * np.outer(tt, th - e0)))
+    return G if np.ndim(times) else G[..., 0]
 
 
 class HShell:

@@ -356,7 +356,16 @@ int dmrgx_dimer_matrix(dmrgx_kron k, const double* d_psi, dmrgx_int nbonds, cons
 
 int dmrgx_spectral_lanczos(dmrgx_kron k, const double* d_psi, dmrgx_hshell h_target, int op, dmrgx_int nvec, const double* coef, dmrgx_int nsteps,
                            double* alpha, double* beta, double* norm2, dmrgx_int* nsteps_done, double* flops) {
-    return guard([&] { spectral_lanczos(K(k), d_psi, H(h_target), op, nvec, coef, nsteps, alpha, beta, norm2, nsteps_done, flops); });
+    return guard([&] { spectral_lanczos(K(k), d_psi, H(h_target), op, nvec, coef, nsteps, alpha, beta, norm2, nsteps_done, nullptr, flops); });
+}
+
+int dmrgx_spectral_lanczos_overlaps(dmrgx_kron k, const double* d_psi, dmrgx_hshell h_target, int op, dmrgx_int nvec, const double* coef,
+                                    dmrgx_int nsteps, double* alpha, double* beta, double* norm2, dmrgx_int* nsteps_done, double* overlaps,
+                                    double* flops) {
+    return guard([&] {
+        if (!overlaps) throw Err(ERR_ARG_WRONG, "the overlaps array is NULL.");
+        spectral_lanczos(K(k), d_psi, H(h_target), op, nvec, coef, nsteps, alpha, beta, norm2, nsteps_done, overlaps, flops);
+    });
 }
 
 /* microbenchmark of the chain engine on one plain product C[M,N] = A·B (selectable operand layouts), for profiling */

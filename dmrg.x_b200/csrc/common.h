@@ -251,8 +251,9 @@ void corr_matrix(const Kron*, const double* d_psi, double* szsz, double* spsm, d
 /* corr.cpp: the bond–bond correlators of nb isotropic bonds (extension; host nb×nb and nb outputs) */
 void dimer_matrix(const Kron*, const double* d_psi, long long nb, const long long* bond_i, const long long* bond_j, double* dd, double* d,
                   double* flops);
-/* corr.cpp: continued-fraction (Lanczos) coefficients of nvec start vectors Σ_s coef_s O_s psi under the target shell (extension) */
+/* corr.cpp: continued-fraction (Lanczos) coefficients of nvec start vectors Σ_s coef_s O_s psi under the target shell (extension);
+   overlaps (nvec × nsteps × n, may be NULL): <O_s psi, v_t> of every Lanczos vector with every single-site panel */
 void spectral_lanczos(const Kron*, const double* d_psi, HShell* h_target, int op, long long nvec, const double* coef, long long nsteps,
-                      double* alpha, double* beta, double* norm2, long long* nsteps_done, double* flops);
+                      double* alpha, double* beta, double* norm2, long long* nsteps_done, double* overlaps, double* flops);
 
 }  // namespace dmrgx

@@ -18,7 +18,9 @@
  *  The spectral recurrence (continued-fraction method, K. Hallberg, PRB 52, R9827 (1995)) starts from  phi_v = Σ_s coef[v][s] O_s psi
  *  in the sector qn + op: the n single-operator panels are one chain-kernel plan, the start vectors of a batch are one GEMM
  *  plan  Phi = C·P  over them, and every vector then runs a plain three-term Lanczos recurrence of the target shell, the whole
- *  batch advanced by dev::lanczos_batch with no host synchronisation until the batch is finished.
+ *  batch advanced by dev::lanczos_batch with no host synchronisation until the batch is finished.  With overlaps, every step
+ *  also takes the rectangular Gram block <O_s psi, v_t> of the n panels against the batch's freshly normalised Lanczos vectors
+ *  (dev::gram_rect), from which any matrix element <O_s psi| f(H) |phi_v> follows on the host.
  */
 #include <algorithm>
 #include <cmath>
@@ -255,7 +257,7 @@ constexpr double SPECTRAL_BATCH_BYTES = 2.0 * (1LL << 30);
 constexpr double SPECTRAL_ZERO_REL = 1e-12;
 
 void spectral_lanczos(const Kron* kron, const double* d_psi, HShell* h, int op, long long nvec, const double* coef, long long nsteps,
-                      double* alpha, double* beta, double* norm2, long long* nsteps_done, double* flops) {
+                      double* alpha, double* beta, double* norm2, long long* nsteps_done, double* overlaps, double* flops) {
     if (!d_psi) throw Err(ERR_ARG_WRONG, "psi is NULL.");
     if (!h) throw Err(ERR_ARG_WRONG, "the target shell is NULL.");
     if (!coef) throw Err(ERR_ARG_WRONG, "the coefficient array is NULL.");
@@ -278,7 +280,8 @@ void spectral_lanczos(const Kron* kron, const double* d_psi, HShell* h, int op, 
     if (tk->L != L || tk->R != R || tq.size() != 1 || *tq.begin() != qn + op)
         throw Err(ERR_ARG_WRONGSTATE, "the target shell must be built on a Kron of the same two blocks whose single sector is qn + op = " +
                                           std::to_string(qn + op) + ".");
-    std::vector<char> used(n, 0);
+    /* the overlaps are taken against every site's panel, so each site then needs its operators */
+    std::vector<char> used(n, overlaps ? 1 : 0);
     for (long long i = 0; i < nvec * n; ++i)
         if (coef[i] != 0.0) used[i % n] = 1;
     for (int s = 0; s < n; ++s)
@@ -287,6 +290,7 @@ void spectral_lanczos(const Kron* kron, const double* d_psi, HShell* h, int op, 
     std::fill(beta, beta + nvec * nsteps, 0.0);
     std::fill(norm2, norm2 + nvec, 0.0);
     std::fill(nsteps_done, nsteps_done + nvec, 0LL);
+    if (overlaps) std::fill(overlaps, overlaps + nvec * nsteps * n, 0.0);
     const long long D = tk->nstates(), ld = (D + 1) & ~1LL;
     double total = 0;
     if (D > 0) {
@@ -327,6 +331,8 @@ void spectral_lanczos(const Kron* kron, const double* d_psi, HShell* h, int op, 
         lb.zero2 = zero2; lb.partials = zero2 + nb;
         lb.ndone = ints->as<long long>(); lb.done = (int*)(lb.ndone + nb); lb.tickets = (unsigned int*)(lb.done + nb);
         dev::memset0(st, lb.tickets, (size_t)nb * 4);
+        /* overlaps of a batch on the device, [c][t][s]: column c of step t's Gram block at ov + t·n, stride nsteps·n */
+        BufRef ovb = overlaps ? std::make_shared<DevBuf>(ctx, (size_t)((long long)nb * nsteps * n) * 8) : nullptr;
         std::vector<double> hz(nb);
         for (long long b0 = 0; b0 < nvec; b0 += nb) {
             const int m = (int)std::min<long long>(nb, nvec - b0);
@@ -357,6 +363,8 @@ void spectral_lanczos(const Kron* kron, const double* d_psi, HShell* h, int op, 
             for (long long t = 0; t < nsteps; ++t) {
                 for (int c = 0; c < m; ++c) hshell_apply(h, slot[ic] + (long long)c * ld, slot[iy] + (long long)c * ld);
                 dev::lanczos_batch(st, lb, 1, (int)t, slot[ip], slot[ic], slot[iy]);
+                /* pass 1 has just normalised v_t in place; a done column's slot is stale, and only its own entries see it */
+                if (overlaps) dev::gram_rect(st, P, ld, n, slot[ic], ld, m, D, ovb->as<double>() + t * n, 1, nsteps * n);
                 if (t + 1 < nsteps) {
                     dev::lanczos_batch(st, lb, 2, (int)t, slot[ip], slot[ic], slot[iy]);
                     rotate();
@@ -366,9 +374,14 @@ void spectral_lanczos(const Kron* kron, const double* d_psi, HShell* h, int op, 
             dev::d2h(st, beta + b0 * nsteps, lb.beta, (size_t)m * nsteps * 8);
             dev::d2h(st, norm2 + b0, lb.norm2, (size_t)m * 8);
             dev::d2h(st, nsteps_done + b0, lb.ndone, (size_t)m * 8);
+            if (overlaps) dev::d2h(st, overlaps + b0 * nsteps * n, ovb->p, (size_t)((long long)m * nsteps * n) * 8);
             dev::sync(st); /* the combine plan and hz are reused by the next batch */
+            if (overlaps)
+                for (long long c = b0; c < b0 + m; ++c)
+                    std::fill(overlaps + (c * nsteps + nsteps_done[c]) * n, overlaps + (c + 1) * nsteps * n, 0.0);
         }
         total += (double)nvec * (double)nsteps * h->alg_flops + (double)nvec * (10.0 * (double)nsteps + 2.0) * (double)D;
+        if (overlaps) total += (double)nvec * (double)nsteps * 2.0 * (double)n * (double)D;
     }
     if (flops) *flops = total;
 }

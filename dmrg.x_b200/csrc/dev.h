@@ -166,6 +166,12 @@ void dot(Stream*, const double* x, const double* y, long long n, double* d_out);
    the rows are cut into fixed slabs whose partial tiles are summed in a fixed order (no atomics: two calls on the same
    data give the same bits), then mirrored.  Two launches. */
 void gram(Stream*, const double* P, long long ldp, int np, long long n, double* d_G);
+/* Rectangular Gram matrix of two column panels: d_G[i·gs + j·gc] = Σ_{r<n} P[i][r]·Q[j][r] for i < np, j < nq, columns
+   P + i·ldp and Q + j·ldq (gram's alignment preconditions for both).  gram's tiles, slabs and fixed slab order, every tile
+   computed; the bits of G[i][j] depend only on column i of P, column j of Q and n, never on np, nq or the tile that holds
+   them.  n <= 0 writes zeros.  Two launches. */
+void gram_rect(Stream*, const double* P, long long ldp, int np, const double* Q, long long ldq, int nq, long long n, double* d_G, long long gs,
+               long long gc);
 
 /* Plain three-term Lanczos recurrence over nb independent columns (spectral.cpp), all state on the device.  Column c of a
    slot is slot + c·ld, rows [0, n).  The caller keeps three slots per column and rotates them (prev, cur, y) <- (cur, y, prev)

@@ -69,6 +69,7 @@ struct Stream {
     int spmm_smem = 0;           /* dynamic shared memory spmm_kernel has been configured for on this device */
     bool chain_cfg = false;      /* chain_kernel's dynamic shared memory attribute has been set on this device */
     bool gram_cfg = false;       /* the same for gram_kernel */
+    bool gram_rect_cfg = false;  /* the same for gram_kernel<true> (gram_rect) */
     cudaStream_t aux = nullptr;  /* side stream: the small-block eigensolver runs beside the block-Jacobi launches */
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
 };
@@ -909,6 +910,10 @@ void dot(Stream* st, const double* x, const double* y, long long n, double* d_ou
  *  partials are summed in shared memory in warp order.  The slab partial is written to a scratch area; gram_reduce_kernel
  *  sums the slabs in index order and writes both G[i][j] and G[j][i] from the same sum.  The columns are contiguous, so
  *  the arithmetic intensity is set by the tile width: about 4 flop per byte staged, ~np/4 per byte of DRAM traffic.
+ *  RECT (gram_rect): G = PᵀQ of two panels, one CTA per (32×32 tile of every row tile of P × column tile of Q, slab), the same
+ *  staging and DMMA body with no diagonal tile; gram_rect_reduce_kernel sums the slabs in index order into strided G.  An
+ *  element's accumulator position, warp rows and slab order do not depend on np, nq or its tile, so its bits depend only on
+ *  its two columns and n.
  * ============================================================================================== */
 constexpr int GR_T = 32, GR_BK = 64, GR_S = GR_BK + 4 /* ≡ 4 mod 16: conflict-free fragment reads */, GR_THREADS = 128;
 constexpr long long GR_SLAB = 8192;
@@ -919,14 +924,20 @@ __device__ __forceinline__ void cp_async16(double* smem_dst, const double* gsrc,
     asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;\n" ::"r"(s), "l"(gsrc), "r"(src_bytes));
 }
 
-__global__ void __launch_bounds__(GR_THREADS) gram_kernel(const double* __restrict__ P, long long ldp, int np, long long n, int nt, int ntri,
-                                                          double* __restrict__ part) {
+/* symmetric (RECT false): Q = P, nt tiles per side, ntri tiles on or above the diagonal; RECT: nt = the tiles of Q, ntri = all tiles */
+template <bool RECT>
+__global__ void __launch_bounds__(GR_THREADS) gram_kernel(const double* __restrict__ P, long long ldp, int np, const double* __restrict__ Q, long long ldq,
+                                                          int nq, long long n, int nt, int ntri, double* __restrict__ part) {
     extern __shared__ __align__(16) double gr_smem[];
     const int tri = blockIdx.x % ntri, slab = blockIdx.x / ntri;
-    int ti = 0, r = tri;
-    while (r >= nt - ti) { r -= nt - ti; ++ti; }
-    const int tj = ti + r;
-    const bool diag = ti == tj;
+    int ti = 0, tj = 0;
+    if (RECT) { ti = tri / nt; tj = tri % nt; }
+    else {
+        int r = tri;
+        while (r >= nt - ti) { r -= nt - ti; ++ti; }
+        tj = ti + r;
+    }
+    const bool diag = !RECT && ti == tj;
     const long long r0 = (long long)slab * GR_SLAB, r1 = min(n, r0 + GR_SLAB);
     const int nchunks = (int)((r1 - r0 + GR_BK - 1) / GR_BK);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
@@ -939,7 +950,7 @@ __global__ void __launch_bounds__(GR_THREADS) gram_kernel(const double* __restri
     for (int i = 0; i < 8; ++i) {
         const int q = tid + GR_THREADS * i, col = q >> 5, pr = q & 31;
         srcA[i] = P + (long long)min(ti * GR_T + col, np - 1) * ldp + r0 + 2 * pr;
-        srcB[i] = P + (long long)min(tj * GR_T + col, np - 1) * ldp + r0 + 2 * pr;
+        srcB[i] = Q + (long long)min(tj * GR_T + col, nq - 1) * ldq + r0 + 2 * pr;
     }
     auto issue = [&](int c) {
         double* as = gr_smem + (c & 1) * GR_STAGE;
@@ -953,7 +964,7 @@ __global__ void __launch_bounds__(GR_THREADS) gram_kernel(const double* __restri
             const int bytes = left >= 2 ? 16 : (left == 1 ? 8 : 0);
             const long long adv = (long long)c * GR_BK;
             cp_async16(as + col * GR_S + 2 * pr, bytes ? srcA[i] + adv : P, bytes);
-            if (!diag) cp_async16(bs + col * GR_S + 2 * pr, bytes ? srcB[i] + adv : P, bytes);
+            if (!diag) cp_async16(bs + col * GR_S + 2 * pr, bytes ? srcB[i] + adv : Q, bytes);
         }
     };
 
@@ -1027,15 +1038,50 @@ void gram(Stream* st, const double* P, long long ldp, int np, long long n, doubl
     constexpr int smem = 2 * GR_STAGE * (int)sizeof(double);
     static_assert(4 * GR_T * GR_T <= 2 * GR_STAGE, "the warp partials reuse the staging buffers");
     if (!st->gram_cfg) {
-        CUDA_OK(cudaFuncSetAttribute(gram_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+        CUDA_OK(cudaFuncSetAttribute(gram_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         st->gram_cfg = true;
     }
     double* part = (double*)malloc_bytes(st, sizeof(double) * nslabs * ntri * GR_T * GR_T);
-    gram_kernel<<<(unsigned)(nslabs * ntri), GR_THREADS, smem, st->s>>>(P, ldp, np, n, nt, ntri, part);
+    gram_kernel<false><<<(unsigned)(nslabs * ntri), GR_THREADS, smem, st->s>>>(P, ldp, np, P, ldp, np, n, nt, ntri, part);
     LAUNCH_CHECK();
     gram_reduce_kernel<<<(unsigned)(((long long)np * np + 255) / 256), 256, 0, st->s>>>(part, np, nt, ntri, (int)nslabs, d_G);
     LAUNCH_CHECK();
     free_bytes(st, part); /* stream-ordered heap: the next user of the range is queued behind the reduction */
+}
+
+__global__ void __launch_bounds__(256) gram_rect_reduce_kernel(const double* __restrict__ part, int np, int nq, int ntq, int ntiles, int nslabs,
+                                                               double* __restrict__ G, long long gs, long long gc) {
+    const long long e = (long long)blockIdx.x * 256 + threadIdx.x;
+    if (e >= (long long)np * nq) return;
+    const int i = (int)(e / nq), j = (int)(e % nq);
+    const double* p = part + (long long)((i / GR_T) * ntq + j / GR_T) * (GR_T * GR_T) + (i % GR_T) * GR_T + (j % GR_T);
+    double s = 0.0;
+    for (int k = 0; k < nslabs; ++k) s += p[(long long)k * ntiles * (GR_T * GR_T)];
+    G[i * gs + j * gc] = s;
+}
+
+void gram_rect(Stream* st, const double* P, long long ldp, int np, const double* Q, long long ldq, int nq, long long n, double* d_G, long long gs,
+               long long gc) {
+    if (np <= 0 || nq <= 0) return;
+    if ((ldp & 1) || (ldq & 1) || ((uintptr_t)P & 15) || ((uintptr_t)Q & 15))
+        throw std::runtime_error("gram_rect: columns must be 16-byte aligned (P and Q aligned, ldp and ldq even)");
+    const int ntp = (np + GR_T - 1) / GR_T, ntq = (nq + GR_T - 1) / GR_T, ntiles = ntp * ntq;
+    const long long nslabs = n > 0 ? (n + GR_SLAB - 1) / GR_SLAB : 0;
+    constexpr int smem = 2 * GR_STAGE * (int)sizeof(double);
+    double* part = nullptr;
+    if (nslabs > 0) {
+        if (!st->gram_rect_cfg) {
+            CUDA_OK(cudaFuncSetAttribute(gram_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+            st->gram_rect_cfg = true;
+        }
+        part = (double*)malloc_bytes(st, sizeof(double) * nslabs * ntiles * GR_T * GR_T);
+        gram_kernel<true><<<(unsigned)(nslabs * ntiles), GR_THREADS, smem, st->s>>>(P, ldp, np, Q, ldq, nq, n, ntq, ntiles, part);
+        LAUNCH_CHECK();
+    }
+    /* n <= 0: no slab, every element written as 0 */
+    gram_rect_reduce_kernel<<<(unsigned)(((long long)np * nq + 255) / 256), 256, 0, st->s>>>(part, np, nq, ntq, ntiles, (int)nslabs, d_G, gs, gc);
+    LAUNCH_CHECK();
+    if (part) free_bytes(st, part);
 }
 
 /* ================================================================================================

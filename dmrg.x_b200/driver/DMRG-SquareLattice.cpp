@@ -3,8 +3,9 @@
  *      DMRG-SquareLattice.x -Lx 12 -Ly 6 -J1 0.5 -Jz1 1 -J2 0.25 -Jz2 0.5 -mwarmup 128 -msweeps 512,1024,2048 \
  *                           [-H_eps_tol 1e-12] [-data_dir out/] [-device 0] [-verbose] [-wavefunction_prediction 1] [-do_correlation_matrix 1]
  *                           [-do_dimer_matrix 1] [-do_spectral_function 1 [-spectral_nsteps 64] [-spectral_ops zz,pm,mp]]
+ *                           [-do_dynamical_correlations 1 [-dynamical_sources i,j,...]]
  *
- *  Same options (plus -device and the opt-in -wavefunction_prediction, -do_correlation_matrix, -do_dimer_matrix and -do_spectral_function, which the reference does not have), same stdout banner, same JSON files; one process drives one B200 through the C ABI
+ *  Same options (plus -device and the opt-in -wavefunction_prediction, -do_correlation_matrix, -do_dimer_matrix, -do_spectral_function and -do_dynamical_correlations, which the reference does not have), same stdout banner, same JSON files; one process drives one B200 through the C ABI
  *  (include/dmrgx.h).  There is no CPU path: without a CUDA device the context creation fails and the
  *  program exits non-zero.
  */
@@ -15,7 +16,13 @@ static char help[] = "DMRG executable for the Spin-1/2 J1-J2 XY Model on a two-d
                      "                             dimer structure factors of the x and y bonds -> DimerMatrix.json\n"
                      "  -do_spectral_function 1    continued-fraction coefficients of the dynamical structure factor S(q, w) on\n"
                      "                             the Lx x Ly momentum grid -> SpectralFunction.json (single-GPU runs only)\n"
-                     "  -spectral_nsteps N         Lanczos steps per momentum and operator (default 64)\n"
+                     "  -do_dynamical_correlations 1\n"
+                     "                             the real-space dynamical correlation matrix <O_s| f(H) |O_c> (S_ij(w), G_ij(t))\n"
+                     "                             from single-site sources c: Lanczos coefficients and the overlaps of every\n"
+                     "                             Lanczos vector with every site -> DynamicalCorrelations.json (single-GPU runs\n"
+                     "                             only; about 20 MB per record at 12x6 with 64 steps and every site a source)\n"
+                     "  -dynamical_sources i,j,... the source sites (default every site; a central column is the usual cheap choice)\n"
+                     "  -spectral_nsteps N         Lanczos steps per momentum / source and operator (default 64)\n"
                      "  -spectral_ops zz,pm,mp     which of <Sz Sz>, <S+ S->, <S- S+> to compute (default all three)\n";
 
 #include <unistd.h>

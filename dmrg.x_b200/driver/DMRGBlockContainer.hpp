@@ -158,12 +158,34 @@ public:
             }
             if (!any) SETERRQ(mpi_comm, PETSC_ERR_ARG_WRONG, "-spectral_ops: the list is empty (the items are zz, pm and mp).");
         }
+        /* EXTENSION, off by default: the real-space dynamical correlation matrix <O_s psi| f(H) |O_c psi> from single-site sources c
+           at every measurement step, in DynamicalCorrelations.json (-spectral_nsteps, -spectral_ops); rank 0 of a single-GPU run */
+        o.GetBool("-do_dynamical_correlations", &do_dyncorr, NULL);
+        if (o.Has("-dynamical_sources")) {
+            std::string list;
+            o.GetString("-dynamical_sources", list, NULL);
+            for (char& c : list) if (c == ',') c = ' ';
+            std::istringstream iss(list);
+            std::set<PetscInt> seen;
+            for (std::string item; iss >> item;) {
+                size_t end = 0;
+                long long v = -1;
+                try { v = std::stoll(item, &end); } catch (...) { end = 0; }
+                if (end != item.size() || v < 0 || v >= (long long)num_sites)
+                    SETERRQ2(mpi_comm, PETSC_ERR_ARG_WRONG, "-dynamical_sources: '%s' is not a site index in [0, %lld).", item.c_str(), LLD(num_sites));
+                if (!seen.insert((PetscInt)v).second) SETERRQ1(mpi_comm, PETSC_ERR_ARG_WRONG, "-dynamical_sources: site %lld is listed twice.", v);
+                dyncorr_sources.push_back((PetscInt)v);
+            }
+            if (dyncorr_sources.empty()) SETERRQ(mpi_comm, PETSC_ERR_ARG_WRONG, "-dynamical_sources: the list is empty.");
+        }
         {
             int rank = 0, world = 1;
             dmrgx_ctx_rank(DmrgxContext(), &rank, &world);
             /* the recurrence applies H on one GPU; the sharded apply is collective and a rank-0-only pass cannot use it */
             if (world > 1 && do_spectral) SETERRQ1(mpi_comm, PETSC_ERR_SUP, "-do_spectral_function runs on one GPU only (this run has %d ranks).", world);
-            if (rank != 0) do_corr_matrix = do_dimer_matrix = do_spectral = PETSC_FALSE;
+            if (world > 1 && do_dyncorr)
+                SETERRQ1(mpi_comm, PETSC_ERR_SUP, "-do_dynamical_correlations runs on one GPU only (this run has %d ranks).", world);
+            if (rank != 0) do_corr_matrix = do_dimer_matrix = do_spectral = do_dyncorr = PETSC_FALSE;
         }
         if (do_corr_matrix) {
             fp_corrmat = fopen((data_dir + "CorrelationMatrix.json").c_str(), "w");
@@ -182,6 +204,12 @@ public:
             if (!fp_spectral) SETERRQ1(mpi_comm, 1, "cannot open %sSpectralFunction.json", data_dir.c_str());
             fprintf(fp_spectral, "[\n");
             fflush(fp_spectral);
+        }
+        if (do_dyncorr) {
+            fp_dyncorr = fopen((data_dir + "DynamicalCorrelations.json").c_str(), "w");
+            if (!fp_dyncorr) SETERRQ1(mpi_comm, 1, "cannot open %sDynamicalCorrelations.json", data_dir.c_str());
+            fprintf(fp_dyncorr, "[\n");
+            fflush(fp_dyncorr);
         }
         SaveStepHeaders(); fprintf(fp_step, "[\n");
         SaveTimingsHeaders(); fprintf(fp_timings, "[\n");
@@ -248,6 +276,7 @@ public:
         if (fp_corrmat) { fprintf(fp_corrmat, "\n]\n"); fclose(fp_corrmat); fp_corrmat = NULL; }
         if (fp_dimer) { fprintf(fp_dimer, "\n]\n"); fclose(fp_dimer); fp_dimer = NULL; }
         if (fp_spectral) { fprintf(fp_spectral, "\n]\n"); fclose(fp_spectral); fp_spectral = NULL; }
+        if (fp_dyncorr) { fprintf(fp_dyncorr, "\n]\n"); fclose(fp_dyncorr); fp_dyncorr = NULL; }
         init = PETSC_FALSE;
         return 0;
     }
@@ -526,8 +555,9 @@ private:
         total_matvecs += eps_stats.nmatvec;
         double h_bytes = 0, h_flops = 0;
         { dmrgx_int hn, hnt, t1, t2; dmrgx_hshell_stats(H.h, &hn, &hnt, &h_bytes, &h_flops, &t1, &t2); }
-        /* -do_spectral_function: the zz recurrence runs on this step's H, which then lives until the measurement */
-        if (!(do_measurements && do_spectral)) { ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr); }
+        /* -do_spectral_function, -do_dynamical_correlations: the zz recurrence runs on this step's H, which then lives until the
+           measurement */
+        if (!(do_measurements && (do_spectral || do_dyncorr))) { ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr); }
         const double tdiag = Tick();
         total_matvec_flops += h_flops * (double)eps_stats.nmatvec;
         timings_data.tDiag = tdiag - tkron;
@@ -548,8 +578,11 @@ private:
         if (do_measurements && do_dimer_matrix) { ierr = CalculateDimerMatrix(KronBlocks, gsv_r); CHKERRQ(ierr); }
         if (do_measurements && do_spectral) {
             ierr = CalculateSpectralFunction(KronBlocks, H, gsv_r, gse_r, NumSitesTotal, Terms, SysBlockEnl, EnvBlockEnl); CHKERRQ(ierr);
-            ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr);
         }
+        if (do_measurements && do_dyncorr) {
+            ierr = CalculateDynamicalCorrelations(KronBlocks, H, gsv_r, gse_r, NumSitesTotal, Terms, SysBlockEnl, EnvBlockEnl); CHKERRQ(ierr);
+        }
+        if (do_measurements && (do_spectral || do_dyncorr)) { ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr); }
         if (do_prediction) {
             /* both candidates: which block grows in the next step is the caller's business (the left one in the first half of a sweep,
                the right one in the second, :996-1088); the transformations that created this step's input blocks are captured now,
@@ -757,6 +790,27 @@ private:
         return 0;
     }
 
+    /** The target shell of the recurrences of op at this step, handed to `call` (which returns a dmrgx code): this step's H for
+        Sz, else a shell on the sector qn + op built from the enlarged blocks and destroyed afterwards.  An empty shifted sector
+        makes no call, so its outputs stay zero. */
+    template <class F>
+    PetscErrorCode WithSpectralTarget(const ShellMat& H, int op, const std::vector<Hamiltonians::Term>& Terms, Block& SysBlockEnl, Block& EnvBlockEnl,
+                                      const char* what, F&& call) {
+        if (op == DMRGX_OP_SZ) {
+            const int e = call(H.h);
+            if (e) fprintf(stderr, "[dmrgx] %s -> %d: %s\n", what, e, dmrgx_last_error());
+            return e;
+        }
+        KronBlocks_t shifted(SysBlockEnl, EnvBlockEnl, {qn_sector + op}, NULL, GlobIdx);
+        if (shifted.NumStates() == 0) return 0;
+        ShellMat Hs;
+        PetscErrorCode ierr = shifted.KronSumConstruct(Terms, Hs); CHKERRQ(ierr);
+        const int e = call(Hs.h);
+        if (e) fprintf(stderr, "[dmrgx] %s: %s\n", what, dmrgx_last_error());
+        ierr = MatDestroy_KronSumShell(&Hs); CHKERRQ(ierr);
+        return e;
+    }
+
     /** EXTENSION (-do_spectral_function): one record of SpectralFunction.json — the continued-fraction coefficients of the
         dynamical structure factor from dmrgx_spectral_lanczos.  For every q = (2π kx/Lx, 2π ky/Ly) the start vectors are
             A_cos psi = Σ_s cos(q·r_s)/√N · O_s psi,   A_sin psi = Σ_s sin(q·r_s)/√N · O_s psi   (superblock site s is lattice site s),
@@ -793,21 +847,11 @@ private:
             if (!spectral_ops[k]) continue;
             std::vector<double> alpha(nvec * ns, 0.0), beta(nvec * ns, 0.0), norm2(nvec, 0.0);
             std::vector<dmrgx_int> steps(nvec, 0);
-            if (kinds[k].op == DMRGX_OP_SZ) {
-                DMRGX_CALL(dmrgx_spectral_lanczos(KronBlocks.Handle(), gsv_r.d, H.h, DMRGX_OP_SZ, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns,
-                                                  alpha.data(), beta.data(), norm2.data(), steps.data(), NULL));
-            } else {
-                KronBlocks_t shifted(SysBlockEnl, EnvBlockEnl, {qn_sector + kinds[k].op}, NULL, GlobIdx);
-                if (shifted.NumStates() > 0) {
-                    ShellMat Hs;
-                    PetscErrorCode ierr = shifted.KronSumConstruct(Terms, Hs); CHKERRQ(ierr);
-                    const int e = dmrgx_spectral_lanczos(KronBlocks.Handle(), gsv_r.d, Hs.h, kinds[k].op, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns,
-                                                         alpha.data(), beta.data(), norm2.data(), steps.data(), NULL);
-                    if (e) fprintf(stderr, "[dmrgx] dmrgx_spectral_lanczos: %s\n", dmrgx_last_error());
-                    ierr = MatDestroy_KronSumShell(&Hs); CHKERRQ(ierr);
-                    if (e) return e;
-                }
-            }
+            PetscErrorCode ierr = WithSpectralTarget(H, kinds[k].op, Terms, SysBlockEnl, EnvBlockEnl, "dmrgx_spectral_lanczos", [&](dmrgx_hshell t) {
+                return dmrgx_spectral_lanczos(KronBlocks.Handle(), gsv_r.d, t, kinds[k].op, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns, alpha.data(),
+                                              beta.data(), norm2.data(), steps.data(), NULL);
+            });
+            if (ierr) return ierr;
             fprintf(f, ",\n    \"%s\": [", kinds[k].name);
             for (PetscInt kx = 0; kx < Lx; ++kx) {
                 fprintf(f, "%s\n      [", kx ? "," : "");
@@ -830,6 +874,69 @@ private:
         fprintf(f, "\n  }");
         fflush(f);
         ++spectral_records;
+        return 0;
+    }
+
+    /** EXTENSION (-do_dynamical_correlations): one record of DynamicalCorrelations.json — the real-space dynamical correlation
+        matrix from dmrgx_spectral_lanczos_overlaps.  Each source c (-dynamical_sources, default every site) starts one recurrence
+        from O_c psi (coef row e_c) under the targets of CalculateSpectralFunction (zz: O = Sz under this step's H; pm: O = S- under
+        the H of the sector qn - 1; mp: O = S+ under the H of qn + 1), and keeps the overlap of every Lanczos vector v_t with every
+        site's panel O_s psi.  With T the tridiagonal matrix of alpha and beta and ‖O_c psi‖ = √norm2,
+            <O_s psi| f(H) |O_c psi> = √norm2 Σ_t overlaps[t][s] f(T)_{t,0}
+        exactly for f(H) = H^k, k < steps, and approximately for (z - H)^-1 (S_sc(ω) at z = ω + E0 + iη) and e^{-i(H - E0)τ}
+        (G_sc(τ) = <S_s(τ) S_c>).  Written per operator as one entry per source: site, norm2, steps, the first `steps` of alpha
+        and beta (beta[0] = 0) and `steps` rows of n overlaps.  At 12×6 with every site as a source and 64 steps a record holds
+        about 3·72·64·72 numbers (some 20 MB); -dynamical_sources shrinks it in proportion. */
+    PetscErrorCode CalculateDynamicalCorrelations(KronBlocks_t& KronBlocks, const ShellMat& H, const Vec& gsv_r, const PetscScalar E0, const PetscInt nsites,
+                                                  const std::vector<Hamiltonians::Term>& Terms, Block& SysBlockEnl, Block& EnvBlockEnl) {
+        const size_t n = (size_t)nsites, ns = (size_t)spectral_nsteps;
+        std::vector<PetscInt> src = dyncorr_sources;
+        if (src.empty())
+            for (PetscInt s = 0; s < nsites; ++s) src.push_back(s);
+        for (const PetscInt c : src)
+            if (c >= nsites) SETERRQ2(mpi_comm, 1, "-dynamical_sources: site %lld is not in this %lld-site superblock.", LLD(c), LLD(nsites));
+        const size_t nvec = src.size();
+        std::vector<double> coef(nvec * n, 0.0);
+        for (size_t v = 0; v < nvec; ++v) coef[v * n + (size_t)src[v]] = 1.0;
+        std::vector<PetscInt> x(n), y(n);
+        for (size_t s = 0; s < n; ++s) Ham.To2D((PetscInt)s, x[s], y[s]);
+        FILE* f = fp_dyncorr;
+        fprintf(f, "%s  {\n    \"GlobIdx\": %lld,\n    \"LoopIdx\": %lld,\n    \"E0\": %.17g,\n    \"NSteps\": %lld,\n    \"sites\": [",
+                dyncorr_records ? ",\n" : "", LLD(GlobIdx), LLD(LoopIdx), E0, LLD(spectral_nsteps));
+        for (size_t s = 0; s < n; ++s) fprintf(f, "%s[%lld, %lld]", s ? ", " : "", LLD(x[s]), LLD(y[s]));
+        fprintf(f, "],\n    \"sources\": [");
+        for (size_t v = 0; v < nvec; ++v) fprintf(f, "%s%lld", v ? ", " : "", LLD(src[v]));
+        fprintf(f, "]");
+        const struct { const char* name; int op; } kinds[3] = {{"zz", DMRGX_OP_SZ}, {"pm", DMRGX_OP_SM}, {"mp", DMRGX_OP_SP}};
+        for (size_t k = 0; k < 3; ++k) {
+            if (!spectral_ops[k]) continue;
+            std::vector<double> alpha(nvec * ns, 0.0), beta(nvec * ns, 0.0), norm2(nvec, 0.0), ov(nvec * ns * n, 0.0);
+            std::vector<dmrgx_int> steps(nvec, 0);
+            PetscErrorCode ierr = WithSpectralTarget(H, kinds[k].op, Terms, SysBlockEnl, EnvBlockEnl, "dmrgx_spectral_lanczos_overlaps", [&](dmrgx_hshell t) {
+                return dmrgx_spectral_lanczos_overlaps(KronBlocks.Handle(), gsv_r.d, t, kinds[k].op, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns,
+                                                       alpha.data(), beta.data(), norm2.data(), steps.data(), ov.data(), NULL);
+            });
+            if (ierr) return ierr;
+            fprintf(f, ",\n    \"%s\": [", kinds[k].name);
+            for (size_t v = 0; v < nvec; ++v) {
+                fprintf(f, "%s\n      {\"site\": %lld, \"norm2\": %.17g, \"steps\": %lld, \"alpha\": [", v ? "," : "", LLD(src[v]), norm2[v], LLD(steps[v]));
+                for (dmrgx_int t = 0; t < steps[v]; ++t) fprintf(f, "%s%.17g", t ? ", " : "", alpha[v * ns + (size_t)t]);
+                fprintf(f, "], \"beta\": [");
+                for (dmrgx_int t = 0; t < steps[v]; ++t) fprintf(f, "%s%.17g", t ? ", " : "", beta[v * ns + (size_t)t]);
+                fprintf(f, "], \"overlaps\": [");
+                for (dmrgx_int t = 0; t < steps[v]; ++t) {
+                    fprintf(f, "%s\n        [", t ? "," : "");
+                    const double* row = ov.data() + (v * ns + (size_t)t) * n;
+                    for (size_t s = 0; s < n; ++s) fprintf(f, "%s%.17g", s ? ", " : "", row[s]);
+                    fprintf(f, "]");
+                }
+                fprintf(f, "]}");
+            }
+            fprintf(f, "\n    ]");
+        }
+        fprintf(f, "\n  }");
+        fflush(f);
+        ++dyncorr_records;
         return 0;
     }
 
@@ -992,6 +1099,10 @@ private:
     std::vector<bool> spectral_ops = {true, true, true}; /* -spectral_ops: zz, pm, mp */
     FILE* fp_spectral = NULL;
     long long spectral_records = 0;
+    PetscBool do_dyncorr = PETSC_FALSE;       /* -do_dynamical_correlations (extension) */
+    std::vector<PetscInt> dyncorr_sources;    /* -dynamical_sources; empty: every site */
+    FILE* fp_dyncorr = NULL;
+    long long dyncorr_records = 0;
     PetscScalar gse = 0.0;
     std::vector<PetscReal> trunc_err;
     double t0abs = 0.0;

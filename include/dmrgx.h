@@ -244,6 +244,26 @@ int dmrgx_dimer_matrix(dmrgx_kron k, const double* d_psi, dmrgx_int nbonds, cons
 int dmrgx_spectral_lanczos(dmrgx_kron k, const double* d_psi, dmrgx_hshell h_target, int op, dmrgx_int nvec, const double* coef,
                            dmrgx_int nsteps, double* alpha, double* beta, double* norm2, dmrgx_int* nsteps_done, double* flops);
 
+/* ---- EXTENSION: the real-space dynamical correlation matrix (no reference counterpart).  dmrgx_spectral_lanczos, which it calls
+   with the same contract, bits and error codes for alpha, beta, norm2 and nsteps_done, plus at every step the overlap of each
+   normalised Lanczos vector v_t of vector v (v_0 = phi_v/‖phi_v‖) with all n single-site panels:
+       overlaps[(v*nsteps + t)*n + s] = <O_s psi, v_t>      t < nsteps_done[v];  0 for t >= nsteps_done[v].
+   With T_v the tridiagonal matrix of α and β and k < nsteps_done[v], the three-term relation H·V = V·T + β·v·eᵀ, which holds to
+   rounding however much orthogonality is lost, gives the mixed moments exactly
+       <O_s psi| H^k |phi_v> = ‖phi_v‖ Σ_t overlaps[v][t][s] · (T_v^k)_{t,0},
+   and in the same way  <O_s psi| (z - H)^-1 |phi_v> ≈ ‖phi_v‖ Σ_t ov·[(z - T_v)^-1]_{t,0}  and
+   <O_s psi| e^{-i(H - E0)τ} |phi_v> ≈ ‖phi_v‖ Σ_t ov·[e^{-i(T_v - E0)τ}]_{t,0}.  At equal time √norm2[v]·ov[v][0][s] =
+   <O_s psi, phi_v> (the coef-weighted row of SzSz, SpSm or SmSp of dmrgx_corr_matrix for op Sz, S- or S+) and
+   Σ_s coef[v][s]·ov[v][0][s] = √norm2[v].  With coef rows e_c, vector v gives the column c of <O_s psi| f(H) |O_c psi> for
+   every s and any f.  Every site's panel is built, so every site needs Sz and Sp (73 otherwise).  Each step adds one
+   rectangular Gram launch pair over the n panels and the batch's vectors; each element's sums run in a fixed order that
+   depends only on its two columns and D, so a vector's overlaps are the same bits alone or in a batch.  Device memory:
+   (n + 3·nb)·D·8 bytes, plus nb·nsteps·n·8 bytes of overlaps, plus the Gram slab partials (⌈D/8192⌉·⌈n/32⌉·⌈nb/32⌉·8 KiB)
+   and the plans.  flops adds 2·n·D per vector and step.  Errors: those of dmrgx_spectral_lanczos, and 62 overlaps NULL. */
+int dmrgx_spectral_lanczos_overlaps(dmrgx_kron k, const double* d_psi, dmrgx_hshell h_target, int op, dmrgx_int nvec, const double* coef,
+                                    dmrgx_int nsteps, double* alpha, double* beta, double* norm2, dmrgx_int* nsteps_done, double* overlaps,
+                                    double* flops);
+
 /* ---- Hamiltonians::J1J2XXZModel_SquareLattice::H(nsites): src/Hamiltonians.cpp:73-122 (host only).
         Returns the number of terms (fills at most maxterms); bc: 0 open, 1 periodic; nsites < 0 = full lattice. ---- */
 dmrgx_int dmrgx_ham_terms(dmrgx_int Lx, dmrgx_int Ly, double J1, double Jz1, double J2, double Jz2, int bcx, int bcy, dmrgx_int nsites,
