@@ -133,6 +133,7 @@ public:
         fp_data = fopen((data_dir + "DMRGRun.json").c_str(), "w");
         fp_corr = fopen((data_dir + "Correlations.json").c_str(), "w");
         if (!fp_step || !fp_timings || !fp_entanglement || !fp_data || !fp_corr) SETERRQ1(mpi_comm, 1, "cannot open output files in %s", data_dir.c_str());
+        PetscBool do_corr_matrix = PETSC_FALSE, do_dimer_matrix = PETSC_FALSE, do_spectral = PETSC_FALSE, do_dyncorr = PETSC_FALSE;
         /* EXTENSION, off by default: the full two-point spin correlation matrix and the structure factor at every measurement
            step, in CorrelationMatrix.json; computed and written by rank 0 only */
         o.GetBool("-do_correlation_matrix", &do_corr_matrix, NULL);
@@ -145,29 +146,22 @@ public:
         o.GetInt("-spectral_nsteps", &spectral_nsteps, NULL);
         if (spectral_nsteps < 1) SETERRQ1(mpi_comm, 1, "-spectral_nsteps must be at least 1. Got %lld.", LLD(spectral_nsteps));
         if (o.Has("-spectral_ops")) {
-            std::string list;
-            o.GetString("-spectral_ops", list, NULL);
-            for (char& c : list) if (c == ',') c = ' ';
-            std::istringstream iss(list);
+            const std::vector<std::string> items = ListItems(o, "-spectral_ops");
             spectral_ops = {false, false, false};
-            bool any = false;
-            for (std::string item; iss >> item; any = true) {
-                const int k = item == "zz" ? 0 : item == "pm" ? 1 : item == "mp" ? 2 : -1;
-                if (k < 0) SETERRQ1(mpi_comm, PETSC_ERR_ARG_WRONG, "-spectral_ops: unknown item '%s' (the items are zz, pm and mp).", item.c_str());
-                spectral_ops[(size_t)k] = true;
+            for (const std::string& item : items) {
+                size_t k = 0;
+                while (k < 3 && item != spectral_kinds[k].name) ++k;
+                if (k == 3) SETERRQ1(mpi_comm, PETSC_ERR_ARG_WRONG, "-spectral_ops: unknown item '%s' (the items are zz, pm and mp).", item.c_str());
+                spectral_ops[k] = true;
             }
-            if (!any) SETERRQ(mpi_comm, PETSC_ERR_ARG_WRONG, "-spectral_ops: the list is empty (the items are zz, pm and mp).");
+            if (items.empty()) SETERRQ(mpi_comm, PETSC_ERR_ARG_WRONG, "-spectral_ops: the list is empty (the items are zz, pm and mp).");
         }
         /* EXTENSION, off by default: the real-space dynamical correlation matrix <O_s psi| f(H) |O_c psi> from single-site sources c
            at every measurement step, in DynamicalCorrelations.json (-spectral_nsteps, -spectral_ops); rank 0 of a single-GPU run */
         o.GetBool("-do_dynamical_correlations", &do_dyncorr, NULL);
         if (o.Has("-dynamical_sources")) {
-            std::string list;
-            o.GetString("-dynamical_sources", list, NULL);
-            for (char& c : list) if (c == ',') c = ' ';
-            std::istringstream iss(list);
             std::set<PetscInt> seen;
-            for (std::string item; iss >> item;) {
+            for (const std::string& item : ListItems(o, "-dynamical_sources")) {
                 size_t end = 0;
                 long long v = -1;
                 try { v = std::stoll(item, &end); } catch (...) { end = 0; }
@@ -187,30 +181,10 @@ public:
                 SETERRQ1(mpi_comm, PETSC_ERR_SUP, "-do_dynamical_correlations runs on one GPU only (this run has %d ranks).", world);
             if (rank != 0) do_corr_matrix = do_dimer_matrix = do_spectral = do_dyncorr = PETSC_FALSE;
         }
-        if (do_corr_matrix) {
-            fp_corrmat = fopen((data_dir + "CorrelationMatrix.json").c_str(), "w");
-            if (!fp_corrmat) SETERRQ1(mpi_comm, 1, "cannot open %sCorrelationMatrix.json", data_dir.c_str());
-            fprintf(fp_corrmat, "[\n");
-            fflush(fp_corrmat);
-        }
-        if (do_dimer_matrix) {
-            fp_dimer = fopen((data_dir + "DimerMatrix.json").c_str(), "w");
-            if (!fp_dimer) SETERRQ1(mpi_comm, 1, "cannot open %sDimerMatrix.json", data_dir.c_str());
-            fprintf(fp_dimer, "[\n");
-            fflush(fp_dimer);
-        }
-        if (do_spectral) {
-            fp_spectral = fopen((data_dir + "SpectralFunction.json").c_str(), "w");
-            if (!fp_spectral) SETERRQ1(mpi_comm, 1, "cannot open %sSpectralFunction.json", data_dir.c_str());
-            fprintf(fp_spectral, "[\n");
-            fflush(fp_spectral);
-        }
-        if (do_dyncorr) {
-            fp_dyncorr = fopen((data_dir + "DynamicalCorrelations.json").c_str(), "w");
-            if (!fp_dyncorr) SETERRQ1(mpi_comm, 1, "cannot open %sDynamicalCorrelations.json", data_dir.c_str());
-            fprintf(fp_dyncorr, "[\n");
-            fflush(fp_dyncorr);
-        }
+        if (do_corr_matrix) { ierr = corrmat.Open(data_dir, "CorrelationMatrix.json"); CHKERRQ(ierr); }
+        if (do_dimer_matrix) { ierr = dimer.Open(data_dir, "DimerMatrix.json"); CHKERRQ(ierr); }
+        if (do_spectral) { ierr = spectral.Open(data_dir, "SpectralFunction.json"); CHKERRQ(ierr); }
+        if (do_dyncorr) { ierr = dyncorr.Open(data_dir, "DynamicalCorrelations.json"); CHKERRQ(ierr); }
         SaveStepHeaders(); fprintf(fp_step, "[\n");
         SaveTimingsHeaders(); fprintf(fp_timings, "[\n");
         fprintf(fp_entanglement, "[\n");
@@ -273,10 +247,7 @@ public:
         fprintf(fp_data, "\n}\n"); fclose(fp_data);
         if (corr_headers_printed) fprintf(fp_corr, "\n  ]\n}\n");
         fclose(fp_corr);
-        if (fp_corrmat) { fprintf(fp_corrmat, "\n]\n"); fclose(fp_corrmat); fp_corrmat = NULL; }
-        if (fp_dimer) { fprintf(fp_dimer, "\n]\n"); fclose(fp_dimer); fp_dimer = NULL; }
-        if (fp_spectral) { fprintf(fp_spectral, "\n]\n"); fclose(fp_spectral); fp_spectral = NULL; }
-        if (fp_dyncorr) { fprintf(fp_dyncorr, "\n]\n"); fclose(fp_dyncorr); fp_dyncorr = NULL; }
+        for (RecordFile* r : {&corrmat, &dimer, &spectral, &dyncorr}) r->Close();
         init = PETSC_FALSE;
         return 0;
     }
@@ -455,6 +426,40 @@ public:
 private:
     typedef enum { SWEEP_MODE_NULL, SWEEP_MODE_NSWEEPS, SWEEP_MODE_MSWEEPS, SWEEP_MODE_TOLERANCE_TEST } SweepMode_t;
     typedef enum { WarmupStep = 0, SweepStep = 1, NullStep = 2 } Step_t;
+    /** An extension's output file: a JSON array with one record per measurement step, each record opening with GlobIdx and
+        LoopIdx.  The record count places the commas between records. */
+    struct RecordFile {
+        FILE* f = NULL;
+        long long records = 0;
+        explicit operator bool() const { return f != NULL; }
+        PetscErrorCode Open(const std::string& data_dir, const char* name) {
+            f = fopen((data_dir + name).c_str(), "w");
+            if (!f) SETERRQ2(PETSC_COMM_SELF, 1, "cannot open %s%s", data_dir.c_str(), name);
+            fprintf(f, "[\n"); fflush(f);
+            return 0;
+        }
+        FILE* BeginRecord(PetscInt GlobIdx, PetscInt LoopIdx) {
+            fprintf(f, "%s  {\n    \"GlobIdx\": %lld,\n    \"LoopIdx\": %lld", records ? ",\n" : "", LLD(GlobIdx), LLD(LoopIdx));
+            return f;
+        }
+        void EndRecord() { fprintf(f, "\n  }"); fflush(f); ++records; }
+        void Close() { if (f) { fprintf(f, "\n]\n"); fclose(f); f = NULL; } }
+    };
+    /** The lattice coordinates (x[s], y[s]) of points s */
+    struct Coords { std::vector<PetscInt> x, y; };
+    /** The recurrences of -do_spectral_function and -do_dynamical_correlations, in the order of -spectral_ops' flags */
+    struct SpectralKind { const char* name; int op; };
+    static constexpr SpectralKind spectral_kinds[3] = {{"zz", DMRGX_OP_SZ}, {"pm", DMRGX_OP_SM}, {"mp", DMRGX_OP_SP}};
+    /** The items of a list option, separated by commas or blanks; empty items are dropped */
+    static std::vector<std::string> ListItems(PetscOptions& o, const char* key) {
+        std::string list;
+        o.GetString(key, list, NULL);
+        for (char& c : list) if (c == ',') c = ' ';
+        std::istringstream iss(list);
+        std::vector<std::string> items;
+        for (std::string item; iss >> item;) items.push_back(item);
+        return items;
+    }
     static const char* SweepModeToString(SweepMode_t m) {
         switch (m) {
             case SWEEP_MODE_NSWEEPS: return "SWEEP_MODE_NSWEEPS";
@@ -557,7 +562,7 @@ private:
         { dmrgx_int hn, hnt, t1, t2; dmrgx_hshell_stats(H.h, &hn, &hnt, &h_bytes, &h_flops, &t1, &t2); }
         /* -do_spectral_function, -do_dynamical_correlations: the zz recurrence runs on this step's H, which then lives until the
            measurement */
-        if (!(do_measurements && (do_spectral || do_dyncorr))) { ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr); }
+        if (!(do_measurements && (spectral || dyncorr))) { ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr); }
         const double tdiag = Tick();
         total_matvec_flops += h_flops * (double)eps_stats.nmatvec;
         timings_data.tDiag = tdiag - tkron;
@@ -574,15 +579,12 @@ private:
         ierr = BT_R.Load(); CHKERRQ(ierr);
         ierr = SaveEntanglementSpectra(BT_L, SysBlockEnl.Magnetization.List(), BT_R, EnvBlockEnl.Magnetization.List()); CHKERRQ(ierr);
         ierr = CalculateCorrelations_BlockDiag(KronBlocks, gsv_r, do_measurements); CHKERRQ(ierr);
-        if (do_measurements && do_corr_matrix) { ierr = CalculateCorrelationMatrix(KronBlocks, gsv_r, NumSitesTotal); CHKERRQ(ierr); }
-        if (do_measurements && do_dimer_matrix) { ierr = CalculateDimerMatrix(KronBlocks, gsv_r); CHKERRQ(ierr); }
-        if (do_measurements && do_spectral) {
-            ierr = CalculateSpectralFunction(KronBlocks, H, gsv_r, gse_r, NumSitesTotal, Terms, SysBlockEnl, EnvBlockEnl); CHKERRQ(ierr);
-        }
-        if (do_measurements && do_dyncorr) {
-            ierr = CalculateDynamicalCorrelations(KronBlocks, H, gsv_r, gse_r, NumSitesTotal, Terms, SysBlockEnl, EnvBlockEnl); CHKERRQ(ierr);
-        }
-        if (do_measurements && (do_spectral || do_dyncorr)) { ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr); }
+        const Coords r = do_measurements ? SiteCoords(NumSitesTotal) : Coords();
+        if (do_measurements && corrmat) { ierr = CalculateCorrelationMatrix(KronBlocks, gsv_r, r); CHKERRQ(ierr); }
+        if (do_measurements && dimer) { ierr = CalculateDimerMatrix(KronBlocks, gsv_r); CHKERRQ(ierr); }
+        if (do_measurements && spectral) { ierr = CalculateSpectralFunction(KronBlocks, H, gsv_r, gse_r, r, Terms, SysBlockEnl, EnvBlockEnl); CHKERRQ(ierr); }
+        if (do_measurements && dyncorr) { ierr = CalculateDynamicalCorrelations(KronBlocks, H, gsv_r, gse_r, r, Terms, SysBlockEnl, EnvBlockEnl); CHKERRQ(ierr); }
+        if (do_measurements && (spectral || dyncorr)) { ierr = MatDestroy_KronSumShell(&H); CHKERRQ(ierr); }
         if (do_prediction) {
             /* both candidates: which block grows in the next step is the caller's business (the left one in the first half of a sweep,
                the right one in the second, :996-1088); the transformations that created this step's input blocks are captured now,
@@ -689,40 +691,64 @@ private:
         fprintf(f, "\n    ]");
     }
 
+    /** The lattice coordinates of the sites of an nsites-site superblock (superblock site s is lattice site s) */
+    Coords SiteCoords(const PetscInt nsites) const {
+        Coords r{std::vector<PetscInt>((size_t)nsites), std::vector<PetscInt>((size_t)nsites)};
+        for (PetscInt s = 0; s < nsites; ++s) Ham.To2D(s, r.x[(size_t)s], r.y[(size_t)s]);
+        return r;
+    }
+    /** `,\n    "sites": [[x, y], ...]` of a record */
+    static void WriteSites(FILE* f, const Coords& r) {
+        fprintf(f, ",\n    \"sites\": [");
+        for (size_t s = 0; s < r.x.size(); ++s) fprintf(f, "%s[%lld, %lld]", s ? ", " : "", LLD(r.x[s]), LLD(r.y[s]));
+        fprintf(f, "]");
+    }
+    /** The structure factor (1/N) Σ_ab cos(q·(r_a - r_b)) M_ab of the N points r and the N×N row-major M, for every
+        q = (2π kx/Lx, 2π ky/Ly), as [kx][ky]; all zero when there is no point */
+    std::vector<double> StructureFactor(const Coords& r, const std::vector<double>& M) const {
+        const PetscInt Lx = Ham.Lx(), Ly = Ham.Ly();
+        const size_t n = r.x.size();
+        std::vector<double> sq((size_t)(Lx * Ly), 0.0);
+        for (PetscInt kx = 0; kx < Lx && n > 0; ++kx)
+            for (PetscInt ky = 0; ky < Ly; ++ky) {
+                const double qx = 2.0 * M_PI * (double)kx / (double)Lx, qy = 2.0 * M_PI * (double)ky / (double)Ly;
+                double s = 0;
+                for (size_t a = 0; a < n; ++a)
+                    for (size_t b = 0; b < n; ++b)
+                        s += std::cos(qx * (double)(r.x[a] - r.x[b]) + qy * (double)(r.y[a] - r.y[b])) * M[a * n + b];
+                sq[(size_t)(kx * Ly + ky)] = s / (double)n;
+            }
+        return sq;
+    }
+    /** `"alpha": [...], "beta": [...]` — the first `steps` coefficients of a recurrence */
+    static void WriteAlphaBeta(FILE* f, const double* alpha, const double* beta, const dmrgx_int steps) {
+        fprintf(f, "\"alpha\": [");
+        for (dmrgx_int t = 0; t < steps; ++t) fprintf(f, "%s%.17g", t ? ", " : "", alpha[t]);
+        fprintf(f, "], \"beta\": [");
+        for (dmrgx_int t = 0; t < steps; ++t) fprintf(f, "%s%.17g", t ? ", " : "", beta[t]);
+        fprintf(f, "]");
+    }
+
     /** EXTENSION (-do_correlation_matrix): one record of CorrelationMatrix.json — every <S_i S_j> of the superblock from
         dmrgx_corr_matrix (superblock site s is lattice site s), and the static structure factor
             S(q) = (1/N) Σ_ij cos(q·(r_i - r_j)) <S_i·S_j>,   <S_i·S_j> = SzSz + (SpSm + SmSp)/2,   q = (2π kx/Lx, 2π ky/Ly),
         written as StructureFactor[kx][ky]. */
-    PetscErrorCode CalculateCorrelationMatrix(KronBlocks_t& KronBlocks, const Vec& gsv_r, const PetscInt nsites) {
-        const size_t n = (size_t)nsites;
+    PetscErrorCode CalculateCorrelationMatrix(KronBlocks_t& KronBlocks, const Vec& gsv_r, const Coords& r) {
+        const size_t n = r.x.size();
         std::vector<double> szsz(n * n), spsm(n * n), smsp(n * n), sz(n);
         DMRGX_CALL(dmrgx_corr_matrix(KronBlocks.Handle(), gsv_r.d, szsz.data(), spsm.data(), smsp.data(), sz.data(), NULL));
-        const PetscInt Lx = Ham.Lx(), Ly = Ham.Ly();
-        std::vector<PetscInt> x(n), y(n);
-        for (size_t s = 0; s < n; ++s) Ham.To2D((PetscInt)s, x[s], y[s]);
-        FILE* f = fp_corrmat;
-        fprintf(f, "%s  {\n    \"GlobIdx\": %lld,\n    \"LoopIdx\": %lld,\n    \"sites\": [", corrmat_records ? ",\n" : "", LLD(GlobIdx), LLD(LoopIdx));
-        for (size_t s = 0; s < n; ++s) fprintf(f, "%s[%lld, %lld]", s ? ", " : "", LLD(x[s]), LLD(y[s]));
-        fprintf(f, "],\n    \"Sz\": [");
+        FILE* f = corrmat.BeginRecord(GlobIdx, LoopIdx);
+        WriteSites(f, r);
+        fprintf(f, ",\n    \"Sz\": [");
         for (size_t s = 0; s < n; ++s) fprintf(f, "%s%.17g", s ? ", " : "", sz[s]);
         fprintf(f, "]");
         WriteJsonMatrix(f, "SzSz", szsz, n, n);
         WriteJsonMatrix(f, "SpSm", spsm, n, n);
         WriteJsonMatrix(f, "SmSp", smsp, n, n);
-        std::vector<double> sq((size_t)(Lx * Ly), 0.0);
-        for (PetscInt kx = 0; kx < Lx; ++kx)
-            for (PetscInt ky = 0; ky < Ly; ++ky) {
-                const double qx = 2.0 * M_PI * (double)kx / (double)Lx, qy = 2.0 * M_PI * (double)ky / (double)Ly;
-                double s = 0;
-                for (size_t i = 0; i < n; ++i)
-                    for (size_t j = 0; j < n; ++j)
-                        s += std::cos(qx * (double)(x[i] - x[j]) + qy * (double)(y[i] - y[j])) * (szsz[i * n + j] + 0.5 * (spsm[i * n + j] + smsp[i * n + j]));
-                sq[(size_t)(kx * Ly + ky)] = s / (double)n;
-            }
-        WriteJsonMatrix(f, "StructureFactor", sq, (size_t)Lx, (size_t)Ly);
-        fprintf(f, "\n  }");
-        fflush(f);
-        ++corrmat_records;
+        std::vector<double> ss(n * n);
+        for (size_t k = 0; k < n * n; ++k) ss[k] = szsz[k] + 0.5 * (spsm[k] + smsp[k]);
+        WriteJsonMatrix(f, "StructureFactor", StructureFactor(r, ss), (size_t)Ham.Lx(), (size_t)Ham.Ly());
+        corrmat.EndRecord();
         return 0;
     }
 
@@ -757,8 +783,8 @@ private:
         for (size_t a = 0; a < nb; ++a) { si[a] = bonds[a].i; sj[a] = bonds[a].j; }
         std::vector<double> dd(nb * nb), d(nb);
         DMRGX_CALL(dmrgx_dimer_matrix(KronBlocks.Handle(), gsv_r.d, (dmrgx_int)nb, si.data(), sj.data(), dd.data(), d.data(), NULL));
-        FILE* f = fp_dimer;
-        fprintf(f, "%s  {\n    \"GlobIdx\": %lld,\n    \"LoopIdx\": %lld,\n    \"bonds\": [", dimer_records ? ",\n" : "", LLD(GlobIdx), LLD(LoopIdx));
+        FILE* f = dimer.BeginRecord(GlobIdx, LoopIdx);
+        fprintf(f, ",\n    \"bonds\": [");
         for (size_t a = 0; a < nb; ++a) {
             const Bond& b = bonds[a];
             fprintf(f, "%s\n      {\"sites\": [%lld, %lld], \"coords\": [[%lld, %lld], [%lld, %lld]], \"orientation\": \"%c\", \"origin\": [%lld, %lld]}",
@@ -770,23 +796,16 @@ private:
         WriteJsonMatrix(f, "DimerDimer", dd, nb, nb);
         for (const char dir : {'x', 'y'}) {
             std::vector<size_t> in;
+            Coords origins;
             for (size_t a = 0; a < nb; ++a)
-                if (bonds[a].dir == dir) in.push_back(a);
-            std::vector<double> sq((size_t)(Lx * Ly), 0.0);
-            for (PetscInt kx = 0; kx < Lx && !in.empty(); ++kx)
-                for (PetscInt ky = 0; ky < Ly; ++ky) {
-                    const double qx = 2.0 * M_PI * (double)kx / (double)Lx, qy = 2.0 * M_PI * (double)ky / (double)Ly;
-                    double s = 0;
-                    for (const size_t a : in)
-                        for (const size_t b : in)
-                            s += std::cos(qx * (double)(bonds[a].ox - bonds[b].ox) + qy * (double)(bonds[a].oy - bonds[b].oy)) * (dd[a * nb + b] - d[a] * d[b]);
-                    sq[(size_t)(kx * Ly + ky)] = s / (double)in.size();
-                }
-            WriteJsonMatrix(f, dir == 'x' ? "DimerStructureFactorX" : "DimerStructureFactorY", sq, (size_t)Lx, (size_t)Ly);
+                if (bonds[a].dir == dir) { in.push_back(a); origins.x.push_back(bonds[a].ox); origins.y.push_back(bonds[a].oy); }
+            const size_t m = in.size();
+            std::vector<double> conn(m * m);
+            for (size_t a = 0; a < m; ++a)
+                for (size_t b = 0; b < m; ++b) conn[a * m + b] = dd[in[a] * nb + in[b]] - d[in[a]] * d[in[b]];
+            WriteJsonMatrix(f, dir == 'x' ? "DimerStructureFactorX" : "DimerStructureFactorY", StructureFactor(origins, conn), (size_t)Lx, (size_t)Ly);
         }
-        fprintf(f, "\n  }");
-        fflush(f);
-        ++dimer_records;
+        dimer.EndRecord();
         return 0;
     }
 
@@ -820,50 +839,44 @@ private:
         empty shifted sector gives zeros.  Written per operator as [kx][ky] -> {"cos": ..., "sin": ...}, each part holding norm2,
         steps (the recurrence length) and the first `steps` of alpha and beta (beta[0] = 0).  At equal time,
         Σ_parts (zz + (pm + mp)/2) norm2 = StructureFactor[kx][ky] of CorrelationMatrix.json. */
-    PetscErrorCode CalculateSpectralFunction(KronBlocks_t& KronBlocks, const ShellMat& H, const Vec& gsv_r, const PetscScalar E0, const PetscInt nsites,
+    PetscErrorCode CalculateSpectralFunction(KronBlocks_t& KronBlocks, const ShellMat& H, const Vec& gsv_r, const PetscScalar E0, const Coords& r,
                                              const std::vector<Hamiltonians::Term>& Terms, Block& SysBlockEnl, Block& EnvBlockEnl) {
         const PetscInt Lx = Ham.Lx(), Ly = Ham.Ly();
-        const size_t n = (size_t)nsites, nq = (size_t)(Lx * Ly), nvec = 2 * nq, ns = (size_t)spectral_nsteps;
-        std::vector<PetscInt> x(n), y(n);
-        for (size_t s = 0; s < n; ++s) Ham.To2D((PetscInt)s, x[s], y[s]);
+        const size_t n = r.x.size(), nq = (size_t)(Lx * Ly), nvec = 2 * nq, ns = (size_t)spectral_nsteps;
         std::vector<double> coef(nvec * n);
         for (PetscInt kx = 0; kx < Lx; ++kx)
             for (PetscInt ky = 0; ky < Ly; ++ky) {
                 const double qx = 2.0 * M_PI * (double)kx / (double)Lx, qy = 2.0 * M_PI * (double)ky / (double)Ly;
                 const size_t v = 2 * (size_t)(kx * Ly + ky);
                 for (size_t s = 0; s < n; ++s) {
-                    const double ph = qx * (double)x[s] + qy * (double)y[s];
+                    const double ph = qx * (double)r.x[s] + qy * (double)r.y[s];
                     coef[v * n + s] = std::cos(ph) / std::sqrt((double)n);
                     coef[(v + 1) * n + s] = std::sin(ph) / std::sqrt((double)n);
                 }
             }
-        FILE* f = fp_spectral;
-        fprintf(f, "%s  {\n    \"GlobIdx\": %lld,\n    \"LoopIdx\": %lld,\n    \"E0\": %.17g,\n    \"NSteps\": %lld,\n    \"sites\": [",
-                spectral_records ? ",\n" : "", LLD(GlobIdx), LLD(LoopIdx), E0, LLD(spectral_nsteps));
-        for (size_t s = 0; s < n; ++s) fprintf(f, "%s[%lld, %lld]", s ? ", " : "", LLD(x[s]), LLD(y[s]));
-        fprintf(f, "]");
-        const struct { const char* name; int op; } kinds[3] = {{"zz", DMRGX_OP_SZ}, {"pm", DMRGX_OP_SM}, {"mp", DMRGX_OP_SP}};
+        FILE* f = spectral.BeginRecord(GlobIdx, LoopIdx);
+        fprintf(f, ",\n    \"E0\": %.17g,\n    \"NSteps\": %lld", E0, LLD(spectral_nsteps));
+        WriteSites(f, r);
         for (size_t k = 0; k < 3; ++k) {
             if (!spectral_ops[k]) continue;
+            const SpectralKind& kind = spectral_kinds[k];
             std::vector<double> alpha(nvec * ns, 0.0), beta(nvec * ns, 0.0), norm2(nvec, 0.0);
             std::vector<dmrgx_int> steps(nvec, 0);
-            PetscErrorCode ierr = WithSpectralTarget(H, kinds[k].op, Terms, SysBlockEnl, EnvBlockEnl, "dmrgx_spectral_lanczos", [&](dmrgx_hshell t) {
-                return dmrgx_spectral_lanczos(KronBlocks.Handle(), gsv_r.d, t, kinds[k].op, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns, alpha.data(),
+            PetscErrorCode ierr = WithSpectralTarget(H, kind.op, Terms, SysBlockEnl, EnvBlockEnl, "dmrgx_spectral_lanczos", [&](dmrgx_hshell t) {
+                return dmrgx_spectral_lanczos(KronBlocks.Handle(), gsv_r.d, t, kind.op, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns, alpha.data(),
                                               beta.data(), norm2.data(), steps.data(), NULL);
             });
             if (ierr) return ierr;
-            fprintf(f, ",\n    \"%s\": [", kinds[k].name);
+            fprintf(f, ",\n    \"%s\": [", kind.name);
             for (PetscInt kx = 0; kx < Lx; ++kx) {
                 fprintf(f, "%s\n      [", kx ? "," : "");
                 for (PetscInt ky = 0; ky < Ly; ++ky) {
                     fprintf(f, "%s{", ky ? ",\n       " : "");
                     for (size_t part = 0; part < 2; ++part) {
                         const size_t v = 2 * (size_t)(kx * Ly + ky) + part;
-                        fprintf(f, "%s\"%s\": {\"norm2\": %.17g, \"steps\": %lld, \"alpha\": [", part ? ", " : "", part ? "sin" : "cos", norm2[v], LLD(steps[v]));
-                        for (dmrgx_int t = 0; t < steps[v]; ++t) fprintf(f, "%s%.17g", t ? ", " : "", alpha[v * ns + (size_t)t]);
-                        fprintf(f, "], \"beta\": [");
-                        for (dmrgx_int t = 0; t < steps[v]; ++t) fprintf(f, "%s%.17g", t ? ", " : "", beta[v * ns + (size_t)t]);
-                        fprintf(f, "]}");
+                        fprintf(f, "%s\"%s\": {\"norm2\": %.17g, \"steps\": %lld, ", part ? ", " : "", part ? "sin" : "cos", norm2[v], LLD(steps[v]));
+                        WriteAlphaBeta(f, &alpha[v * ns], &beta[v * ns], steps[v]);
+                        fprintf(f, "}");
                     }
                     fprintf(f, "}");
                 }
@@ -871,9 +884,7 @@ private:
             }
             fprintf(f, "\n    ]");
         }
-        fprintf(f, "\n  }");
-        fflush(f);
-        ++spectral_records;
+        spectral.EndRecord();
         return 0;
     }
 
@@ -887,9 +898,10 @@ private:
         (G_sc(τ) = <S_s(τ) S_c>).  Written per operator as one entry per source: site, norm2, steps, the first `steps` of alpha
         and beta (beta[0] = 0) and `steps` rows of n overlaps.  At 12×6 with every site as a source and 64 steps a record holds
         about 3·72·64·72 numbers (some 20 MB); -dynamical_sources shrinks it in proportion. */
-    PetscErrorCode CalculateDynamicalCorrelations(KronBlocks_t& KronBlocks, const ShellMat& H, const Vec& gsv_r, const PetscScalar E0, const PetscInt nsites,
+    PetscErrorCode CalculateDynamicalCorrelations(KronBlocks_t& KronBlocks, const ShellMat& H, const Vec& gsv_r, const PetscScalar E0, const Coords& r,
                                                   const std::vector<Hamiltonians::Term>& Terms, Block& SysBlockEnl, Block& EnvBlockEnl) {
-        const size_t n = (size_t)nsites, ns = (size_t)spectral_nsteps;
+        const PetscInt nsites = (PetscInt)r.x.size();
+        const size_t n = r.x.size(), ns = (size_t)spectral_nsteps;
         std::vector<PetscInt> src = dyncorr_sources;
         if (src.empty())
             for (PetscInt s = 0; s < nsites; ++s) src.push_back(s);
@@ -898,32 +910,27 @@ private:
         const size_t nvec = src.size();
         std::vector<double> coef(nvec * n, 0.0);
         for (size_t v = 0; v < nvec; ++v) coef[v * n + (size_t)src[v]] = 1.0;
-        std::vector<PetscInt> x(n), y(n);
-        for (size_t s = 0; s < n; ++s) Ham.To2D((PetscInt)s, x[s], y[s]);
-        FILE* f = fp_dyncorr;
-        fprintf(f, "%s  {\n    \"GlobIdx\": %lld,\n    \"LoopIdx\": %lld,\n    \"E0\": %.17g,\n    \"NSteps\": %lld,\n    \"sites\": [",
-                dyncorr_records ? ",\n" : "", LLD(GlobIdx), LLD(LoopIdx), E0, LLD(spectral_nsteps));
-        for (size_t s = 0; s < n; ++s) fprintf(f, "%s[%lld, %lld]", s ? ", " : "", LLD(x[s]), LLD(y[s]));
-        fprintf(f, "],\n    \"sources\": [");
+        FILE* f = dyncorr.BeginRecord(GlobIdx, LoopIdx);
+        fprintf(f, ",\n    \"E0\": %.17g,\n    \"NSteps\": %lld", E0, LLD(spectral_nsteps));
+        WriteSites(f, r);
+        fprintf(f, ",\n    \"sources\": [");
         for (size_t v = 0; v < nvec; ++v) fprintf(f, "%s%lld", v ? ", " : "", LLD(src[v]));
         fprintf(f, "]");
-        const struct { const char* name; int op; } kinds[3] = {{"zz", DMRGX_OP_SZ}, {"pm", DMRGX_OP_SM}, {"mp", DMRGX_OP_SP}};
         for (size_t k = 0; k < 3; ++k) {
             if (!spectral_ops[k]) continue;
+            const SpectralKind& kind = spectral_kinds[k];
             std::vector<double> alpha(nvec * ns, 0.0), beta(nvec * ns, 0.0), norm2(nvec, 0.0), ov(nvec * ns * n, 0.0);
             std::vector<dmrgx_int> steps(nvec, 0);
-            PetscErrorCode ierr = WithSpectralTarget(H, kinds[k].op, Terms, SysBlockEnl, EnvBlockEnl, "dmrgx_spectral_lanczos_overlaps", [&](dmrgx_hshell t) {
-                return dmrgx_spectral_lanczos_overlaps(KronBlocks.Handle(), gsv_r.d, t, kinds[k].op, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns,
+            PetscErrorCode ierr = WithSpectralTarget(H, kind.op, Terms, SysBlockEnl, EnvBlockEnl, "dmrgx_spectral_lanczos_overlaps", [&](dmrgx_hshell t) {
+                return dmrgx_spectral_lanczos_overlaps(KronBlocks.Handle(), gsv_r.d, t, kind.op, (dmrgx_int)nvec, coef.data(), (dmrgx_int)ns,
                                                        alpha.data(), beta.data(), norm2.data(), steps.data(), ov.data(), NULL);
             });
             if (ierr) return ierr;
-            fprintf(f, ",\n    \"%s\": [", kinds[k].name);
+            fprintf(f, ",\n    \"%s\": [", kind.name);
             for (size_t v = 0; v < nvec; ++v) {
-                fprintf(f, "%s\n      {\"site\": %lld, \"norm2\": %.17g, \"steps\": %lld, \"alpha\": [", v ? "," : "", LLD(src[v]), norm2[v], LLD(steps[v]));
-                for (dmrgx_int t = 0; t < steps[v]; ++t) fprintf(f, "%s%.17g", t ? ", " : "", alpha[v * ns + (size_t)t]);
-                fprintf(f, "], \"beta\": [");
-                for (dmrgx_int t = 0; t < steps[v]; ++t) fprintf(f, "%s%.17g", t ? ", " : "", beta[v * ns + (size_t)t]);
-                fprintf(f, "], \"overlaps\": [");
+                fprintf(f, "%s\n      {\"site\": %lld, \"norm2\": %.17g, \"steps\": %lld, ", v ? "," : "", LLD(src[v]), norm2[v], LLD(steps[v]));
+                WriteAlphaBeta(f, &alpha[v * ns], &beta[v * ns], steps[v]);
+                fprintf(f, ", \"overlaps\": [");
                 for (dmrgx_int t = 0; t < steps[v]; ++t) {
                     fprintf(f, "%s\n        [", t ? "," : "");
                     const double* row = ov.data() + (v * ns + (size_t)t) * n;
@@ -934,9 +941,7 @@ private:
             }
             fprintf(f, "\n    ]");
         }
-        fprintf(f, "\n  }");
-        fflush(f);
-        ++dyncorr_records;
+        dyncorr.EndRecord();
         return 0;
     }
 
@@ -1088,21 +1093,14 @@ private:
     PetscInt LoopIdx = 0, StepIdx = 0;
     std::vector<Correlator> measurements;
     PetscBool corr_headers_printed = PETSC_FALSE, corr_printed_first = PETSC_FALSE;
-    PetscBool do_corr_matrix = PETSC_FALSE;   /* -do_correlation_matrix (extension) */
-    FILE* fp_corrmat = NULL;
-    long long corrmat_records = 0;
-    PetscBool do_dimer_matrix = PETSC_FALSE;  /* -do_dimer_matrix (extension) */
-    FILE* fp_dimer = NULL;
-    long long dimer_records = 0;
-    PetscBool do_spectral = PETSC_FALSE;      /* -do_spectral_function (extension) */
+    /* the extensions' output files; one that is not open means the extension is off */
+    RecordFile corrmat;                       /* -do_correlation_matrix */
+    RecordFile dimer;                         /* -do_dimer_matrix */
+    RecordFile spectral;                      /* -do_spectral_function */
+    RecordFile dyncorr;                       /* -do_dynamical_correlations */
     PetscInt spectral_nsteps = 64;            /* -spectral_nsteps */
-    std::vector<bool> spectral_ops = {true, true, true}; /* -spectral_ops: zz, pm, mp */
-    FILE* fp_spectral = NULL;
-    long long spectral_records = 0;
-    PetscBool do_dyncorr = PETSC_FALSE;       /* -do_dynamical_correlations (extension) */
+    std::vector<bool> spectral_ops = {true, true, true}; /* -spectral_ops, in the order of spectral_kinds */
     std::vector<PetscInt> dyncorr_sources;    /* -dynamical_sources; empty: every site */
-    FILE* fp_dyncorr = NULL;
-    long long dyncorr_records = 0;
     PetscScalar gse = 0.0;
     std::vector<PetscReal> trunc_err;
     double t0abs = 0.0;

@@ -29,10 +29,12 @@ where the data are exact (dyadic Gram inputs, copies, splitmix64) exact equality
 import ctypes as C
 import os
 import subprocess
-import zlib
 
 import numpy as np
 import pytest
+
+from devcheck_common import (LD, SENT, U, Backend, assert_bound, assert_guards, assert_unchanged, bits, guard_for, rng_for,
+                             sentinel, wrap)
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CSRC = os.path.join(ROOT, "dmrg.x_b200", "csrc")
@@ -41,10 +43,6 @@ LIBS = {"host": os.path.join(ROOT, "tests", "devcheck", "libdevcheck_host.so"),
 # DMRGX_DEVCHECK_CUDA: run the cuda flavour against another build of the shim (for example over a modified dev_cuda.cu)
 CUDA_OVERRIDE = os.environ.get("DMRGX_DEVCHECK_CUDA")
 
-U = 2.0 ** -53
-LD = np.longdouble
-SENT = np.uint64(0xC3D5A5A55A5A0F0F)   # output guard / gap sentinel (a finite double no kernel here produces)
-MIN_GUARD = 512                          # 4 KiB of doubles
 DEEP_BELOW = 1800                        # run_chain: launches below this many items take the three-stage copy ring
 RED_BLOCKS = 592                         # grid of the streaming kernels
 SP_MAX_NR = 3072
@@ -68,41 +66,6 @@ CELL = 80   # rows / columns of the operand cells the work items cut their tiles
 # ---------------------------------------------------------------------------------------------------------------------
 #  backend and buffers
 # ---------------------------------------------------------------------------------------------------------------------
-class Backend:
-    def __init__(self, name, path):
-        self.name = name
-        self.lib = C.CDLL(path)
-        self.lib.dc_error.restype = C.c_char_p
-
-    def __call__(self, fn, *args):
-        conv = []
-        for a in args:
-            if isinstance(a, np.ndarray):
-                assert a.flags.c_contiguous
-                conv.append(C.c_void_p(a.ctypes.data))
-            elif a is None:
-                conv.append(C.c_void_p(None))
-            elif isinstance(a, float):
-                conv.append(C.c_double(a))
-            elif isinstance(a, tuple):          # ("u64", value)
-                conv.append(C.c_ulonglong(a[1]))
-            else:
-                conv.append(C.c_longlong(int(a)))
-        return getattr(self.lib, fn)(*conv)
-
-    def ok(self, fn, *args):
-        rc = self(fn, *args)
-        assert rc == 0, "%s: %s" % (fn, self.error())
-
-    def refused(self, fn, *args):
-        rc = self(fn, *args)
-        assert rc != 0, "%s was not refused" % fn
-        return self.error()
-
-    def error(self):
-        return self.lib.dc_error().decode()
-
-
 def _lib_path(name):
     if name == "cuda" and CUDA_OVERRIDE:
         return CUDA_OVERRIDE
@@ -117,59 +80,6 @@ def dc(request):
     # the int arguments of every dc_* entry point are declared long long or int; ctypes passes c_longlong, which is
     # also right for int arguments on x86-64 / aarch64 (registers and 8-byte stack slots)
     return Backend(request.param, _lib_path(request.param))
-
-
-def guard_for(ld=0):
-    g = max(MIN_GUARD, int(ld))
-    return g + (g & 1)
-
-
-def wrap(payload, g, fill="nan"):
-    """[guard | payload | guard]; fill: 'nan' (operands) or 'sent' (outputs)"""
-    payload = np.ascontiguousarray(payload)
-    full = np.empty(payload.size + 2 * g, payload.dtype)
-    if fill == "sent":
-        full.view(np.uint64)[:] = SENT
-    elif payload.dtype == np.float64:
-        full[:] = np.nan
-    else:
-        full[:] = 0
-    full[g:g + payload.size] = payload.ravel()
-    return full
-
-
-def sentinel(n, g):
-    full = np.empty(n + 2 * g)
-    full.view(np.uint64)[:] = SENT
-    return full
-
-
-def bits(a):
-    return np.ascontiguousarray(a).view(np.uint64)
-
-
-def assert_guards(full, g, what="output"):
-    assert (bits(full[:g]) == SENT).all() and (bits(full[-g:]) == SENT).all(), "%s guard overwritten" % what
-
-
-def assert_unchanged(after, before, sel, what):
-    assert (bits(after[sel]) == bits(before[sel])).all(), "%s changed where it must not" % what
-
-
-def assert_bound(got, ref, absref, N, what):
-    got = np.asarray(got, np.float64)
-    ref = np.asarray(ref, LD)
-    bound = (np.asarray(N, LD) + 2) * LD(U) * np.asarray(absref, LD)
-    err = np.abs(got.astype(LD) - ref)
-    bad = ~(err <= bound)
-    if bad.any():
-        i = np.flatnonzero(bad.ravel())[0]
-        raise AssertionError("%s: %d elements outside (N+2)·u·Σ|terms|; first at flat %d: got %r ref %r bound %r"
-                             % (what, int(bad.sum()), i, float(got.ravel()[i]), float(ref.ravel()[i]), float(np.broadcast_to(bound, got.shape).ravel()[i])))
-
-
-def rng_for(*key):
-    return np.random.default_rng([zlib.crc32(str(k).encode()) for k in key])
 
 
 # ---------------------------------------------------------------------------------------------------------------------

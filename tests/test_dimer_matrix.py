@@ -4,75 +4,21 @@ library."""
 import ctypes as C
 import json
 import os
-import subprocess
 
 import numpy as np
 import pytest
 
 import driver_common as dc
-import libswitch
-from test_correlation_matrix import EXE, HEIS_CHAIN12, J1J2_CYL, PLANCHECK, ROOT, SM, SP, SZ, exact_halves, oracle_blocks, random_psi, site_op
-
-# D_a = Sz_i Sz_j + ½ S+_i S-_j + ½ S-_i S+_j, as (O_i, O_j, coefficient); the transpose of O
-TERMS = ((SZ, SZ, 1.0), (SP, SM, 0.5), (SM, SP, 0.5))
-T = {SZ: SZ, SP: SM, SM: SP}
-
-
-@pytest.fixture(scope="module", params=["plancheck", pytest.param("cuda", marks=pytest.mark.gpu)])
-def P(request):
-    import dmrgx_loader
-    P = dmrgx_loader.load_package()
-    if request.param == "plancheck":
-        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "dmrg.x_b200", "csrc"), "plancheck"])
-        libswitch.use_library(P, PLANCHECK)
-    else:
-        libswitch.use_library(P, None)
-    P.kind = request.param
-    yield P
-    libswitch.use_library(P, None)
-
-
-@pytest.fixture()
-def ctx(P):
-    c = P.Context(0)
-    yield c
-    c.close()
+from measure_common import (DRIVER_M, DRIVER_RUN, HEIS_CHAIN12, J1J2_CYL, SM, SP, SZ, P, ctx,  # noqa: F401
+                            exact_diagonalisation, exact_halves, exe, ham_terms, nn_bonds, oracle_blocks,
+                            per_correlator_dimer, random_psi)
 
 
 # ---- references --------------------------------------------------------------------------------------------------------
 
-def product_expect(P, kb, dpsi, nL, n, ops):
-    """<psi| O_1 O_2 ... |psi> for superblock-site operators [(op, site), ...] through dmrgx_hshell_create_product +
-    dmrgx_expect; each block's operators keep their list order (operators of different blocks commute)."""
-    lops = [(o, s) for o, s in ops if s < nL]
-    rops = [(o, n - 1 - s) for o, s in ops if s >= nL]
-    L = P.lib()
-    la = np.array([o for o, _ in lops], np.int32); ls = np.array([s for _, s in lops], np.int64)
-    ra = np.array([o for o, _ in rops], np.int32); rs = np.array([s for _, s in rops], np.int64)
-    h = C.c_void_p()
-    assert L.dmrgx_hshell_create_product(kb.h, C.c_longlong(len(lops)), la.ctypes.data_as(C.c_void_p), ls.ctypes.data_as(C.c_void_p),
-                                         C.c_longlong(len(rops)), ra.ctypes.data_as(C.c_void_p), rs.ctypes.data_as(C.c_void_p), C.byref(h)) == 0, \
-        L.dmrgx_last_error()
-    v = C.c_double()
-    assert L.dmrgx_expect(h, dpsi.ptr, C.byref(v)) == 0
-    L.dmrgx_hshell_destroy(h)
-    return v.value
-
-
-def per_correlator_dimer(P, kb, dpsi, nL, n, a, b=None):
-    """<psi| D_a |psi>, or <D_a psi, D_b psi> as the 9 products [O_jᵀ, O_iᵀ, O_k, O_l] of the per-correlator path"""
-    i, j = a
-    if b is None:
-        return sum(c * product_expect(P, kb, dpsi, nL, n, [(oi, i), (oj, j)]) for oi, oj, c in TERMS)
-    k, l_ = b
-    return sum(ca * cb * product_expect(P, kb, dpsi, nL, n, [(T[oj], j), (T[oi], i), (ok, k), (ol, l_)])
-               for oi, oj, ca in TERMS for ok, ol, cb in TERMS)
-
-
 def lattice_pairs(P, ham, n):
     """distinct (i, j), i < j, of the lattice's Sz·Sz terms with both sites below n, split into nearest (Jz1) and next-nearest (Jz2)"""
-    N = ham["Lx"] * ham["Ly"]
-    terms = P.HamiltonianTerms(ham["Lx"], ham["Ly"], ham["J1"], ham["Jz1"], ham["J2"], ham["Jz2"], N, ham["bcx"], ham["bcy"])
+    terms = ham_terms(P, ham, ham["Lx"] * ham["Ly"])
     nn, nnn = [], []
     for a, io, i, jo, j in terms:
         if io != SZ or max(i, j) >= n:
@@ -99,22 +45,11 @@ def mixed_bonds(P, nL, n):
     return bonds
 
 
-def bond_op(N, i, j):
-    return site_op(N, SZ, i) @ site_op(N, SZ, j) + 0.5 * (site_op(N, SP, i) @ site_op(N, SM, j) + site_op(N, SM, i) @ site_op(N, SP, j))
-
-
 def exact_dimers(terms, N, bonds):
     """exact diagonalisation in the Sz = 0 sector: ground-state energy, gap, <D_a D_b> and <D_a>"""
-    import scipy.sparse.linalg as sla
-    H = sum(a * (site_op(N, io, i) @ site_op(N, jo, j)) for (a, io, i, jo, j) in terms)
-    nup = np.array([bin(b).count("1") for b in range(2 ** N)])
-    sec = np.nonzero(nup == N // 2)[0]
-    w, v = sla.eigsh(H[sec][:, sec], k=2, which="SA", tol=1e-14)
-    order = np.argsort(w)
-    w, v = w[order], v[:, order]
-    psi = np.zeros(2 ** N)
-    psi[sec] = v[:, 0]
-    Dpsi = np.array([bond_op(N, i, j) @ psi for i, j in bonds])
+    w, psi, _, ops, _ = exact_diagonalisation(terms, N, k=2)
+    bond_op = lambda i, j: ops[(SZ, i)] @ ops[(SZ, j)] + 0.5 * (ops[(SP, i)] @ ops[(SM, j)] + ops[(SM, i)] @ ops[(SP, j)])
+    Dpsi = np.array([bond_op(i, j) @ psi for i, j in bonds])
     return w[0], w[1] - w[0], Dpsi @ Dpsi.T, Dpsi @ psi
 
 
@@ -128,7 +63,7 @@ def test_every_entry_matches_the_per_correlator_path(P, ctx, orc, case):
     nL, nR, spin = {"L=R": (8, 8, 1), "L!=R": (8, 6, 1), "spin1": (8, 8, 2)}[case]
     pL, pR = oracle_blocks(orc, P, ctx, nL, nR, spin)
     kb = P.KronBlocks(pL, pR, [0.0])
-    dpsi = random_psi(ctx, kb.NumStates(), 17)
+    dpsi, _ = random_psi(ctx, kb.NumStates(), 17)
     n = nL + nR
     bonds = mixed_bonds(P, nL, n)
     got = kb.DimerMatrix(dpsi, bonds)
@@ -147,7 +82,7 @@ def test_dimer_equals_the_spin_matrix_combination(P, ctx, orc, qn):
     """On truncated blocks <D_a> = SzSz + ½(SpSm + SmSp) at [i][j] of the spin correlation matrix, in either bond order."""
     pL, pR = oracle_blocks(orc, P, ctx, 8, 6)
     kb = P.KronBlocks(pL, pR, [qn])
-    dpsi = random_psi(ctx, kb.NumStates(), 5)
+    dpsi, _ = random_psi(ctx, kb.NumStates(), 5)
     n = 14
     nn, nnn = lattice_pairs(P, J1J2_CYL, n)
     bonds = nn + [p[::-1] for p in nnn] + [(0, n - 1), (n - 1, 0)]
@@ -197,7 +132,7 @@ def test_errors(P, ctx, orc):
     56: not exactly one sector; 73: a block without Sz_i / Sp_i at a site some bond uses (site in the message)."""
     pL, pR = oracle_blocks(orc, P, ctx, 8, 8)
     kb = P.KronBlocks(pL, pR, [0.0])
-    dpsi = random_psi(ctx, kb.NumStates(), 2)
+    dpsi, _ = random_psi(ctx, kb.NumStates(), 2)
     with pytest.raises(P.DmrgxError) as e:
         kb.DimerMatrix(None, [(0, 1)])
     assert e.value.code == 62
@@ -240,7 +175,7 @@ def test_two_calls_are_bitwise_equal(P, ctx):
         pytest.skip("the CUDA kernels only")
     blk, _ = exact_halves(P, ctx, J1J2_CYL)
     kb = P.KronBlocks(blk, blk, [0.0])
-    dpsi = random_psi(ctx, kb.NumStates(), 9)
+    dpsi, _ = random_psi(ctx, kb.NumStates(), 9)
     nn, nnn = lattice_pairs(P, J1J2_CYL, 16)
     a, b = kb.DimerMatrix(dpsi, nn + nnn), kb.DimerMatrix(dpsi, nn + nnn)
     for k in ("DD", "D"):
@@ -250,45 +185,7 @@ def test_two_calls_are_bitwise_equal(P, ctx):
 # ---- the driver ----------------------------------------------------------------------------------------------------------
 
 # the 4x4 J1-J2 cylinder, and a 4x2 one whose rungs NeighborPairs lists twice (periodic y with Ly = 2)
-DRIVER_RUNS = [(["-Lx", 4, "-Ly", 4, "-J1", 0.5, "-Jz1", 1, "-J2", 0.25, "-Jz2", 0.5], J1J2_CYL),
-               (["-Lx", 4, "-Ly", 2, "-J1", 0.5, "-Jz1", 1, "-J2", 0.25, "-Jz2", 0.5], dict(J1J2_CYL, Ly=2))]
-DRIVER_M = {"plancheck": (16, [16]), "cuda": (256, [256])}
-
-
-@pytest.fixture(scope="module")
-def exe(P):
-    if P.kind == "plancheck":
-        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "dmrg.x_b200", "driver"), "plancheck"])
-    assert os.path.exists(EXE[P.kind]), "build it with __graft_entry__.build()"
-    return EXE[P.kind]
-
-
-def nn_bonds(ham):
-    """the distinct nearest-neighbour bonds in NeighborPairs order (1-D snake numbering), with orientation and origin: the site
-    from which the +x / +y step leads, for a wrap-around bond the one in the last column / row (a two-leg rung: y = 0)"""
-    Lx, Ly = ham["Lx"], ham["Ly"]
-    to1d = lambda x, y: x * Ly + y if x % 2 == 0 else (x + 1) * Ly - (y + 1)
-    xy = {}
-    for x in range(Lx):
-        for y in range(Ly):
-            xy[to1d(x, y)] = (x, y)
-    out = []
-    for s in range(Lx * Ly):
-        x, y = xy[s]
-        nbr = []
-        if y < Ly - 1 or ham["bcy"]:
-            nbr.append(("y", to1d(x, (y + 1) % Ly)))
-        if x < Lx - 1 or ham["bcx"]:
-            nbr.append(("x", to1d((x + 1) % Lx, y)))
-        for o, t in nbr:
-            p = (min(s, t), max(s, t))
-            if t == s or p in [b[0] for b in out]:
-                continue
-            u = {"x": 0, "y": 1}[o]
-            a, b = xy[p[0]], xy[p[1]]
-            origin = a if a[u] + 1 == b[u] else b if b[u] + 1 == a[u] else max(a, b, key=lambda c: c[u])
-            out.append((p, o, origin))
-    return out
+DRIVER_RUNS = [DRIVER_RUN, (["-Lx", 4, "-Ly", 2, "-J1", 0.5, "-Jz1", 1, "-J2", 0.25, "-Jz2", 0.5], dict(J1J2_CYL, Ly=2))]
 
 
 def check_records(recs, cms, docs, ham):

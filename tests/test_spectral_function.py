@@ -10,110 +10,12 @@ import numpy as np
 import pytest
 
 import driver_common as dc
-import libswitch
-import parity_common as pc
-
-ROOT = dc.ROOT
-PLANCHECK = os.path.join(ROOT, "tests", "plancheck", "libdmrgx_plancheck.so")
-EXE = {"plancheck": os.path.join(ROOT, "tests", "plancheck", "DMRG-SquareLattice.plancheck.x"),
-       "cuda": os.path.join(ROOT, "dmrg.x_b200", "DMRG-SquareLattice.x")}
-SM, SZ, SP = -1, 0, 1
-J1J2_CYL = dict(Lx=4, Ly=4, J1=0.5, Jz1=1.0, J2=0.25, Jz2=0.5, bcx=0, bcy=1)
-HEIS_CHAIN12 = dict(Lx=12, Ly=1, J1=0.5, Jz1=1.0, J2=0.0, Jz2=0.0, bcx=0, bcy=0)
-
-
-@pytest.fixture(scope="module", params=["plancheck", pytest.param("cuda", marks=pytest.mark.gpu)])
-def P(request):
-    import dmrgx_loader
-    P = dmrgx_loader.load_package()
-    if request.param == "plancheck":
-        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "dmrg.x_b200", "csrc"), "plancheck"])
-        libswitch.use_library(P, PLANCHECK)
-    else:
-        libswitch.use_library(P, None)
-    P.kind = request.param
-    yield P
-    libswitch.use_library(P, None)
-
-
-@pytest.fixture()
-def ctx(P):
-    c = P.Context(0)
-    yield c
-    c.close()
-
-
-def ngpus():
-    try:
-        import torch
-        return torch.cuda.device_count()
-    except Exception:
-        return 0
+from measure_common import (DRIVER_M, DRIVER_RUN, HEIS_CHAIN12, J1J2_CYL, SM, SP, SZ, P, ctx, dense_shell,  # noqa: F401
+                            exact_diagonalisation, exact_halves, exe, ham_terms, ngpus, oracle_blocks, random_psi,
+                            start_vectors, tridiag)
 
 
 # ---- references --------------------------------------------------------------------------------------------------------
-
-def ham_terms(P, ham, nsites):
-    return P.HamiltonianTerms(ham["Lx"], ham["Ly"], ham["J1"], ham["Jz1"], ham["J2"], ham["Jz2"], nsites, ham["bcx"], ham["bcy"])
-
-
-def oracle_blocks(orc, P, ctx, nsites_L, nsites_R, spin_twice=1):
-    """oracle warm-up blocks of the 4x4 J1-J2 cylinder, enlarged by one site, uploaded to the product"""
-    h = J1J2_CYL
-    d = orc.DMRG(h["Lx"], h["Ly"], h["J1"], h["Jz1"], h["J2"], h["Jz2"], spin_twice=spin_twice)
-    d.warmup(20)
-    enl = lambda k: orc.kron_eye(d.block(k - 2), orc.Block.single_site(spin_twice), pc.lr_terms(orc, h, k))
-    pL = pc.upload_block(P, ctx, enl(nsites_L), orc)
-    pR = pL if nsites_R == nsites_L else pc.upload_block(P, ctx, enl(nsites_R), orc)
-    return pL, pR
-
-
-def exact_halves(P, ctx, ham):
-    """the two un-truncated halves of a lattice (every Sz_i / Sp_i exact) and the terms of the whole lattice"""
-    N = ham["Lx"] * ham["Ly"]
-    site = P.Block.SingleSite(ctx)
-    blk = P.Block.SingleSite(ctx)
-    for k in range(2, N // 2 + 1):
-        blk = P.KronEye_Explicit(blk, site, ham_terms(P, ham, k))
-    return blk, ham_terms(P, ham, N)
-
-
-def kron_index(kb, nR):
-    """full L⊗R index (a·NR + b) of every state of a Kron, in the Kron's order"""
-    qn, il, ir, sz, off = kb.data()
-    Lq, Ls = kb.left.sectors()
-    Rq, Rs = kb.right.sectors()
-    Lo, Ro = np.concatenate([[0], np.cumsum(Ls)]), np.concatenate([[0], np.cumsum(Rs)])
-    idx = []
-    for p in range(len(qn)):
-        for a in range(Lo[il[p]], Lo[il[p] + 1]):
-            idx.extend(a * nR + np.arange(Ro[ir[p]], Ro[ir[p] + 1]))
-    return np.array(idx, np.int64)
-
-
-def start_vectors(kb, tk, psi, op, coef):
-    """phi_v = Σ_s coef[v, s] O_s psi on the target Kron, from the dense block operators embedded with the Kron offsets"""
-    L, R = kb.left, kb.right
-    nL, nR = L.NumSites(), R.NumSites()
-    NL, NR = L.NumStates(), R.NumStates()
-    dense = lambda blk, i: pc.dense_op(blk, SP, i).T if op == SM else pc.dense_op(blk, op, i)
-    full = np.zeros(NL * NR)
-    full[kron_index(kb, NR)] = psi
-    X = full.reshape(NL, NR)
-    panels = []
-    for s in range(nL + nR):
-        Y = dense(L, s) @ X if s < nL else X @ dense(R, nL + nR - 1 - s).T
-        panels.append(Y.reshape(-1)[kron_index(tk, NR)])
-    return np.asarray(coef) @ np.array(panels)
-
-
-def dense_shell(shell, n):
-    return np.array([shell.MatMult_host(e) for e in np.eye(n)]).T
-
-
-def tridiag(a, b, k):
-    return np.diag(a[:k]) + np.diag(b[1:k], 1) + np.diag(b[1:k], -1)
-
 
 def lanczos_moments(r, v, kmax, shift=0.0):
     k = int(r["nsteps_done"][v])
@@ -126,12 +28,6 @@ def lanczos_moments(r, v, kmax, shift=0.0):
         mu.append(r["norm2"][v] * x[0])
         x = T @ x
     return np.array(mu)
-
-
-def random_psi(ctx, n, seed):
-    x = np.random.default_rng(seed).standard_normal(n)
-    x /= np.linalg.norm(x)
-    return ctx.vec(n, x), x
 
 
 # ---- the library ---------------------------------------------------------------------------------------------------------
@@ -165,25 +61,6 @@ def test_moments_under_truncation(P, ctx, orc, case):
                 assert abs(got[k] - ref[k]) <= 1e-10 * ref[0] * scale ** k, (op, v, k, got[k], ref[k])
 
 
-def site_op(N, o, i):
-    import scipy.sparse as sp
-    loc = {SZ: np.diag([0.5, -0.5]), SP: np.array([[0.0, 1.0], [0.0, 0.0]]), SM: np.array([[0.0, 0.0], [1.0, 0.0]])}[o]
-    return sp.kron(sp.kron(sp.identity(2 ** i), sp.csr_matrix(loc)), sp.identity(2 ** (N - 1 - i)), format="csr")
-
-
-def exact_diagonalisation(terms, N):
-    """ground state (Sz = 0 sector, full 2^N vector), its energy, H and the single-site operators"""
-    import scipy.sparse.linalg as sla
-    ops = {(o, i): site_op(N, o, i) for o in (SZ, SP, SM) for i in range(N)}
-    H = sum(a * (ops[(io, i)] @ ops[(jo, j)]) for (a, io, i, jo, j) in terms).tocsr()
-    ndown = np.array([bin(b).count("1") for b in range(2 ** N)])
-    sec = np.nonzero(ndown == N // 2)[0]
-    w, v = sla.eigsh(H[sec][:, sec], k=1, which="SA", tol=1e-14)
-    psi = np.zeros(2 ** N)
-    psi[sec] = v[:, 0]
-    return w[0], psi, H, ops, ndown
-
-
 def chain_coefs(N):
     """cos and sin of every chain momentum q = 2πk/N over the sites, /√N: rows 2k and 2k + 1"""
     c = []
@@ -201,7 +78,8 @@ def _check_exact(P, ctx, ham, pole_steps):
     H0 = kb.KronSumConstruct(terms)
     e0, dpsi, st = H0.EPSSolve(tol=1e-12)
     assert st["converged"]
-    e_ed, psi, H, ops, ndown = exact_diagonalisation(terms, N)
+    w0, psi, H, ops, ndown = exact_diagonalisation(terms, N)
+    e_ed = w0[0]
     assert abs(e0 - e_ed) < 1e-9 * abs(e_ed)
     coef = chain_coefs(N) if ham["Ly"] == 1 else None
     if coef is None:
@@ -372,18 +250,6 @@ def test_determinism(P, ctx):
 
 
 # ---- the driver ----------------------------------------------------------------------------------------------------------
-
-DRIVER_RUN = (["-Lx", 4, "-Ly", 4, "-J1", 0.5, "-Jz1", 1, "-J2", 0.25, "-Jz2", 0.5], J1J2_CYL)
-DRIVER_M = {"plancheck": (16, [16]), "cuda": (256, [256])}
-
-
-@pytest.fixture(scope="module")
-def exe(P):
-    if P.kind == "plancheck":
-        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "dmrg.x_b200", "driver"), "plancheck"])
-    assert os.path.exists(EXE[P.kind]), "build it with __graft_entry__.build()"
-    return EXE[P.kind]
-
 
 def test_driver_writes_the_spectral_function(P, exe, tmp_path):
     """-do_spectral_function 1 (with -do_correlation_matrix 1): one record per Correlations.json row; summed over cos / sin,

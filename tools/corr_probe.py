@@ -24,7 +24,7 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import dmrgx_loader  # noqa: E402
 import bench_workload as W  # noqa: E402
 from bench import fp64_peak_tflops  # noqa: E402
-from test_correlation_matrix import per_correlator, SM, SZ, SP  # noqa: E402
+from measure_common import SM, SP, SZ, product_expect  # noqa: E402
 
 
 def card():
@@ -90,11 +90,12 @@ def main():
             j = int(rng.integers(nside)) + (0 if (len(sample) % 2 == 0) == (i < nside) else nside)
             sample.append((list(names)[len(sample) % 3], i, j))
         cmax = max(np.abs(got[k]).max() for k in names)
-        per_correlator(P, kb, psi, nside, nside, *(sample[0][1], names[sample[0][0]][0], sample[0][2], names[sample[0][0]][1]))  # warm-up
+        k, i, j = sample[0]
+        product_expect(P, kb, psi, nside, n, [(names[k][0], i), (names[k][1], j)])  # warm-up
         worst = 0.0
         t0 = time.perf_counter()
         for k, i, j in sample:
-            v = per_correlator(P, kb, psi, nside, nside, i, names[k][0], j, names[k][1])
+            v = product_expect(P, kb, psi, nside, n, [(names[k][0], i), (names[k][1], j)])
             worst = max(worst, abs(v - got[k][i, j]))
         per_entry = (time.perf_counter() - t0) / len(sample)
         r = dict(m=m, D=D, sites=n, launches=launches, ms=ms, ms_min=1e3 * min(ts), flops=got["flops"], tflops=tflops, fp64_matmul_tflops=peak,

@@ -25,7 +25,7 @@ import dmrgx_loader  # noqa: E402
 import bench_workload as W  # noqa: E402
 from bench import fp64_peak_tflops  # noqa: E402
 from corr_probe import card, superblock  # noqa: E402
-from test_dimer_matrix import nn_bonds, per_correlator_dimer  # noqa: E402
+from measure_common import nn_bonds, per_correlator_dimer  # noqa: E402
 
 
 def main():
