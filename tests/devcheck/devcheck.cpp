@@ -1,4 +1,4 @@
-/*  TEST-ONLY shim over csrc/dev.h for tests/test_device_kernels.py — NOT part of the product.
+/*  TEST-ONLY shim over csrc/dev.h for tests/test_device_kernels.py and tests/test_sparse_eig_kernels.py — NOT part of the product.
  *
  *  A thin extern "C" layer for ctypes: each entry point copies host arrays to the device, calls one dev:: function and
  *  copies the results back.  It is built twice (csrc/Makefile): libdevcheck_host.so links the host emulation of dev.h
@@ -16,8 +16,12 @@
  *  computes from the kernel's own addressing every element each (work item, segment) pair can touch — clamped rows
  *  included — and refuses a plan that reaches outside its buffer: a mistake in a test is an error return, never a fault.
  *
+ *  Sparse-sector and eigensolver entries (dc_spmm, dc_syevd, tests/test_sparse_eig_kernels.py) follow the same rules; their
+ *  conventions are stated above each of them.
+ *
  *  Every entry point returns 0 or -1; dc_error() holds the message (a refusal of the shim, or what dev:: threw).
  */
+#include <algorithm>
 #include <cmath>
 #include <cstdint>
 #include <cstring>
@@ -34,6 +38,8 @@ using dev::WorkItem;
 using dev::ReduceItem;
 
 static_assert(sizeof(Segment) == 96 && sizeof(WorkItem) == 48 && sizeof(ReduceItem) == 40, "record layouts of tests/test_device_kernels.py");
+static_assert(sizeof(dev::SpTile) == 64 && sizeof(dev::SpASlot) == 64 && sizeof(dev::SpSSlot) == 64 && sizeof(dev::SpBSlot) == 112,
+              "record layouts of tests/devcheck_common.py");
 
 std::string g_msg;
 dev::Stream* g_st = nullptr;
@@ -382,22 +388,113 @@ int dc_gather_rows_reversed(double* src, long long nsrc, int n, int m, double* d
     });
 }
 
-/* run_spmm on one 1×1 tile with no terms, staged for max_nR: only its argument check is of interest */
-int dc_spmm_args(int max_nR) {
+/* One run_spmm launch over the pools X (psi, read), Y (written at X's offsets), I (ELL columns) and V (ELL values).
+   Offsets as in the product: SpTile.off, SpASlot.src and SpBSlot.src are element offsets into X (and Y); SpBSlot.ecol
+   and .eval arrive as element offsets into I and V and are rebased here.  Validation covers every address spmm_kernel
+   forms, including the rows r >= nrows of a partial tile that it reads (but never writes) and the shared-memory stage
+   of SP_ROWS·max_nR doubles that its in-tile offsets index.  Y comes back. */
+int dc_spmm(const void* tiles, int ntiles, const void* aslots, int na, const void* sslots, int ns, const void* bslots, int nb, long long guard, double* X,
+            long long nX, double* Y, long long nY, int* I, long long nI, double* V, long long nV, int max_nR) {
     return guarded([&] {
-        REFUSE_IF(max_nR < 1, "max_nR");
+        using dev::SP_ROWS;
+        REFUSE_IF(ntiles < 0 || na < 0 || ns < 0 || nb < 0 || max_nR < 1, "ntiles, slot counts or max_nR");
+        REFUSE_IF(guard < (long long)SP_ROWS * max_nR, "Y: guard of %lld elements is below SP_ROWS·max_nR = %lld", guard, (long long)SP_ROWS * max_nR);
+        Buf<double> x, y, v;
+        Buf<int> ib;
+        x.set(X, nX, guard, 1, 0, false, "X"); y.set(Y, nY, guard, 1, 0, true, "Y");
+        ib.set(I, nI, guard, 1, 0, false, "I"); v.set(V, nV, guard, 1, 0, false, "V");
+        const long long px = x.n(), stage = (long long)SP_ROWS * max_nR;
+        const int* Ih = I + guard;
+        std::vector<dev::SpTile> tl((const dev::SpTile*)tiles, (const dev::SpTile*)tiles + ntiles);
+        std::vector<dev::SpASlot> as((const dev::SpASlot*)aslots, (const dev::SpASlot*)aslots + na);
+        std::vector<dev::SpSSlot> ss((const dev::SpSSlot*)sslots, (const dev::SpSSlot*)sslots + ns);
+        std::vector<dev::SpBSlot> bs((const dev::SpBSlot*)bslots, (const dev::SpBSlot*)bslots + nb);
+        auto in_x = [&](long long lo, long long n, int w, const char* what) {
+            REFUSE_IF(lo < 0 || lo + n > px, "tile %d: %s [%lld, %lld) outside the %lld-element X", w, what, lo, lo + n, px);
+        };
+        /* an in-tile offset: inside the staged rows for r < nrows, inside the shared-memory stage for r >= nrows */
+        auto in_tile = [&](long long lo, long long hi, int r, const dev::SpTile& t, int w, const char* what) {
+            const long long lim = r < t.nrows ? (long long)t.nrows * t.nR : stage;
+            REFUSE_IF(lo < 0 || hi >= lim, "tile %d row %d: %s [%lld, %lld] outside [0, %lld)", w, r, what, lo, hi, lim);
+        };
+        for (int w = 0; w < ntiles; ++w) {
+            const dev::SpTile& t = tl[(size_t)w];
+            REFUSE_IF(t.nrows < 1 || t.nrows > SP_ROWS || t.nR < 1 || t.nR > max_nR, "tile %d: nrows %d or nR %d (max_nR %d)", w, t.nrows, t.nR, max_nR);
+            in_x(t.off, (long long)t.nrows * t.nR, w, "rows");
+            REFUSE_IF(t.off + (long long)t.nrows * t.nR > y.n(), "tile %d: rows outside Y", w);
+            REFUSE_IF(t.a_begin < 0 || t.a_count < 0 || t.a_begin + t.a_count > na || t.s_begin < 0 || t.s_count < 0 || t.s_begin + t.s_count > ns ||
+                          t.b_begin < 0 || t.b_count < 0 || t.b_begin + t.b_count > nb, "tile %d: slot ranges", w);
+            for (int k = t.a_begin; k < t.a_begin + t.a_count; ++k)
+                for (int r = 0; r < SP_ROWS; ++r) in_x(as[(size_t)k].src[r], t.nR, w, "a-slot source row");
+            for (int k = t.s_begin; k < t.s_begin + t.s_count; ++k)
+                for (int r = 0; r < SP_ROWS; ++r) in_tile(ss[(size_t)k].roff[r], ss[(size_t)k].roff[r] + t.nR - 1LL, r, t, w, "s-slot source row");
+            for (int k = t.b_begin; k < t.b_begin + t.b_count; ++k) {
+                const dev::SpBSlot& b = bs[(size_t)k];
+                REFUSE_IF(b.W < 0 || b.ld < t.nR, "tile %d b-slot %d: W %d or ld %d below nR %d", w, k, b.W, b.ld, t.nR);
+                if (b.W == 0) continue;
+                const long long e0 = (long long)(intptr_t)b.ecol, v0 = (long long)(intptr_t)b.eval, span = (long long)(b.W - 1) * b.ld + t.nR;
+                REFUSE_IF(e0 < 0 || e0 + span > ib.n() || v0 < 0 || v0 + span > v.n(), "tile %d b-slot %d: ELL columns or values outside I / V", w, k);
+                int cmin = 0x7fffffff, cmax = -1;
+                for (int q = 0; q < b.W; ++q)
+                    for (int c = 0; c < t.nR; ++c) { const int col = Ih[e0 + (long long)q * b.ld + c]; cmin = std::min(cmin, col); cmax = std::max(cmax, col); }
+                REFUSE_IF(cmin < 0, "tile %d b-slot %d: negative column", w, k);
+                for (int r = 0; r < SP_ROWS; ++r) {
+                    if (b.all_in) in_tile((long long)b.roff[r] + cmin, (long long)b.roff[r] + cmax, r, t, w, "all_in gather");
+                    else in_x(b.src[r] + cmin, cmax - cmin + 1LL, w, "b-slot gather");
+                }
+            }
+        }
+        for (auto& b : bs) { b.ecol = ib.p() + (intptr_t)b.ecol; b.eval = v.p() + (intptr_t)b.eval; }
         dev::Stream* st = stream();
-        dev::SpTile tile{};
-        tile.nR = 1; tile.nrows = 1;
-        std::vector<double> zero(8, 0.0);
-        Buf<dev::SpTile> t; Buf<double> x, y;
-        t.dev_base = (dev::SpTile*)dev::malloc_bytes(st, sizeof tile);
-        dev::h2d(st, t.dev_base, &tile, sizeof tile);
-        x.dev_base = (double*)dev::malloc_bytes(st, 64);
-        y.dev_base = (double*)dev::malloc_bytes(st, 64);
-        dev::h2d(st, x.dev_base, zero.data(), 64);
-        dev::run_spmm(st, t.dev_base, 1, nullptr, nullptr, nullptr, x.dev_base, y.dev_base, max_nR);
+        Buf<dev::SpTile> dt; Buf<dev::SpASlot> da; Buf<dev::SpSSlot> ds; Buf<dev::SpBSlot> db;
+        auto upload = [&](auto& buf, auto& vec) {   /* at least one record, as the product allocates */
+            using T = typename std::decay_t<decltype(vec)>::value_type;
+            buf.dev_base = (T*)dev::malloc_bytes(st, sizeof(T) * std::max<size_t>(1, vec.size()));
+            dev::h2d(st, buf.dev_base, vec.data(), sizeof(T) * vec.size());
+        };
+        upload(dt, tl); upload(da, as); upload(ds, ss); upload(db, bs);
+        dev::run_spmm(st, dt.dev_base, ntiles, da.dev_base, ds.dev_base, db.dev_base, x.p(), y.p(), max_nR);
+        y.back();
         dev::sync(st);
+    });
+}
+
+/* One syevd_batch call on nblocks blocks: block b is n[b]×n[b] at element offset a_off[b] of the pool A, its eigenvalues
+   go to w_off[b] of W.  The pools are uploaded and read back whole with the shim's async copies on the main stream and no
+   synchronisation before the call, so the solver runs ordered after queued work as dev.h promises.  A payload closer than
+   `guard` elements to another payload or to an end of its pool is refused. */
+int dc_syevd(int nblocks, const int* n, const long long* a_off, const long long* w_off, double* A, long long nA, double* W, long long nW, long long guard) {
+    return guarded([&] {
+        REFUSE_IF(nblocks < 0 || guard < MIN_GUARD, "nblocks, or guard below 4 KiB");
+        auto check_pool = [&](const long long* off, bool square, long long total, const char* name) {
+            std::vector<std::pair<long long, long long>> iv;
+            for (int b = 0; b < nblocks; ++b) {
+                REFUSE_IF(n[b] < 0, "block %d: n %d", b, n[b]);
+                iv.push_back({off[b], off[b] + (square ? (long long)n[b] * n[b] : n[b])});
+            }
+            std::sort(iv.begin(), iv.end());
+            long long end = 0;   /* the pool's start counts as a payload ending at 0 */
+            for (auto& p : iv) {
+                REFUSE_IF(p.first < end + guard, "%s: a payload at %lld is closer than %lld elements to the previous payload or the pool start", name, p.first, guard);
+                end = std::max(end, p.second);
+            }
+            REFUSE_IF(end + guard > total, "%s: a payload ends closer than %lld elements to the pool end (%lld elements)", name, guard, total);
+        };
+        check_pool(a_off, true, nA, "A");
+        check_pool(w_off, false, nW, "W");
+        dev::Stream* st = stream();
+        double* dA = (double*)dev::malloc_bytes(st, sizeof(double) * (size_t)nA);
+        double* dW = (double*)dev::malloc_bytes(st, sizeof(double) * (size_t)nW);
+        struct Free { double *a, *w; ~Free() { dev::free_bytes(g_st, a); dev::free_bytes(g_st, w); } } fr{dA, dW};
+        dev::h2d(st, dA, A, sizeof(double) * (size_t)nA);
+        dev::h2d(st, dW, W, sizeof(double) * (size_t)nW);
+        std::vector<double*> pa((size_t)nblocks), pw((size_t)nblocks);
+        for (int b = 0; b < nblocks; ++b) { pa[(size_t)b] = dA + a_off[b]; pw[(size_t)b] = dW + w_off[b]; }
+        const int rc = dev::syevd_batch(st, nblocks, n, pa.data(), pw.data());
+        dev::d2h(st, A, dA, sizeof(double) * (size_t)nA);
+        dev::d2h(st, W, dW, sizeof(double) * (size_t)nW);
+        dev::sync(st);
+        REFUSE_IF(rc != 0, "syevd_batch returned %d: %s", rc, dev::last_error());
     });
 }
 

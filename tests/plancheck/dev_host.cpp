@@ -206,33 +206,36 @@ void gather_rows_reversed(Stream*, const double* src, int n, int m, double* dst)
     ++g_launches;
     for (int k = 0; k < m; ++k) std::memcpy(dst + (size_t)k * n, src + (size_t)(n - 1 - k) * n, sizeof(double) * n);
 }
-/* cyclic Jacobi; row k of A on exit = k-th eigenvector, ascending eigenvalues */
-static void jacobi(int n, double* A, double* w) {
+/* cyclic Jacobi; row k of A on exit = k-th eigenvector, ascending eigenvalues.  The rotations run in long double: in
+   double, sequential Jacobi leaves about 2n·u·||A|| in the eigenvalues and 6n·u in the orthogonality, above what the
+   eigensolver tests (tests/test_sparse_eig_kernels.py) require of syevd_batch at a few hundred states. */
+static void jacobi(int n, double* A0, double* w) {
     ++g_launches;
-    std::vector<double> V((size_t)n * n, 0.0);
-    for (int i = 0; i < n; ++i) V[(size_t)i * n + i] = 1.0;
-    auto a = [&](int i, int j) -> double& { return A[(size_t)i * n + j]; };
+    typedef long double R;
+    std::vector<R> A(A0, A0 + (size_t)n * n), V((size_t)n * n, 0.0L);
+    for (int i = 0; i < n; ++i) V[(size_t)i * n + i] = 1.0L;
+    auto a = [&](int i, int j) -> R& { return A[(size_t)i * n + j]; };
     for (int sweep = 0; sweep < 100; ++sweep) {
-        double off = 0, diag = 0;
+        R off = 0, diag = 0;
         for (int i = 0; i < n; ++i) { diag += a(i, i) * a(i, i); for (int j = i + 1; j < n; ++j) off += a(i, j) * a(i, j); }
-        if (off <= 1e-32 * (diag + off) || off == 0.0) break;
+        if (off <= 1e-34L * (diag + off) || off == 0.0L) break;
         for (int p = 0; p < n; ++p)
             for (int q = p + 1; q < n; ++q) {
-                if (a(p, q) == 0.0) continue;
-                double theta = (a(q, q) - a(p, p)) / (2.0 * a(p, q));
-                double t = (theta >= 0 ? 1.0 : -1.0) / (std::fabs(theta) + std::sqrt(theta * theta + 1.0));
-                double c = 1.0 / std::sqrt(t * t + 1.0), s = t * c;
-                for (int k = 0; k < n; ++k) { double akp = a(k, p), akq = a(k, q); a(k, p) = c * akp - s * akq; a(k, q) = s * akp + c * akq; }
-                for (int k = 0; k < n; ++k) { double apk = a(p, k), aqk = a(q, k); a(p, k) = c * apk - s * aqk; a(q, k) = s * apk + c * aqk; }
-                for (int k = 0; k < n; ++k) { double vkp = V[(size_t)k * n + p], vkq = V[(size_t)k * n + q]; V[(size_t)k * n + p] = c * vkp - s * vkq; V[(size_t)k * n + q] = s * vkp + c * vkq; }
+                if (a(p, q) == 0.0L) continue;
+                R theta = (a(q, q) - a(p, p)) / (2.0L * a(p, q));
+                R t = (theta >= 0 ? 1.0L : -1.0L) / (std::fabs(theta) + std::sqrt(theta * theta + 1.0L));
+                R c = 1.0L / std::sqrt(t * t + 1.0L), s = t * c;
+                for (int k = 0; k < n; ++k) { R akp = a(k, p), akq = a(k, q); a(k, p) = c * akp - s * akq; a(k, q) = s * akp + c * akq; }
+                for (int k = 0; k < n; ++k) { R apk = a(p, k), aqk = a(q, k); a(p, k) = c * apk - s * aqk; a(q, k) = s * apk + c * aqk; }
+                for (int k = 0; k < n; ++k) { R vkp = V[(size_t)k * n + p], vkq = V[(size_t)k * n + q]; V[(size_t)k * n + p] = c * vkp - s * vkq; V[(size_t)k * n + q] = s * vkp + c * vkq; }
             }
     }
     std::vector<int> ord(n);
     for (int i = 0; i < n; ++i) ord[i] = i;
-    std::vector<double> d(n);
+    std::vector<R> d(n);
     for (int i = 0; i < n; ++i) d[i] = a(i, i);
     std::stable_sort(ord.begin(), ord.end(), [&](int x, int y) { return d[x] < d[y]; });
-    for (int k = 0; k < n; ++k) { w[k] = d[ord[k]]; for (int i = 0; i < n; ++i) A[(size_t)k * n + i] = V[(size_t)i * n + ord[k]]; }
+    for (int k = 0; k < n; ++k) { w[k] = (double)d[ord[k]]; for (int i = 0; i < n; ++i) A0[(size_t)k * n + i] = (double)V[(size_t)i * n + ord[k]]; }
 }
 
 int syevd_batch(Stream*, int nblocks, const int* n, double* const* A, double* const* w) {

@@ -27,25 +27,15 @@ bit-reproducibility (two calls, the two ring depths, a Lanczos column alone or i
 where the data are exact (dyadic Gram inputs, copies, splitmix64) exact equality.
 """
 import ctypes as C
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
-from devcheck_common import (LD, SENT, U, Backend, assert_bound, assert_guards, assert_unchanged, bits, guard_for, rng_for,
-                             sentinel, wrap)
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-CSRC = os.path.join(ROOT, "dmrg.x_b200", "csrc")
-LIBS = {"host": os.path.join(ROOT, "tests", "devcheck", "libdevcheck_host.so"),
-        "cuda": os.path.join(ROOT, "tests", "devcheck", "libdevcheck_cuda.so")}
-# DMRGX_DEVCHECK_CUDA: run the cuda flavour against another build of the shim (for example over a modified dev_cuda.cu)
-CUDA_OVERRIDE = os.environ.get("DMRGX_DEVCHECK_CUDA")
+from devcheck_common import (LD, SENT, SP_ASLOT, SP_BSLOT, SP_MAX_NR, SP_ROWS, SP_SSLOT, SP_TILE, U, Backend, assert_bound, assert_guards,
+                             assert_unchanged, bits, guard_for, lib_path, rng_for, sentinel, wrap)
 
 DEEP_BELOW = 1800                        # run_chain: launches below this many items take the three-stage copy ring
 RED_BLOCKS = 592                         # grid of the streaming kernels
-SP_MAX_NR = 3072
 MAX_BASIS = 39
 SEG_GEMM, SEG_AXPY, SEG_DIAG, SEG_CSRA, SEG_CSRB, SEG_CSRADD = range(6)
 SEGF_A_X, SEGF_B_X = 1, 2
@@ -66,20 +56,11 @@ CELL = 80   # rows / columns of the operand cells the work items cut their tiles
 # ---------------------------------------------------------------------------------------------------------------------
 #  backend and buffers
 # ---------------------------------------------------------------------------------------------------------------------
-def _lib_path(name):
-    if name == "cuda" and CUDA_OVERRIDE:
-        return CUDA_OVERRIDE
-    path = LIBS[name]
-    if not os.path.exists(path):
-        subprocess.check_call(["make", "-s", "-C", CSRC, "devcheck-" + name])
-    return path
-
-
 @pytest.fixture(scope="module", params=["host", pytest.param("cuda", marks=pytest.mark.gpu)])
 def dc(request):
     # the int arguments of every dc_* entry point are declared long long or int; ctypes passes c_longlong, which is
     # also right for int arguments on x86-64 / aarch64 (registers and 8-byte stack slots)
-    return Backend(request.param, _lib_path(request.param))
+    return Backend(request.param, lib_path(request.param))
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -476,7 +457,7 @@ def test_chain_refuses_plans_past_their_buffers(dc):
 def test_emulation_refuses_stager_offsets_past_32_bits():
     """host emulation: a GEMM whose staged element offsets need more than 32 bits is refused (chain_kernel's Stager keeps
     them in int); the nearest legal plan passes"""
-    lib = C.CDLL(_lib_path("host"))
+    lib = C.CDLL(lib_path("host"))
     msg = C.create_string_buffer(512)
     it = np.zeros(1, ITEM); it["tm"], it["tn"], it["seg_end"] = 64, 64, 1
     sg = np.zeros(1, SEG); sg["type"], sg["K"], sg["coef"] = SEG_GEMM, 16, 1.0
@@ -721,8 +702,19 @@ def test_basis_limits_are_refused(dc):
     assert "gs_pass" in dc.refused("dc_gs_pass", V, V.size, n, MAX_BASIS + 1, w, w.size, n, c, c.size, r, r.size, None, 0, g)
     assert "gs_final" in dc.refused("dc_gs_final", V, V.size, n, MAX_BASIS + 2, w, w.size, n, c, c.size, nin, nin.size, r, r.size, o, o.size, g)
     assert "ritz_rotate" in dc.refused("dc_ritz_rotate", V, V.size, n, n, MAX_BASIS + 2, c, c.size, 1, g)
-    assert "run_spmm" in dc.refused("dc_spmm_args", SP_MAX_NR + 1)
-    dc.ok("dc_spmm_args", SP_MAX_NR)
+    # run_spmm: one 1×1 tile without terms, staged for max_nR; the guard covers SP_ROWS·max_nR as dc_spmm requires
+    for max_nr, ok in ((SP_MAX_NR + 1, False), (SP_MAX_NR, True)):
+        gs = guard_for(SP_ROWS * max_nr)
+        tile = np.zeros(1, SP_TILE)
+        tile["nR"], tile["nrows"] = 1, 1
+        X, Y, I, Vv = wrap(np.zeros(1), gs), sentinel(1, gs), wrap(np.zeros(1, np.int32), gs), wrap(np.zeros(1), gs)
+        args = ("dc_spmm", tile, 1, np.zeros(1, SP_ASLOT), 0, np.zeros(1, SP_SSLOT), 0, np.zeros(1, SP_BSLOT), 0, gs, X, X.size, Y, Y.size, I, I.size,
+                Vv, Vv.size, max_nr)
+        if ok:
+            dc.ok(*args)
+            assert Y[gs] == 0.0
+        else:
+            assert "run_spmm" in dc.refused(*args)
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -881,7 +873,7 @@ def test_lanczos_batch_passes(dc, n):
 
 
 def test_lanczos_emulation_refuses_short_ld():
-    dc = Backend("host", _lib_path("host"))
+    dc = Backend("host", lib_path("host"))
     L = Lanczos(dc, 16, 16, 2, [np.ones(16)] * 2, [0.0, 0.0])
     L.ld = 15
     assert "ld below n" in dc.refused("dc_lanczos", 0, 0, 2, 2, 16, 15, *[L.full[k] for k in ("alpha", "beta", "norm2", "ndone", "a", "scale", "zero2", "done", "tickets")],

@@ -9,6 +9,7 @@ import libswitch
 import pytest
 
 import parity_common as pc
+from devcheck_common import eig_inputs
 
 pytestmark = pytest.mark.gpu
 
@@ -241,43 +242,6 @@ def _eig_selftest(P, ctx, mats):
     return out, ms.value
 
 
-def _rho_like(rng, n):
-    k = max(1, (2 * n) // 3)                                   # rank-deficient like rho_L of a wide psi block
-    X = rng.standard_normal((n, k)) * np.exp(-0.35 * np.arange(k))[None, :]
-    R = X @ X.T
-    return R / np.trace(R)
-
-
-def _with_spectrum(rng, lam):
-    Q, _ = np.linalg.qr(rng.standard_normal((len(lam), len(lam))))
-    R = (Q * lam[None, :]) @ Q.T
-    return (R + R.T) / 2
-
-
-def _eig_inputs(case):
-    """rho-like blocks at the listed sizes, or the named input family"""
-    rng = np.random.default_rng(12)
-    if isinstance(case, list):
-        return [_rho_like(rng, n) for n in case]
-    if case == "multiplets":   # exact multiplicities 2-8, as SU(2)-symmetric rho blocks have, on both solver paths
-        out = []
-        for n in (36, 150):
-            lam = np.concatenate([np.full(mult, v) for mult, v in zip(np.resize(np.arange(2, 9), n), np.exp(-rng.uniform(0, 20, n)))])[:n]
-            out.append(_with_spectrum(rng, np.sort(lam)[::-1]))
-        return out
-    if case == "diagonal":     # already converged
-        return [np.diag(rng.standard_normal(n)) for n in (1, 30, 64, 100, 193)]
-    if case == "zero":
-        return [np.zeros((n, n)) for n in (1, 10, 64, 70, 129)]
-    if case == "indefinite":   # padding coordinates must keep their trailing positions among negative eigenvalues
-        return [_with_spectrum(rng, rng.standard_normal(n)) for n in (50, 65, 130, 193)]
-    if case == "negative-definite":
-        return [-_rho_like(rng, n) - 0.1 * np.eye(n) for n in (64, 65, 129, 192)]
-    if case == "batch-300":
-        return [_rho_like(rng, int(n)) for n in rng.integers(1, 65, 300)]
-    raise ValueError(case)
-
-
 @pytest.mark.parametrize("case", [[65, 96, 128], [130, 200, 333, 64, 17, 1], [512, 700, 257], [832, 640, 448, 250, 120, 832, 640, 448, 250, 120],
                                   [1, 2, 63, 64, 65, 127, 128, 129, 192, 193], "multiplets", "diagonal", "zero", "indefinite", "negative-definite",
                                   "batch-300"],
@@ -289,7 +253,7 @@ def test_batched_block_jacobi_eigensolver(P, ctx, case):
     the sizes of the cyclic-Jacobi / block-Jacobi switch and of the 64-padding, exact multiplets, diagonal, zero,
     indefinite and negative-definite inputs and one batch of 300 small blocks, against numpy's LAPACK: eigenvalues to
     5e-14 of the norm, residual and orthogonality to 1e-13."""
-    mats = _eig_inputs(case)
+    mats = eig_inputs(case)
     res, ms = _eig_selftest(P, ctx, mats)
     for (w, V), R in zip(res, mats):
         ref = np.linalg.eigvalsh(R)
