@@ -109,13 +109,15 @@ double eigs_smallest(HShell* H, const EigsOpts& opts, double* d_psi, EigsStats* 
     const bool early_test = early_env ? NG >= atoll(early_env) : (NG >= 50000LL && H->alg_flops >= (dist ? 2e11 : (have_start ? 1e9 : 1e10)));
     int nc = ld, k = 0;
     double theta = 0, resid = 0;
+    long long nreseed = 0;
     for (long long it = 0; it < max_it; ++it) {
         double beta_last = 0;
-        bool invariant = false;
+        bool invariant = false, reseeded = false;
         nc = ld;
         int absorbed = k; /* rows [k, absorbed) of the coefficient table are already in T */
         /* bring the coefficient rows [absorbed, upto) to the host and enter them into the projected matrix; true when an
-           invariant subspace was reached (the steps queued after it worked on a null direction and are ignored) */
+           invariant subspace was reached after row nc - 1 (the steps queued after it worked on a null direction: their rows
+           are not absorbed) */
         auto absorb_rows = [&](int upto) -> bool {
             if (upto <= absorbed) return false;
             dev::d2h(st, hh.data() + (size_t)absorbed * RW, d_tab + (size_t)absorbed * RW, (size_t)(upto - absorbed) * RW * 8);
@@ -129,24 +131,18 @@ double eigs_smallest(HShell* H, const EigsOpts& opts, double* d_psi, EigsStats* 
                 }
                 const double b = std::sqrt(std::max(0.0, r[2 * (ld + 1) + 1]));
                 beta_last = b;
-                if (!(b >= 1e-14)) { nc = j + 1; invariant = true; absorbed = upto; return true; }
+                if (!(b >= 1e-14)) { nc = j + 1; invariant = true; absorbed = j + 1; return true; }
             }
             absorbed = upto;
             return false;
         };
-        for (int j = k; j < nc; ++j) {
-            if (dist) {
-                dev::d2d(st, xfull->as<double>() + R0, V + (size_t)j * N, (size_t)N * 8);
-                hshell_apply_sharded(H, xfull->as<double>(), w - R0);
-            } else {
-                hshell_apply(H, V + (size_t)j * N, w);
-            }
-            stats.nmatvec++;
-            /* classical Gram-Schmidt against the whole basis, twice, as three fused passes over the basis with TWO reductions:
-                 dots  |  update + dots + ||w'||^2  |  update + normalise,
-               the last norm by Pythagoras, ||w''||^2 = ||w'||^2 - |h2|^2 (the second-pass coefficients are round-off sized: no
-               cancellation), so the third pass needs no reduction — on several GPUs two all-reduces per step instead of three.
-               The coefficients stay on the device until the end of the cycle. */
+        /* classical Gram-Schmidt of w against V_0..V_{j}, twice, into V_{j+1}, with the coefficients in row j of the table: three
+           fused passes over the basis with TWO reductions,
+             dots  |  update + dots + ||w'||^2  |  update + normalise,
+           the last norm by Pythagoras, ||w''||^2 = ||w'||^2 - |h2|^2 (the second-pass coefficients are round-off sized: no
+           cancellation), so the third pass needs no reduction — on several GPUs two all-reduces per step instead of three.
+           The coefficients stay on the device until the end of the cycle. */
+        auto orthonormalise = [&](int j) {
             double* d_h = d_tab + (size_t)j * RW;
             double* d_h2 = d_h + (ld + 1);
             double* d_n = d_h2 + (ld + 1);   /* ||w'||^2, directly behind the pass-2 coefficients: one all-reduce covers both */
@@ -156,19 +152,44 @@ double eigs_smallest(HShell* H, const EigsOpts& opts, double* d_psi, EigsStats* 
             dev::gs_pass(st, V, N, j + 1, w, N, d_h, d_h2, d_n);
             if (dist) dev::allreduce_sum(st, d_h2, (ld + 1) + 1);
             dev::gs_final(st, V, N, j + 1, w, N, d_h2, d_n, d_b2, V + (size_t)(j + 1) * N);
-            /* On large superblocks (a matvec costs far more than a host round trip) the stopping test is also made inside the
-               cycle, after every step from the second new one on, instead of only at the restart boundary: saves the 4 or so
-               matvecs a converged solve would otherwise still run to fill the basis. */
-            if (early_test && j + 1 < nc && j >= k + 1) {
-                if (absorb_rows(j + 1)) break;
-                const int nj = j + 1;
-                std::vector<double> Tj((size_t)nj * nj), evj, Sj;
-                for (int a = 0; a < nj; ++a) for (int b = 0; b < nj; ++b) Tj[(size_t)a * nj + b] = T[(size_t)a * ld + b];
-                small_sym_eig(nj, Tj, evj, Sj);
-                if (std::fabs(beta_last * Sj[(size_t)(nj - 1) * nj + 0]) <= opts.tol * std::max(std::fabs(evj[0]), 1e-300)) { nc = nj; break; }
+        };
+        for (int j0 = k;;) {
+            for (int j = j0; j < nc; ++j) {
+                if (dist) {
+                    dev::d2d(st, xfull->as<double>() + R0, V + (size_t)j * N, (size_t)N * 8);
+                    hshell_apply_sharded(H, xfull->as<double>(), w - R0);
+                } else {
+                    hshell_apply(H, V + (size_t)j * N, w);
+                }
+                stats.nmatvec++;
+                orthonormalise(j);
+                /* On large superblocks (a matvec costs far more than a host round trip) the stopping test is also made inside the
+                   cycle, after every step from the second new one on, instead of only at the restart boundary: saves the 4 or so
+                   matvecs a converged solve would otherwise still run to fill the basis. */
+                if (early_test && !reseeded && j + 1 < nc && j >= k + 1) {
+                    if (absorb_rows(j + 1)) break;
+                    const int nj = j + 1;
+                    std::vector<double> Tj((size_t)nj * nj), evj, Sj;
+                    for (int a = 0; a < nj; ++a) for (int b = 0; b < nj; ++b) Tj[(size_t)a * nj + b] = T[(size_t)a * ld + b];
+                    small_sym_eig(nj, Tj, evj, Sj);
+                    if (std::fabs(beta_last * Sj[(size_t)(nj - 1) * nj + 0]) <= opts.tol * std::max(std::fabs(evj[0]), 1e-300)) { nc = nj; break; }
+                }
             }
+            if (!invariant) absorb_rows(nc);
+            /* An invariant subspace smaller than the basis need not hold the wanted pair (a start vector without a ground-state
+               component reaches one, e.g. an exact excited eigenvector).  As ARPACK's dgetv0 does, the cycle then goes on from a
+               fresh seeded random direction, orthogonalised twice against the basis: its couplings to the exhausted block are
+               round-off sized and enter T as such.  The in-cycle stopping test stays off for the rest of the cycle, so a Ritz
+               pair of the exhausted block is only accepted after the new direction has had its steps. */
+            if (!invariant || nc >= ld) break;
+            ++nreseed;
+            dev::fill_random(st, w, N, opts.seed ^ (0xD1B54A32D192ED03ULL * (unsigned long long)nreseed), R0);
+            orthonormalise(nc - 1);
+            invariant = false;
+            reseeded = true;
+            j0 = nc;
+            nc = ld;
         }
-        if (!invariant) absorb_rows(nc);
         std::vector<double> Tm((size_t)nc * nc), ev, S;
         for (int i = 0; i < nc; ++i) for (int j = 0; j < nc; ++j) Tm[(size_t)i * nc + j] = T[(size_t)i * ld + j];
         small_sym_eig(nc, Tm, ev, S); /* ascending: the wanted pair is column 0 */

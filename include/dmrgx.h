@@ -150,7 +150,14 @@ typedef struct { dmrgx_int nmatvec, nrestart, converged; double resid; } dmrgx_e
 int dmrgx_eigs_smallest(dmrgx_hshell h, const dmrgx_eigs_opts* opts, double* e0, double* d_psi, dmrgx_eigs_stats* stats);
 /* EXTENSION (no reference counterpart: EPSSolve is never given an initial space there).  The same solve started from
    d_initial (device, global length; on several GPUs every rank passes the whole vector) — the seeded random vector is used
-   when d_initial is NULL, zero or not finite.  Same eigenpair to `tol`, fewer H*psi when the guess is good. */
+   when d_initial is NULL, zero or not finite.  Same eigenpair to `tol`, fewer H*psi when the guess is good.  A guess with no
+   component along the ground state (an exact eigenvector of a block of H, or any vector of an exactly invariant subspace
+   without it, such as a symmetry sector) makes the Krylov space break down (||r|| < 1e-14) before the basis is full; the
+   solve then goes on from a fresh seeded random direction orthogonal to the basis and does not stop before the end of that
+   restart cycle.  It returns the ground state when the steps left in that cycle find a Ritz value below the lowest one of
+   the exhausted space (a space of dimension close to ncv leaves too few of them).  A guess whose ground-state component is
+   rounding-sized but not zero does not break down: its Krylov space leaves the subspace along that noise, and the result
+   depends on it.  An exact ground state as the guess still costs one whole cycle, min(ncv, dimension) H*psi. */
 int dmrgx_eigs_smallest_from(dmrgx_hshell h, const dmrgx_eigs_opts* opts, const double* d_initial, double* e0, double* d_psi, dmrgx_eigs_stats* stats);
 
 /* ---- EXTENSION: wave-function transformation (S. R. White, PRL 77, 3633 (1996)) — the guess for dmrgx_eigs_smallest_from.
